@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU implementation
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also writes the index of the last timed step
 
 A step = one complete FM-index build (pack, suffix sort, BWT, HuffWT + BitRank) of one synthetic
 sample.  N=1: the 1 Gbp sample of BASELINE.json configs[2] (SURVEY 8d "C3": 10M x 100-bp reads,
@@ -51,7 +52,7 @@ CPU_SAMPLE = dict(seed=1, pool_seed=1, pool_size=10, n_genomes=10, genome_len=10
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed loop (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C3", choices=sorted(WORKLOADS))
@@ -64,7 +65,14 @@ def parse_args():
                     help="N>4: rebuild the full collection on one GPU as well (minutes of host time at 8 x 1 Gbp; default only up to N=4)")
     ap.add_argument("--shared-genomes", action="store_true",
                     help="N>1: all ranks draw their reads from the SAME genomes (strong-scaling shape of C4 / C5: --reads = total / N)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="one GPU: write the index the last timed step built to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU build computed (--impl ours)")
+    return args
 
 
 class ClockSampler:
@@ -214,6 +222,50 @@ def sha256_file(path):
                 break
             h.update(blk)
     return h.hexdigest(), os.path.getsize(path)
+
+
+DUMP_SAMPLE = 1 << 20  # entries sampled from each of the three bit-vector arrays of the wavelet tree
+
+
+def dump_outputs(out_dir, idx):
+    """--dump-outputs: the index as dsmfm_fetch hands it to a caller, written to <out_dir>/<name>.npy so that two builds
+    of the project can be compared array for array.  header (n, samplerate, number_of_texts, max_text_length, n_nodes),
+    C, codetable (count, bits, code per symbol) and nodes (leaf, ch, nbits, integers per node, pre-order) are complete,
+    in float64.  The wavelet tree's bit vectors (about 0.8 GB at C3) are sampled: DUMP_SAMPLE positions drawn with a
+    fixed seed over each array of the internal nodes concatenated in pre-order -- wt_words (64-bit words as four 16-bit
+    parts, low first, float32), wt_rs (superblock ranks, float64), wt_rb (block ranks, float32).  About 30 MB in all."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, arr):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+    nodes = [idx.nodes[i] for i in range(idx.n_nodes)]
+    save("header", np.array([idx.n, idx.samplerate, idx.number_of_texts, idx.max_text_length, idx.n_nodes], dtype=np.float64))
+    save("C", np.array(idx.C[:], dtype=np.float64))
+    save("codetable", np.array([(c.count, c.bits, c.code) for c in idx.codetable], dtype=np.float64).reshape(-1, 3))
+    save("nodes", np.array([(nd.leaf, nd.ch, nd.nbits, nd.integers) for nd in nodes], dtype=np.float64).reshape(-1, 4))
+
+    inner = [nd for nd in nodes if not nd.leaf]
+
+    def sample(field, length, dtype, seed):
+        sizes = [length(nd) for nd in inner]
+        off = np.concatenate([[0], np.cumsum(sizes, dtype=np.int64)])
+        total = int(off[-1])
+        rng = np.random.default_rng(seed)
+        pos = np.sort(rng.integers(0, total, size=DUMP_SAMPLE)) if total > DUMP_SAMPLE else np.arange(total)
+        which = np.searchsorted(off, pos, side="right") - 1
+        out = np.empty(pos.size, dtype=dtype)
+        for j, nd in enumerate(inner):
+            sel = which == j
+            if sel.any():
+                out[sel] = np.ctypeslib.as_array(getattr(nd, field), shape=(sizes[j],))[pos[sel] - off[j]]
+        return out
+
+    words = sample("data", lambda nd: nd.integers, np.uint64, 1)
+    save("wt_words", ((words[:, None] >> np.arange(0, 64, 16, dtype=np.uint64)) & np.uint64(0xFFFF)).astype(np.float32))
+    save("wt_rs", sample("Rs", lambda nd: nd.nbits // 256 + 1, np.uint64, 2).astype(np.float64))
+    save("wt_rb", sample("Rb", lambda nd: nd.nbits // 64 + 1, np.uint8, 3).astype(np.float32))
 
 
 def multi_gpu_parity(args, dist, torch, dsmfm, dsmgen, multigpu, engine, host_docs, kw, rank, world, local):
@@ -377,12 +429,11 @@ def fasta_front_end(args, kw, local, stream, torch, dsmfm, dsmgen):
     for _ in range(2):
         step()
     torch.cuda.synchronize()
-    steps = max(2, min(args.steps, 3))
     t0 = time.perf_counter()
-    for _ in range(steps):
+    for _ in range(args.steps):
         info, s = step()
     torch.cuda.synchronize()
-    dt = (time.perf_counter() - t0) / steps
+    dt = (time.perf_counter() - t0) / args.steps
     return {"value": round(bases / dt / 1e6, 2), "unit": "Mbp/s", "ms_per_step": round(1000 * dt, 2),
             "fasta_bytes_per_step": int(host.numel()), "documents": int(info["documents"]),
             "api": "dsmfm_create / dsmfm_append_fasta (pinned host buffer, parsed on the GPU) / dsmfm_finish / dsmfm_destroy",
@@ -391,7 +442,7 @@ def fasta_front_end(args, kw, local, stream, torch, dsmfm, dsmgen):
             "fetch_wall_ms": round(s.ms_wall_fetch, 2)}
 
 
-def query_side(host_docs, local, stream, torch, dsmfm):
+def query_side(host_docs, local, stream, torch, dsmfm, reps):
     """dsmfm_searcher_lf_device on the index of the workload: random (symbol, position) LF queries, device arrays,
     CUDA events.  Every query walks the Huffman code of its symbol: per level one 8-byte Rs, one 1-byte Rb and one
     8-byte bit word, each a random access to HBM."""
@@ -411,7 +462,6 @@ def query_side(host_docs, local, stream, torch, dsmfm):
         s.lf_device(qc, qi, out)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
-    reps = 5
     e0.record()
     for _ in range(reps):
         s.lf_device(qc, qi, out)  # runs on the searcher's stream and waits for it
@@ -434,6 +484,8 @@ def main():
     os.dup2(2, 1)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs is for a one-GPU run")
     if world > 1:  # torchrun pins OMP_NUM_THREADS to 1; the read generator (input preparation) is OpenMP code
         os.environ["OMP_NUM_THREADS"] = str(max(1, (os.cpu_count() or 1) // world))
     import torch
@@ -471,6 +523,7 @@ def main():
     dev_docs = host_docs.cuda(non_blocking=False)
     stream = torch.cuda.current_stream()
     flags = 0
+    last_build = [None]
 
     if world > 1:
         import multigpu
@@ -484,18 +537,21 @@ def main():
             launches[0] += s.kernel_launches
             return s, out_bytes
 
-        def device_step():  # inputs resident in HBM, every rank's share of the sections left in its HBM
+        def device_step(last=False):  # inputs resident in HBM, every rank's share of the sections left in its HBM
             return sharded(dev_docs, False)[0]
 
         def e2e_step():
             return sharded(host_docs)
     else:
-        def device_step():
+        def device_step(last=False):
             b = dsmfm.Builder(device=local, stream=stream.cuda_stream, expected_bytes=nbytes, flags=flags)
             b.append_batch_device(dev_docs)
             b.build_device()
             s = b.stats()
-            b.close()
+            if last and args.dump_outputs:
+                last_build[0] = b  # its sections stay in HBM until they are dumped behind the timed region
+            else:
+                b.close()
             return s
 
         def e2e_step():
@@ -521,9 +577,9 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
     stats, step_wall = [], []
-    for _ in range(args.steps):
+    for i in range(args.steps):
         t_s = time.perf_counter()
-        stats.append(device_step())
+        stats.append(device_step(last=i == args.steps - 1))
         step_wall.append(round(1000 * (time.perf_counter() - t_s), 1))
     e1.record(stream)
     barrier()
@@ -532,6 +588,9 @@ def main():
     if dist is not None:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms.item())
+    if last_build[0] is not None:
+        dump_outputs(args.dump_outputs, last_build[0].fetch())
+        last_build[0].close()
 
     # ---- end to end through the C ABI with host buffers ("e2e") ---------------------------------------
     for _ in range(min(args.warmup, 2)):
@@ -663,7 +722,7 @@ def main():
     if world == 1:
         # the same workload with the WHOLE suffix array finished (DSMFM_FLAG_KEEP_SA: what BASELINE.json's "SA" and the
         # .sa sampling need); device-resident inputs, CUDA events on the build stream like `value`
-        sa_steps = max(2, min(args.steps, 3))
+        sa_steps = args.steps
         sa_stats = []
         for i in range(1 + sa_steps):
             b = dsmfm.Builder(device=local, stream=stream.cuda_stream, expected_bytes=nbytes, flags=dsmfm.FLAG_KEEP_SA)
@@ -695,7 +754,7 @@ def main():
 
     if world == 1 and not args.no_extras:
         line["fasta_e2e"] = fasta_front_end(args, kw, local, stream, torch, dsmfm, dsmgen)
-        line["search"] = query_side(host_docs, local, stream, torch, dsmfm)
+        line["search"] = query_side(host_docs, local, stream, torch, dsmfm, args.steps)
 
     if world == 1 and not args.no_cpu_baseline:
         import tempfile
