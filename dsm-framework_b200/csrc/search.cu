@@ -89,14 +89,9 @@ __global__ void __launch_bounds__(256) search_rank_kernel(const QIndex *__restri
     out[q] = lf ? fm_lf(x, c[q], i[q]) : wt_rank(x, c[q], i[q]);
 }
 
-// HuffWT::access(i, rank): the symbol at position i and the number of its occurrences in [0, i]
-__global__ void __launch_bounds__(256) search_access_kernel(const QIndex *__restrict__ x, const uint64_t *__restrict__ i,
-                                                            uint8_t *__restrict__ sym, uint64_t *__restrict__ rank,
-                                                            uint64_t count)
+// HuffWT::access(i, rank): the symbol at position i; *rank = the number of its occurrences in [0, i]
+__device__ __forceinline__ uint32_t wt_access(const QIndex *__restrict__ x, uint64_t p, uint64_t &rank)
 {
-    const uint64_t q = (uint64_t)blockIdx.x * 256 + threadIdx.x;
-    if (q >= count) return;
-    uint64_t p = i[q];
     const QNode *t = &x->nodes[0];
     while (!t->leaf) {
         if (p >= t->nbits) p = t->nbits ? t->nbits - 1 : 0; // never outside the node (see wt_rank)
@@ -110,8 +105,19 @@ __global__ void __launch_bounds__(256) search_access_kernel(const QIndex *__rest
             t = &x->nodes[t->left];
         }
     }
-    sym[q] = t->ch;
-    if (rank) rank[q] = p + 1;
+    rank = p + 1;
+    return t->ch;
+}
+
+__global__ void __launch_bounds__(256) search_access_kernel(const QIndex *__restrict__ x, const uint64_t *__restrict__ i,
+                                                            uint8_t *__restrict__ sym, uint64_t *__restrict__ rank,
+                                                            uint64_t count)
+{
+    const uint64_t q = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (q >= count) return;
+    uint64_t r;
+    sym[q] = (uint8_t)wt_access(x, i[q], r);
+    if (rank) rank[q] = r;
 }
 
 // Query::pushChar for every symbol of a small alphabet at once (Query.h:37-45; EnumerateQuery.cpp:45-55):
@@ -149,6 +155,124 @@ __global__ void __launch_bounds__(256) search_count_kernel(const QIndex *__restr
     }
     sp_out[q] = lo;
     ep_out[q] = hi;
+}
+
+// ---- locate / extract over the SA samples of the .sa file (FMIndex::saveSamples, FMIndex.cpp:125-147) --------
+// The five sections stay in HBM as the file holds them: BitRank `sampled` (data, Rs, Rb) and the bit-packed
+// BlockArrays `suffixes`, `suffixDocId`, `textLength`, `Doc` (fields LSB first, Tools::GetField).  A position is
+// resolved by walking LF to the left until the suffix is sampled or starts a document (L[p] = 0).
+struct QSamples {
+    const uint64_t *data, *Rs; // sampled: one bit per BWT position
+    const uint8_t *Rb;
+    const uint64_t *suf, *sdoc, *tlen, *doc; // BlockArray words
+    uint64_t n;       // BWT length: positions at or behind it are refused
+    uint64_t samples; // ones of `sampled` = entries of suf / sdoc (>= 1 whenever a bit is set)
+    uint64_t D;       // documents = entries of tlen / doc
+    uint64_t maxlen;  // longest document: no walk is longer
+    uint32_t wsuf, wdoc, wlen, wend; // field widths of suffixes, suffixDocId, textLength, Doc
+    uint32_t *flag;  // kSampleWalk / kSamplePos, read back after every call
+};
+
+constexpr uint32_t kSampleWalk = 1; // a walk ran past the longest document: .sa and .fmi do not belong together
+constexpr uint32_t kSamplePos = 2;  // a position at or behind n
+
+// Tools::GetField: field i of width len (0..64) of a BlockArray; i < count keeps every read inside its words
+__host__ __device__ __forceinline__ uint64_t get_field(const uint64_t *w, uint64_t i, uint32_t len)
+{
+    if (!len) return 0;
+    const uint64_t bit = i * len, k = bit >> 6;
+    const uint32_t j = (uint32_t)(bit & 63);
+#ifdef __CUDA_ARCH__
+    uint64_t v = __ldg(w + k) >> j;
+    if (j + len > 64) v |= __ldg(w + k + 1) << (64 - j);
+#else
+    uint64_t v = w[k] >> j;
+    if (j + len > 64) v |= w[k + 1] << (64 - j);
+#endif
+    return len == 64 ? v : v & ((1ull << len) - 1);
+}
+
+// (document, offset) of the suffix at BWT position p; false if the walk does not end within the longest document
+__device__ __forceinline__ bool locate_one(const QIndex *__restrict__ x, const QSamples &S, uint64_t p, uint32_t &doc,
+                                           uint64_t &off)
+{
+    for (uint64_t d = 0; d <= S.maxlen; ++d) {
+        if (p >= S.n) return false;
+        const uint64_t w = __ldg(S.data + (p >> 6));
+        if ((w >> (p & 63)) & 1u) {
+            // sampled suffix j = rank1(p) - 1 = ones in front of p; the directories come from the file: clamp
+            uint64_t j = __ldg(S.Rs + (p >> 8)) + __ldg(S.Rb + (p >> 6)) + (uint64_t)__popcll(w & ((1ull << (p & 63)) - 1));
+            j = j < S.samples ? j : S.samples - 1;
+            doc = (uint32_t)get_field(S.sdoc, j, S.wdoc);
+            off = get_field(S.suf, j, S.wsuf) + d;
+            return true;
+        }
+        uint64_t r;
+        const uint32_t c = wt_access(x, p, r);
+        if (c == 0) { // the suffix starts a document: the r-th end marker in BWT order names it
+            if (!S.D) return false;
+            const uint64_t k = r - 1 < S.D ? r - 1 : S.D - 1;
+            doc = (uint32_t)get_field(S.doc, k, S.wend);
+            off = d;
+            return true;
+        }
+        p = x->C[c] + r - 1; // LF: one text position to the left
+    }
+    return false;
+}
+
+// One thread per position: pos[q], or -- with `starts` -- position q of the intervals [sp[k], sp[k] + starts[k+1] -
+// starts[k]) laid end to end (starts: exclusive prefix sums of the interval sizes, starts[nint] = count).
+__global__ void __launch_bounds__(256) search_locate_kernel(const QIndex *__restrict__ x, const QSamples S,
+                                                            const uint64_t *__restrict__ pos, const uint64_t *__restrict__ sp,
+                                                            const uint64_t *__restrict__ starts, uint64_t nint, uint64_t count,
+                                                            uint32_t *__restrict__ doc, uint64_t *__restrict__ off)
+{
+    const uint64_t q = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (q >= count) return;
+    uint64_t p;
+    if (starts) {
+        uint64_t lo = 0, hi = nint - 1; // last k with starts[k] <= q (empty intervals share their start with the next)
+        while (lo < hi) {
+            const uint64_t mid = (lo + hi + 1) >> 1;
+            if (starts[mid] <= q) lo = mid;
+            else hi = mid - 1;
+        }
+        p = sp[lo] + (q - starts[lo]);
+    } else {
+        p = pos[q];
+    }
+    uint32_t dk = 0;
+    uint64_t o = 0;
+    if (p >= S.n) {
+        atomicOr(S.flag, kSamplePos);
+    } else if (!locate_one(x, S, p, dk, o)) {
+        atomicOr(S.flag, kSampleWalk);
+    }
+    doc[q] = dk;
+    off[q] = o;
+}
+
+// One thread per document: the terminator suffix of document k sorts at BWT position k; walking LF from there reads
+// the document right to left.  out[begin[q] ..) has room for textLength[docs[q]] symbols.
+__global__ void __launch_bounds__(256) search_extract_kernel(const QIndex *__restrict__ x, const QSamples S,
+                                                             const uint32_t *__restrict__ docs, const uint64_t *__restrict__ begin,
+                                                             uint64_t count, uint8_t *__restrict__ out)
+{
+    const uint64_t q = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (q >= count) return;
+    const uint32_t k = docs[q];
+    const uint64_t len = get_field(S.tlen, k, S.wlen);
+    uint8_t *dst = out + begin[q];
+    uint64_t p = k, r, i = len;
+    for (; i > 0; --i) {
+        const uint32_t c = wt_access(x, p, r);
+        if (c == 0) break;
+        dst[i - 1] = (uint8_t)c;
+        p = x->C[c] + r - 1;
+    }
+    // the walk must reach the document's start after exactly textLength steps
+    if (i || wt_access(x, p, r) != 0) atomicOr(S.flag, kSampleWalk);
 }
 
 // ---- the mining client's trie walk, level by level (SURVEY 8 f-4) -----------------------------------------
@@ -350,6 +474,12 @@ struct dsmfm_searcher {
     uint8_t *d_blob = nullptr;
     size_t blob_bytes = 0;
     uint64_t n = 0;
+    uint64_t terminators = 0; // C[1] - C[0]: documents of the index
+    // SA samples (dsmfm_searcher_load_samples): one device allocation that `samples` points into, and the words of
+    // textLength on the host, which size the output of extract
+    uint8_t *d_samples = nullptr;
+    QSamples samples{};
+    std::vector<uint64_t> h_tlen;
     // staging for the host-pointer entry points, grown on demand
     uint8_t *d_stage = nullptr;
     size_t stage_bytes = 0;
@@ -430,6 +560,7 @@ int searcher_from_index(int device, const dsmfm_index *idx, dsmfm_searcher **out
     std::memset(q, 0, sizeof *q);
     s->device = device;
     s->n = idx->n;
+    s->terminators = idx->C[1] - idx->C[0];
     q->n = idx->n;
     std::memcpy(q->C, idx->C, sizeof idx->C);
     q->C[256] = idx->n;
@@ -723,6 +854,301 @@ DSMFM_API int dsmfm_searcher_count(dsmfm_searcher *s, const uint8_t *patterns, c
     return DSMFM_OK;
 }
 
+// ---- locate / extract over the SA samples (FMIndex::loadSamples, FMIndex::locate / getSuffix) -------------------
+namespace {
+
+// The .sa layout FMIndex::saveSamples writes (FMIndex.cpp:134-143; dsmfm_sa_serialize): BitRank `sampled` (BitRank::save:
+// n, integers, 64, 256, data[integers], Rs[n/256+1], Rb[n/64+1]), then the BlockArrays suffixes, suffixDocId,
+// textLength, Doc (BlockArray::Save: count, width, words[count*width/64+1]).  Everything is checked against this index
+// before anything is uploaded; the samples attached before stay in place if the image is refused.
+int samples_set_impl(dsmfm_searcher *s, const uint8_t *img, uint64_t bytes)
+{
+    auto bad = [&](const char *what) { return s->fail(DSMFM_EINVAL, "SA samples: %s", what); };
+    uint64_t pos = 0;
+    auto left = [&]() { return bytes - pos; };
+    auto u64 = [&](uint64_t at) { uint64_t v; std::memcpy(&v, img + at, 8); return v; };
+    if (bytes < 24) return bad("truncated header of `sampled`");
+    const uint64_t n = u64(0), integers = u64(8);
+    uint32_t b, sf;
+    std::memcpy(&b, img + 16, 4);
+    std::memcpy(&sf, img + 20, 4);
+    pos = 24;
+    if (n != s->n)
+        return s->fail(DSMFM_EINVAL, "SA samples of an index of %llu symbols, this index has %llu", (unsigned long long)n,
+                       (unsigned long long)s->n);
+    if (integers != n / 64 + 1 || b != 64 || sf != 256) return bad("malformed BitRank `sampled`");
+    // n is this index's length, so none of these sizes can wrap
+    const uint64_t b_data = 8 * integers, b_rs = 8 * (n / 256 + 1), b_rb = n / 64 + 1;
+    if (b_data > left() || b_rs > left() - b_data || b_rb > left() - b_data - b_rs) return bad("truncated `sampled`");
+    const uint64_t o_data = pos, o_rs = o_data + b_data, o_rb = o_rs + b_rs;
+    pos = o_rb + b_rb;
+    uint64_t ones = 0; // among the first n bits: the kernels never look behind them
+    for (uint64_t w = 0; w <= n / 64; ++w) {
+        uint64_t x = u64(o_data + 8 * w);
+        if (w == n / 64) x &= (1ull << (n & 63)) - 1;
+        ones += (uint64_t)__builtin_popcountll(x);
+    }
+    struct Arr {
+        uint64_t count, width, off, words;
+    } a[4];
+    for (Arr &x : a) {
+        if (left() < 16) return bad("truncated BlockArray header");
+        x.count = u64(pos);
+        x.width = u64(pos + 8);
+        pos += 16;
+        if (x.count > n || x.width > 64) return bad("malformed BlockArray header");
+        x.words = x.count * x.width / 64 + 1;
+        if (x.words > left() / 8) return bad("truncated BlockArray");
+        x.off = pos;
+        pos += 8 * x.words;
+    }
+    if (pos != bytes) return s->fail(DSMFM_EINVAL, "SA samples: %llu bytes behind the last section", (unsigned long long)left());
+    const Arr &suf = a[0], &sdoc = a[1], &tlen = a[2], &doc = a[3];
+    if (sdoc.width > 32 || doc.width > 32) return bad("document ids wider than 32 bits");
+    if (suf.count != ones || sdoc.count != ones)
+        return s->fail(DSMFM_EINVAL, "SA samples: %llu / %llu samples for %llu sampled positions", (unsigned long long)suf.count,
+                       (unsigned long long)sdoc.count, (unsigned long long)ones);
+    const uint64_t D = s->terminators;
+    if (tlen.count != D || doc.count != D)
+        return s->fail(DSMFM_EINVAL, "SA samples: %llu / %llu document entries, the index has %llu documents",
+                       (unsigned long long)tlen.count, (unsigned long long)doc.count, (unsigned long long)D);
+    auto words_of = [&](const Arr &x) {
+        std::vector<uint64_t> v(x.words);
+        std::memcpy(v.data(), img + x.off, 8 * x.words);
+        return v;
+    };
+    std::vector<uint64_t> w_tlen = words_of(tlen);
+    uint64_t sum = 0, maxlen = 0;
+    for (uint64_t k = 0; k < D; ++k) {
+        const uint64_t t = get_field(w_tlen.data(), k, (uint32_t)tlen.width);
+        if (t > n - sum) return bad("document lengths add up to more than the index"); // (sum <= n: cannot wrap)
+        sum += t;
+        maxlen = t > maxlen ? t : maxlen;
+    }
+    if (sum + D != n)
+        return s->fail(DSMFM_EINVAL, "SA samples: document lengths add up to %llu + %llu terminators, the index has %llu symbols",
+                       (unsigned long long)sum, (unsigned long long)D, (unsigned long long)n);
+    for (const Arr *x : {&sdoc, &doc}) {
+        const std::vector<uint64_t> w = words_of(*x);
+        for (uint64_t j = 0; j < x->count; ++j)
+            if (get_field(w.data(), j, (uint32_t)x->width) >= D) return bad("document id out of range");
+    }
+
+    uint8_t *blob = nullptr;
+    try {
+        // flag word, then the sections in file order, each at an 8-byte boundary
+        const uint64_t sizes[7] = {b_data, b_rs, b_rb, 8 * suf.words, 8 * sdoc.words, 8 * tlen.words, 8 * doc.words};
+        const uint64_t from[7] = {o_data, o_rs, o_rb, suf.off, sdoc.off, tlen.off, doc.off};
+        uint64_t at[7], total = 8;
+        for (int i = 0; i < 7; ++i) {
+            at[i] = total;
+            total += up8(sizes[i]);
+        }
+        DSM_CUDA(cudaMalloc(&blob, total));
+        DSM_CUDA(cudaMemsetAsync(blob, 0, 8, s->stream));
+        for (int i = 0; i < 7; ++i)
+            DSM_CUDA(cudaMemcpyAsync(blob + at[i], img + from[i], sizes[i], cudaMemcpyHostToDevice, s->stream));
+        DSM_CUDA(cudaStreamSynchronize(s->stream));
+        QSamples &S = s->samples;
+        S.data = reinterpret_cast<const uint64_t *>(blob + at[0]);
+        S.Rs = reinterpret_cast<const uint64_t *>(blob + at[1]);
+        S.Rb = blob + at[2];
+        S.suf = reinterpret_cast<const uint64_t *>(blob + at[3]);
+        S.sdoc = reinterpret_cast<const uint64_t *>(blob + at[4]);
+        S.tlen = reinterpret_cast<const uint64_t *>(blob + at[5]);
+        S.doc = reinterpret_cast<const uint64_t *>(blob + at[6]);
+        S.n = n;
+        S.samples = ones;
+        S.D = D;
+        S.maxlen = maxlen;
+        S.wsuf = (uint32_t)suf.width;
+        S.wdoc = (uint32_t)sdoc.width;
+        S.wlen = (uint32_t)tlen.width;
+        S.wend = (uint32_t)doc.width;
+        S.flag = reinterpret_cast<uint32_t *>(blob);
+    } catch (const CudaError &e) {
+        if (blob) cudaFree(blob);
+        return s->fail(e.code == cudaErrorMemoryAllocation ? DSMFM_ENOMEM : DSMFM_ECUDA, "CUDA error %d (%s) at %s:%d",
+                       (int)e.code, cudaGetErrorString(e.code), e.file, e.line);
+    }
+    if (s->d_samples) cudaFree(s->d_samples);
+    s->d_samples = blob;
+    s->h_tlen.swap(w_tlen);
+    return DSMFM_OK;
+}
+
+#define SAMPLES_GUARD(s)                                                                                    \
+    SEARCH_GUARD(s);                                                                                        \
+    if (!(s)->d_samples) return (s)->fail(DSMFM_EINVAL, "no SA samples attached (dsmfm_searcher_load_samples)")
+
+// the flag the walks raise; the stream has been synchronised by the caller's copies
+int samples_verdict(dsmfm_searcher *s)
+{
+    uint32_t f = 0;
+    DSM_CUDA(cudaMemcpyAsync(&f, s->samples.flag, 4, cudaMemcpyDeviceToHost, s->stream));
+    DSM_CUDA(cudaStreamSynchronize(s->stream));
+    if (f & kSamplePos) return s->fail(DSMFM_EINVAL, "locate: position outside the index (n = %llu)", (unsigned long long)s->n);
+    if (f & kSampleWalk)
+        return s->fail(DSMFM_EINVAL, "SA samples: a walk ran past the longest document (%llu symbols): the .sa file does not "
+                                     "belong to this index", (unsigned long long)s->samples.maxlen);
+    return DSMFM_OK;
+}
+
+void launch_locate(dsmfm_searcher *s, const uint64_t *d_pos, const uint64_t *d_sp, const uint64_t *d_starts, uint64_t nint,
+                   uint64_t count, uint32_t *d_doc, uint64_t *d_off)
+{
+    DSM_CUDA(cudaMemsetAsync(s->samples.flag, 0, 4, s->stream));
+    search_locate_kernel<<<grid_of(count), 256, 0, s->stream>>>(s->d_index, s->samples, d_pos, d_sp, d_starts, nint, count, d_doc,
+                                                                 d_off);
+    DSM_LAUNCH_CHECK();
+}
+
+int cuda_failure(dsmfm_searcher *s, const CudaError &e)
+{
+    return s->fail(e.code == cudaErrorMemoryAllocation ? DSMFM_ENOMEM : DSMFM_ECUDA, "CUDA error %d (%s) at %s:%d", (int)e.code,
+                   cudaGetErrorString(e.code), e.file, e.line);
+}
+
+} // namespace
+
+DSMFM_API int dsmfm_searcher_set_samples(dsmfm_searcher *s, const uint8_t *image, uint64_t bytes)
+{
+    SEARCH_GUARD(s);
+    if (!image && bytes) return s->fail(DSMFM_EINVAL, "null argument");
+    try {
+        return samples_set_impl(s, image, bytes);
+    } catch (const std::bad_alloc &) {
+        return s->fail(DSMFM_ENOMEM, "host allocation failed");
+    }
+}
+
+DSMFM_API int dsmfm_searcher_load_samples(dsmfm_searcher *s, const char *sa_path)
+{
+    SEARCH_GUARD(s);
+    if (!sa_path) return s->fail(DSMFM_EINVAL, "null argument");
+    try {
+        FILE *f = std::fopen(sa_path, "rb");
+        if (!f) return s->fail(DSMFM_EIO, "unable to open %s", sa_path);
+        std::fseek(f, 0, SEEK_END);
+        const long sz = std::ftell(f);
+        std::fseek(f, 0, SEEK_SET);
+        std::vector<uint8_t> img((size_t)(sz > 0 ? sz : 0));
+        const bool ok = sz >= 0 && std::fread(img.data(), 1, img.size(), f) == img.size();
+        std::fclose(f);
+        if (!ok) return s->fail(DSMFM_EIO, "unable to read %s", sa_path);
+        return samples_set_impl(s, img.data(), img.size());
+    } catch (const std::bad_alloc &) {
+        return s->fail(DSMFM_ENOMEM, "host allocation failed while loading the .sa file");
+    }
+}
+
+DSMFM_API int dsmfm_searcher_locate(dsmfm_searcher *s, const uint64_t *pos, uint64_t count, uint32_t *doc, uint64_t *offset)
+{
+    SAMPLES_GUARD(s);
+    if (count == 0) return DSMFM_OK;
+    if (!pos || !doc || !offset) return s->fail(DSMFM_EINVAL, "null argument");
+    try {
+        uint8_t *st = s->stage(count * 20 + 64);
+        uint64_t *d_pos = reinterpret_cast<uint64_t *>(st), *d_off = d_pos + count;
+        uint32_t *d_doc = reinterpret_cast<uint32_t *>(d_off + count);
+        DSM_CUDA(cudaMemcpyAsync(d_pos, pos, count * 8, cudaMemcpyHostToDevice, s->stream));
+        launch_locate(s, d_pos, nullptr, nullptr, 0, count, d_doc, d_off);
+        DSM_CUDA(cudaMemcpyAsync(doc, d_doc, count * 4, cudaMemcpyDeviceToHost, s->stream));
+        DSM_CUDA(cudaMemcpyAsync(offset, d_off, count * 8, cudaMemcpyDeviceToHost, s->stream));
+        return samples_verdict(s);
+    } catch (const CudaError &e) {
+        return cuda_failure(s, e);
+    }
+}
+
+DSMFM_API int dsmfm_searcher_locate_device(dsmfm_searcher *s, const void *pos_dev, uint64_t count, void *doc_dev, void *offset_dev)
+{
+    SAMPLES_GUARD(s);
+    if (count == 0) return DSMFM_OK;
+    if (!pos_dev || !doc_dev || !offset_dev) return s->fail(DSMFM_EINVAL, "null argument");
+    try {
+        launch_locate(s, static_cast<const uint64_t *>(pos_dev), nullptr, nullptr, 0, count, static_cast<uint32_t *>(doc_dev),
+                      static_cast<uint64_t *>(offset_dev));
+        return samples_verdict(s);
+    } catch (const CudaError &e) {
+        return cuda_failure(s, e);
+    }
+}
+
+DSMFM_API int dsmfm_searcher_locate_ranges(dsmfm_searcher *s, const uint64_t *sp, const uint64_t *ep, uint64_t count,
+                                           uint64_t cap, uint32_t *doc, uint64_t *offset, uint64_t *total)
+{
+    SAMPLES_GUARD(s);
+    if (!total || (count && (!sp || !ep))) return s->fail(DSMFM_EINVAL, "null argument");
+    *total = 0;
+    try {
+        std::vector<uint64_t> starts(count + 1);
+        uint64_t sum = 0;
+        for (uint64_t k = 0; k < count; ++k) {
+            starts[k] = sum;
+            if (sp[k] > ep[k]) continue;
+            if (ep[k] >= s->n)
+                return s->fail(DSMFM_EINVAL, "locate_ranges: interval %llu ends at %llu, outside the index", (unsigned long long)k,
+                               (unsigned long long)ep[k]);
+            sum += ep[k] - sp[k] + 1;
+        }
+        starts[count] = sum;
+        *total = sum;
+        if (sum > cap)
+            return s->fail(DSMFM_ELIMIT, "locate_ranges: %llu occurrences, room for %llu", (unsigned long long)sum,
+                           (unsigned long long)cap);
+        if (sum == 0) return DSMFM_OK;
+        if (!doc || !offset) return s->fail(DSMFM_EINVAL, "null argument");
+        uint8_t *st = s->stage(16 * count + 8 + 12 * sum + 64);
+        uint64_t *d_sp = reinterpret_cast<uint64_t *>(st), *d_starts = d_sp + count, *d_off = d_starts + count + 1;
+        uint32_t *d_doc = reinterpret_cast<uint32_t *>(d_off + sum);
+        DSM_CUDA(cudaMemcpyAsync(d_sp, sp, count * 8, cudaMemcpyHostToDevice, s->stream));
+        DSM_CUDA(cudaMemcpyAsync(d_starts, starts.data(), (count + 1) * 8, cudaMemcpyHostToDevice, s->stream));
+        launch_locate(s, nullptr, d_sp, d_starts, count, sum, d_doc, d_off);
+        DSM_CUDA(cudaMemcpyAsync(doc, d_doc, sum * 4, cudaMemcpyDeviceToHost, s->stream));
+        DSM_CUDA(cudaMemcpyAsync(offset, d_off, sum * 8, cudaMemcpyDeviceToHost, s->stream));
+        return samples_verdict(s);
+    } catch (const CudaError &e) {
+        return cuda_failure(s, e);
+    } catch (const std::bad_alloc &) {
+        return s->fail(DSMFM_ENOMEM, "host allocation failed");
+    }
+}
+
+DSMFM_API int dsmfm_searcher_extract(dsmfm_searcher *s, const uint32_t *docs, uint64_t count, uint8_t *out, uint64_t cap,
+                                     uint64_t *offsets)
+{
+    SAMPLES_GUARD(s);
+    if (!offsets || (count && !docs)) return s->fail(DSMFM_EINVAL, "null argument");
+    const QSamples &S = s->samples;
+    offsets[0] = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if (docs[k] >= S.D)
+            return s->fail(DSMFM_EINVAL, "extract: document %u of %llu", docs[k], (unsigned long long)S.D);
+        offsets[k + 1] = offsets[k] + get_field(s->h_tlen.data(), docs[k], S.wlen);
+    }
+    const uint64_t bytes = offsets[count];
+    if (bytes > cap)
+        return s->fail(DSMFM_ELIMIT, "extract: %llu bytes, room for %llu", (unsigned long long)bytes, (unsigned long long)cap);
+    if (count == 0) return DSMFM_OK;
+    if (bytes && !out) return s->fail(DSMFM_EINVAL, "null argument");
+    try {
+        uint8_t *st = s->stage(8 * (count + 1) + 4 * count + bytes + 64);
+        uint64_t *d_begin = reinterpret_cast<uint64_t *>(st);
+        uint32_t *d_docs = reinterpret_cast<uint32_t *>(d_begin + count + 1);
+        uint8_t *d_out = reinterpret_cast<uint8_t *>(d_docs + count);
+        DSM_CUDA(cudaMemcpyAsync(d_begin, offsets, (count + 1) * 8, cudaMemcpyHostToDevice, s->stream));
+        DSM_CUDA(cudaMemcpyAsync(d_docs, docs, count * 4, cudaMemcpyHostToDevice, s->stream));
+        DSM_CUDA(cudaMemsetAsync(S.flag, 0, 4, s->stream));
+        search_extract_kernel<<<grid_of(count), 256, 0, s->stream>>>(s->d_index, S, d_docs, d_begin, count, d_out);
+        DSM_LAUNCH_CHECK();
+        if (bytes) DSM_CUDA(cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, s->stream));
+        return samples_verdict(s);
+    } catch (const CudaError &e) {
+        return cuda_failure(s, e);
+    }
+}
+
 // ---- EnumerateQuery::enumerate as a byte stream -----------------------------------------------------------
 namespace {
 struct StreamSink {
@@ -953,6 +1379,7 @@ DSMFM_API void dsmfm_searcher_destroy(dsmfm_searcher *s)
     if (!s) return;
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
+    if (s->d_samples) cudaFree(s->d_samples);
     if (s->d_stage) cudaFree(s->d_stage);
     if (s->d_blob) cudaFree(s->d_blob);
     if (s->d_index) cudaFree(s->d_index);

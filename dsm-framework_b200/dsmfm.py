@@ -173,6 +173,13 @@ def lib():
     L.dsmfm_searcher_access.argtypes = [S, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
     L.dsmfm_searcher_extend.argtypes = [S, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
     L.dsmfm_searcher_count.argtypes = [S, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+    L.dsmfm_searcher_load_samples.argtypes = [S, C.c_char_p]
+    L.dsmfm_searcher_set_samples.argtypes = [S, C.c_void_p, C.c_uint64]
+    L.dsmfm_searcher_locate.argtypes = [S, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+    L.dsmfm_searcher_locate_device.argtypes = [S, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+    L.dsmfm_searcher_locate_ranges.argtypes = [S, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
+                                               C.POINTER(C.c_uint64)]
+    L.dsmfm_searcher_extract.argtypes = [S, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
     L.dsmfm_searcher_enumerate.argtypes = [S, C.c_char_p, C.c_uint64, C.c_uint32, C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(C.c_uint64)]
     L.dsmfm_searcher_enumerate_fd.argtypes = [S, C.c_char_p, C.c_uint64, C.c_uint32, C.c_int, C.POINTER(C.c_uint64)]
     L.dsmfm_stream_free.argtypes = [C.POINTER(C.c_uint8)]
@@ -501,6 +508,62 @@ class Searcher:
         self._check(self._L.dsmfm_searcher_count(self._h, blob.ctypes.data, off.ctypes.data, len(patterns),
                                                  sp.ctypes.data, ep.ctypes.data))
         return sp, ep
+
+    # ---- locate / extract over the SA samples (include/dsmfm.h) ----
+    def load_samples(self, source):
+        """source: path of an .sa file, or its bytes (Builder.sa_file()).  Replaces samples attached before."""
+        if isinstance(source, (bytes, bytearray, memoryview)):
+            img = self._np.frombuffer(bytes(source), dtype=self._np.uint8)
+            self._check(self._L.dsmfm_searcher_set_samples(self._h, img.ctypes.data if img.size else None, img.size))
+        else:
+            self._check(self._L.dsmfm_searcher_load_samples(self._h, os.fsencode(source)))
+
+    def locate(self, pos):
+        """BWT positions -> (document uint32, offset in the document uint64)"""
+        np = self._np
+        pos = np.ascontiguousarray(np.asarray(pos, dtype=np.uint64))
+        doc, off = np.empty(pos.shape, dtype=np.uint32), np.empty(pos.shape, dtype=np.uint64)
+        self._check(self._L.dsmfm_searcher_locate(self._h, pos.ctypes.data, pos.size, doc.ctypes.data, off.ctypes.data))
+        return doc, off
+
+    def locate_device(self, pos, doc, offset):
+        """torch tensors on the searcher's device: int64/uint64 [count] in, int32/uint32 [count] and int64/uint64 [count] out"""
+        for t, name, dtypes in ((pos, "pos", ("torch.int64", "torch.uint64")), (doc, "doc", ("torch.int32", "torch.uint32")),
+                                (offset, "offset", ("torch.int64", "torch.uint64"))):
+            if str(t.dtype) not in dtypes or not t.is_cuda or not t.is_contiguous() or t.numel() != pos.numel():
+                raise ValueError("locate_device: %s must be a contiguous CUDA tensor of %d %s entries, got %s %s on %s"
+                                 % (name, pos.numel(), " / ".join(dtypes), tuple(t.shape), t.dtype, t.device))
+        self._check(self._L.dsmfm_searcher_locate_device(self._h, pos.data_ptr(), pos.numel(), doc.data_ptr(), offset.data_ptr()))
+
+    def locate_ranges(self, sp, ep):
+        """Every position of the intervals [sp[k], ep[k]] (sp > ep: none) -> (doc, offset, starts): interval k's
+        occurrences are doc / offset[starts[k]:starts[k+1]], in BWT order."""
+        np = self._np
+        sp = np.ascontiguousarray(np.asarray(sp, dtype=np.uint64))
+        ep = np.ascontiguousarray(np.asarray(ep, dtype=np.uint64))
+        sizes = np.where(sp <= ep, ep - sp + np.uint64(1), np.uint64(0))
+        starts = np.zeros(sp.size + 1, dtype=np.uint64)
+        starts[1:] = np.cumsum(sizes, dtype=np.uint64)
+        cap = int(starts[-1])
+        doc, off = np.empty(cap, dtype=np.uint32), np.empty(cap, dtype=np.uint64)
+        total = C.c_uint64()
+        self._check(self._L.dsmfm_searcher_locate_ranges(self._h, sp.ctypes.data, ep.ctypes.data, sp.size, cap, doc.ctypes.data,
+                                                         off.ctypes.data, C.byref(total)))
+        return doc, off, starts
+
+    def extract(self, docs):
+        """Document ids -> list of their bytes (without terminator)."""
+        np = self._np
+        docs = np.ascontiguousarray(np.asarray(docs, dtype=np.uint32))
+        offsets = np.empty(docs.size + 1, dtype=np.uint64)
+        rc = self._L.dsmfm_searcher_extract(self._h, docs.ctypes.data, docs.size, None, 0, offsets.ctypes.data)
+        if rc != ELIMIT:
+            self._check(rc)
+        out = np.empty(int(offsets[-1]), dtype=np.uint8)
+        self._check(self._L.dsmfm_searcher_extract(self._h, docs.ctypes.data, docs.size, out.ctypes.data, out.size,
+                                                   offsets.ctypes.data))
+        blob = out.tobytes()
+        return [blob[offsets[k]:offsets[k + 1]] for k in range(docs.size)]
 
     def enumerate(self, enforce_path, fmin=10, maxdepth=0):
         """EnumerateQuery::enumerate: the client's byte stream (without the handshake) for the trie below enforce_path."""

@@ -423,6 +423,27 @@ DSMFM_API int dsmfm_searcher_extend(dsmfm_searcher *s, const uint64_t *sp, const
  * the interval of all suffixes: [sp, ep] of its occurrences, sp > ep if there are none */
 DSMFM_API int dsmfm_searcher_count(dsmfm_searcher *s, const uint8_t *patterns, const uint64_t *offsets, uint64_t count,
                                    uint64_t *sp_out, uint64_t *ep_out);
+/* ---- locate / extract over the SA samples (FMIndex::loadSamples, locate and getSuffix of the reference's FMIndex) ----
+ * A position is resolved by LF steps to the left until its suffix is sampled or starts a document (at most
+ * sample rate - 1 steps).  The sample tables stay in HBM bit-packed, as the .sa file holds them.  Calling any of
+ * the entry points below before samples are attached returns DSMFM_EINVAL; so do a position >= n, a document >= D,
+ * and samples whose walks do not end within the longest document (an .sa file of another index).  Every call runs
+ * on the searcher's stream and synchronises it. */
+/* Attach the SA samples of THIS index: a `.sa` file (dsmfm_write_sa, or the reference's FMIndex::saveSamples),
+ * or its bytes in memory (dsmfm_sa_serialize).  Replaces samples attached before. */
+DSMFM_API int dsmfm_searcher_load_samples(dsmfm_searcher *s, const char *sa_path);
+DSMFM_API int dsmfm_searcher_set_samples(dsmfm_searcher *s, const uint8_t *image, uint64_t bytes);
+/* doc[k], offset[k] of the suffix at BWT position pos[k] (pos[k] < n) */
+DSMFM_API int dsmfm_searcher_locate(dsmfm_searcher *s, const uint64_t *pos, uint64_t count, uint32_t *doc, uint64_t *offset);
+DSMFM_API int dsmfm_searcher_locate_device(dsmfm_searcher *s, const void *pos_dev, uint64_t count, void *doc_dev, void *offset_dev);
+/* every position of the intervals [sp[k], ep[k]] as dsmfm_searcher_count returns them (sp > ep: none); *total = their
+ * number; total > cap -> DSMFM_ELIMIT and nothing but *total written */
+DSMFM_API int dsmfm_searcher_locate_ranges(dsmfm_searcher *s, const uint64_t *sp, const uint64_t *ep, uint64_t count,
+                                           uint64_t cap, uint32_t *doc, uint64_t *offset, uint64_t *total);
+/* documents docs[k] (without terminator) at out[offsets[k] .. offsets[k+1]); offsets[0..count] always written;
+ * offsets[count] > cap -> DSMFM_ELIMIT */
+DSMFM_API int dsmfm_searcher_extract(dsmfm_searcher *s, const uint32_t *docs, uint64_t count, uint8_t *out, uint64_t cap,
+                                     uint64_t *offsets);
 /* Replaces: EnumerateQuery::enumerate (EnumerateQuery.cpp:9-37) with nextEnforced / nextSymbol (151-290), pushChar /
  * leftChar (39-103) and the encoding of ClientSocket::putc / putulong (ClientSocket.h:12-39) -- the mining client's
  * walk of the trie of all substrings that occur at least fmin times below `enforce_path`, SURVEY 8(f) row 4.  The
