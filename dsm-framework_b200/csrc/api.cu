@@ -415,8 +415,8 @@ size_t wavelet_fill_bits(cudaStream_t st, const uint8_t *d_seq, uint64_t n, cons
     const int m = shape.n_internal;
     if (m == 0 || n == 0) return 0;
     const uint64_t ntiles = div_up(n, kWtTile);
-    static const bool no_sweep = std::getenv("DSMFM_WT_SWEEP") && std::atoi(std::getenv("DSMFM_WT_SWEEP")) == 0;
-    const bool sweep = wt_sweep_ok(m) && !no_sweep; // one pass (small trees) or count / scan / fill
+    const char *sweep_env = std::getenv("DSMFM_WT_SWEEP"); // 0: count / scan / fill for small trees too (read per call: the tests switch it)
+    const bool sweep = wt_sweep_ok(m) && !(sweep_env && std::atoi(sweep_env) == 0); // one pass (small trees) or count / scan / fill
     const size_t tile_bytes = sizeof(uint64_t) * (sweep ? wt_sweep_status_words(ntiles) + 1 : (size_t)m * ntiles);
     uint8_t *d_info = static_cast<uint8_t *>(dev_alloc((size_t)m * 256, st));
     uint64_t *d_tile = static_cast<uint64_t *>(dev_alloc(tile_bytes, st));
@@ -1234,7 +1234,7 @@ void dsmfm_builder::build()
     if (!sharded && !host_prefetch.joinable()) {
         dsmfm_code tab[256];
         WaveletResult probe;
-        if (build_codetable(counts, tab) <= 31) {
+        if (build_codetable(counts, tab) <= 32) {
             wavelet_prepare(tab, probe);
             if (probe.shape.n_internal > 0) {
                 const size_t want = probe.section_bytes;
@@ -1690,8 +1690,8 @@ void dsmfm_builder::build()
     index.C[0] = 0;
     for (int i = 1; i < 256; ++i) index.C[i] = index.C[i - 1] + counts[i - 1]; // FMIndex.cpp:397-409
     const uint32_t maxbits = build_codetable(counts, index.codetable);
-    if (maxbits > 31)
-        throw CudaError{cudaErrorInvalidValue, "Huffman code longer than 31 bits (the .fmi code field is 32 bits)", __FILE__, __LINE__};
+    if (maxbits > 32)
+        throw CudaError{cudaErrorInvalidValue, "Huffman code longer than 32 bits (the .fmi code field holds 32)", __FILE__, __LINE__};
     if (!sharded) {
         size_t wt_bytes = 0;
         wavelet_build_device(st, d_bwt, n, index.codetable, wt, L, &wt_bytes);
@@ -3178,8 +3178,8 @@ DSMFM_API int dsmfm_dbg_wavelet(int device, const uint8_t *seq, uint64_t n, dsmf
         d->index.samplerate = DSMFM_DEFAULT_SAMPLERATE;
         d->index.C[0] = 0;
         for (int i = 1; i < 256; ++i) d->index.C[i] = d->index.C[i - 1] + counts[i - 1];
-        if (build_codetable(counts, d->index.codetable) > 31)
-            throw CudaError{cudaErrorInvalidValue, "Huffman code longer than 31 bits", __FILE__, __LINE__};
+        if (build_codetable(counts, d->index.codetable) > 32)
+            throw CudaError{cudaErrorInvalidValue, "Huffman code longer than 32 bits (the .fmi code field holds 32)", __FILE__, __LINE__};
         wavelet_build_device(nullptr, d_seq, n, d->index.codetable, d->wt, nullptr, nullptr);
         wavelet_fetch(nullptr, d->wt);
         d->index.n_nodes = (uint32_t)d->wt.shape.nodes.size();

@@ -53,6 +53,7 @@ __device__ __forceinline__ uint64_t wt_rank(const QIndex *__restrict__ x, uint32
 {
     if (!x->present[c]) return 0;
     uint64_t cnt = i + 1; // positions considered; 0 for i = (ulong)-1
+    cnt = cnt < x->n ? cnt : x->n; // i >= n counts as n - 1 also when the root is a leaf (one symbol), not only below it
     uint32_t code = x->code[c];
     const QNode *t = &x->nodes[0];
     while (!t->leaf) {
