@@ -532,6 +532,38 @@ PiecePlan plan_pieces(const WtShape &shape, const uint64_t *hist_all, uint32_t w
     return p;
 }
 
+// One bit vector cut into contiguous per-builder ranges: this builder holds bits [o, o + c) of a vector of `nbits`
+// bits (a wavelet-tree node, or a section of the .sa file).  On the device its bits start at local bit `base` of an
+// array that begins at the superblock holding bit o (word G0 = 4 * (o / 256)), so that local superblocks are global
+// superblocks.  `dirs`: a BitRank with Rs / Rb directories; without them (a BlockArray) the words alone.  `last`: no
+// later builder has bits of the vector.  The ownership rules are those of the comment above dsmfm_pieces_build.
+struct VecPiece {
+    uint64_t o = 0, c = 0, nbits = 0;
+    bool last = false, dirs = true;
+    uint64_t G0 = 0, base = 0, nb = 0, words = 0, nsb = 0, nrb = 0;
+    uint64_t off_data = 0, off_rs = 0, off_rb = 0; // offsets of the local arrays in the builder's blob
+};
+
+VecPiece vec_layout(uint64_t o, uint64_t c, uint64_t nbits, bool last, bool dirs, size_t &blob)
+{
+    VecPiece l;
+    l.o = o;
+    l.c = c;
+    l.nbits = nbits;
+    l.last = last;
+    l.dirs = dirs;
+    l.G0 = 4 * (o / 256);
+    l.base = o - 64 * l.G0;
+    l.nb = l.base + c;
+    l.words = l.nb / 64 + 1;
+    l.nsb = dirs ? l.nb / 256 + 1 : 0;
+    l.nrb = dirs ? l.nb / 64 + 1 : 0;
+    l.off_data = blob; blob += l.words * 8;
+    l.off_rs = blob;   blob += l.nsb * 8;
+    l.off_rb = blob;   blob += align8(l.nrb);
+    return l;
+}
+
 // `ready`: a page-locked buffer of at least section_bytes acquired ahead of time (or nullptr)
 void wavelet_fetch(cudaStream_t st, WaveletResult &r, uint8_t *ready = nullptr)
 {
@@ -735,6 +767,7 @@ struct dsmfm_builder {
         d_sa_hi = nullptr;
         d_bwt = nullptr;
         d_doc_end = nullptr;
+        sah.d_doc_end = sah.d_sampled = sah.d_ends = nullptr;
         dev_now = 0;
         wt.release(stream);
     }
@@ -757,21 +790,38 @@ struct dsmfm_builder {
     struct PieceHost {
         std::vector<dsmfm_piece> piece;
         std::vector<dsmfm_piece_edge> edge;
-        std::vector<uint64_t> bit_off, bit_count; // per internal node
+        std::vector<VecPiece> vec;                // per internal node
         uint8_t *h_blob = nullptr;                // pinned
         size_t h_bytes = 0;
         uint8_t *d_blob = nullptr;                // device pieces until dsmfm_pieces_fetch
         size_t blob_bytes = 0, ch_off = 0;
         bool built = false;
-        std::vector<uint64_t> loc_G0, loc_words, off_data, off_rs, off_rb, nbits_of;
         std::vector<uint32_t> node_of;
-        std::vector<uint8_t> loc_last;
         uint32_t world = 0, rank = 0;
         bool merged = false;
         WtShape shape;
         std::vector<uint64_t> file_off_data, file_off_rs, file_off_rb, file_off_node; // per internal node / per node
         uint64_t file_bytes = 0;
     } ph;
+    // .sa samples of a packed-text build with DSMFM_FLAG_KEEP_SA (dsmfm_sa_*): what build() derives from the text and
+    // the BWT while both are there, then this builder's share of the five bit vectors of the file
+    struct SaHost {
+        bool ready = false;              // derived by build()
+        uint64_t *d_doc_end = nullptr;   // padded position of every terminator of the collection (u64, document order)
+        uint64_t *d_sampled = nullptr;   // the slice's `sampled` bits, laid out as VecPiece of (rank_begin, count)
+        uint64_t *d_ends = nullptr;      // bit p: BWT[p] == 0 (end markers of the slice), from bit 0
+        uint64_t slot_syms = 0;          // symbols per slot of the packed text
+        uint32_t world = 0;
+        dsmfm_sa_info info;
+        bool built = false, merged = false;
+        uint32_t rank = 0;
+        uint64_t samples = 0;            // of the whole collection
+        unsigned wlen = 0, wdoc = 0;
+        VecPiece vec[DSMFM_SA_VECTORS];  // sampled, suffixes, suffixDocId, textLength, Doc
+        dsmfm_piece piece[DSMFM_SA_VECTORS];
+        dsmfm_piece_edge edge[DSMFM_SA_VECTORS];
+        std::vector<uint8_t> h_blob;
+    } sah;
 
     // ---- a text that streams in from host memory (dsmfm_append_batch of a whole collection) ----
     // The copy runs in pieces on a stream of its own; while piece k+1 crosses PCIe the build stream already
@@ -811,6 +861,7 @@ struct dsmfm_builder {
     void build();
     void fetch();
     void make_sa_image();
+    void sa_derive(int bits, uint32_t *L);
 };
 
 // ---------------------------------------------------------------------------
@@ -1733,6 +1784,7 @@ void dsmfm_builder::build()
         dfree(d_last_sorted_vals);
     }
     pos_lo_bits = lo_bits;
+    if (packed_in && keep_sa) sa_derive(bits, L);
 
     float ms;
     cudaEventElapsedTime(&ms, ev[0], ev[5]); stats.ms_total = ms;
@@ -1891,10 +1943,49 @@ void dsmfm_builder::make_sa_image()
     put_block_array(out, h_emdoc.data(), D, wdoc);
 }
 
+// .sa samples of a packed-text build: what needs the replicated text or the slice's BWT is derived here, before the
+// caller releases the text (right after dsmfm_build_packed) and dsmfm_pieces_build the BWT.  Positions are positions
+// in the padded text; the document of a position and its offset follow from the document ends alone.
+void dsmfm_builder::sa_derive(int bits, uint32_t *L)
+{
+    cudaStream_t st = stream;
+    const uint64_t spw = 64 / (uint64_t)bits, n_text = ext->words * spw, D = counts[0];
+    sah = SaHost();
+    sah.slot_syms = ext->geom.slot_words * spw;
+    sah.world = ext->geom.world;
+    sah.d_doc_end = static_cast<uint64_t *>(dmalloc(D * 8 + 16));
+    uint64_t *d_tile = static_cast<uint64_t *>(dmalloc(term_tiles(n_text) * 8));
+    launch_packed_term_positions(st, bits, ext->text, n_text, ext->geom, d_tile, sah.d_doc_end, L);
+    dfree(d_tile);
+    const size_t mark_bytes = (n_text / 32 + 2) * 4;
+    uint32_t *d_mark = static_cast<uint32_t *>(dmalloc(mark_bytes));
+    DSM_CUDA(cudaMemsetAsync(d_mark, 0, mark_bytes, st));
+    launch_sa_mark64(st, sah.d_doc_end, (uint32_t)D, samplerate, sah.slot_syms, d_mark, L);
+    size_t blob = 0;
+    const VecPiece l = vec_layout(shard_rank_begin, shard_m, index.n, false, true, blob);
+    const size_t ends_bytes = (shard_m / 64 + 1) * 8;
+    sah.d_sampled = static_cast<uint64_t *>(dmalloc(l.words * 8));
+    sah.d_ends = static_cast<uint64_t *>(dmalloc(ends_bytes));
+    unsigned long long *d_cnt = static_cast<unsigned long long *>(dmalloc(16));
+    DSM_CUDA(cudaMemsetAsync(sah.d_sampled, 0, l.words * 8, st));
+    DSM_CUDA(cudaMemsetAsync(sah.d_ends, 0, ends_bytes, st));
+    DSM_CUDA(cudaMemsetAsync(d_cnt, 0, 16, st));
+    launch_sa_slice_bits(st, d_sa, d_sa_hi, pos_lo_bits, d_bwt, d_mark, shard_m, sah.d_sampled, l.base, sah.d_ends, d_cnt, L);
+    unsigned long long cnt[2] = {0, 0};
+    DSM_CUDA(cudaMemcpyAsync(cnt, d_cnt, sizeof cnt, cudaMemcpyDeviceToHost, st));
+    DSM_CUDA(cudaStreamSynchronize(st));
+    dfree(d_mark);
+    dfree(d_cnt);
+    sah.info.samples = cnt[0];
+    sah.info.ends = cnt[1];
+    sah.info.documents = block_info.documents;
+    sah.ready = true;
+}
+
 // ---------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------
-#define API_GUARD(b)                                              \
+#define API_GUARD(b)                                             \
     if (!(b)) return DSMFM_EINVAL;                                \
     cudaSetDevice((b)->device)
 
@@ -2221,8 +2312,8 @@ DSMFM_API int dsmfm_build_packed(dsmfm_builder *b, const dsmfm_text_plan *plan, 
         return b->fail(DSMFM_EINVAL, "dsmfm_build_packed: bad arguments");
     if (b->finished) return b->fail(DSMFM_EINVAL, "dsmfm_build_packed: already built");
     if (!b->sealed || b->d_raw) return b->fail(DSMFM_EINVAL, "dsmfm_build_packed: call dsmfm_block_stats and dsmfm_block_pack first");
-    if (b->flags & DSMFM_FLAG_KEEP_SA)
-        return b->fail(DSMFM_EINVAL, "dsmfm_build_packed: DSMFM_FLAG_KEEP_SA is not supported (positions are positions in the padded text)");
+    if ((b->flags & DSMFM_FLAG_KEEP_SA) && plan->documents >= (1ull << 32))
+        return b->fail(DSMFM_ELIMIT, "dsmfm_build_packed: .sa samples of 2^32 documents or more (document ids are u32)");
     if (plan->n == 0) return b->fail(DSMFM_EINVAL, "dsmfm_build_packed: empty collection (build it with dsmfm_finish on one builder)");
     uint64_t total = 0;
     for (int i = 0; i < 4096; ++i) total += top_hist4096[i];
@@ -2543,6 +2634,97 @@ bool pwrite_all(int fd, const void *p, size_t n, uint64_t off)
     }
     return true;
 }
+
+// The owned share (pc) and the edge record (ed) of one vector, from the host copy of the builder's blob.  Returns
+// the bytes owned.
+uint64_t vec_fetch(const VecPiece &l, uint8_t *h_blob, dsmfm_piece &pc, dsmfm_piece_edge &ed)
+{
+    pc = dsmfm_piece();
+    ed = dsmfm_piece_edge();
+    if (!l.c) return 0;
+    uint64_t *h_data = reinterpret_cast<uint64_t *>(h_blob + l.off_data);
+    pc.word_first = div_up(l.o, 64);
+    const uint64_t w_end = l.last ? l.nbits / 64 + 1 : div_up(l.o + l.c, 64);
+    pc.word_count = w_end > pc.word_first ? w_end - pc.word_first : 0;
+    pc.data = h_data + (pc.word_first - l.G0);
+    if (l.dirs) {
+        pc.rb_first = pc.word_first;
+        pc.rb_count = pc.word_count;
+        pc.rs_first = div_up(l.o, 256);
+        const uint64_t s_end = l.last ? l.nbits / 256 + 1 : div_up(l.o + l.c, 256);
+        pc.rs_count = s_end > pc.rs_first ? s_end - pc.rs_first : 0;
+        pc.Rb = h_blob + l.off_rb + (pc.word_first - l.G0);
+        pc.Rs = reinterpret_cast<uint64_t *>(h_blob + l.off_rs) + (pc.rs_first - l.G0 / 4);
+    }
+    ed.count = l.c;
+    ed.first_word = l.o / 64;
+    ed.last_word = (l.o + l.c - 1) / 64;
+    for (int t = 0; t < 4; ++t) {
+        const uint64_t fi = ed.first_word - l.G0 + t;
+        ed.first[t] = fi < l.words ? h_data[fi] : 0ull;
+        const int64_t li = (int64_t)(ed.last_word - l.G0) - 3 + t;
+        ed.last[t] = li >= 0 && (uint64_t)li < l.words ? h_data[li] : 0ull;
+    }
+    return pc.word_count * 8 + pc.rs_count * 8 + pc.rb_count;
+}
+
+// Completes the owned words next to the slice boundaries from the edge records of every builder
+// (edges[q * stride] is builder q's record of this vector).
+void vec_merge(const VecPiece &l, dsmfm_piece &pc, const dsmfm_piece_edge *edges, size_t stride, uint32_t world, uint32_t rank)
+{
+    if (!l.c) return;
+    // what any builder contributes to data word w (first / last windows of its record)
+    auto contribution = [&](uint32_t q, uint64_t w) -> uint64_t {
+        const dsmfm_piece_edge &e = edges[(size_t)q * stride];
+        if (!e.count) return 0ull;
+        uint64_t x = 0;
+        if (w >= e.first_word && w < e.first_word + 4) x |= e.first[w - e.first_word];
+        if (w + 3 >= e.last_word && w <= e.last_word) x |= e.last[w + 3 - e.last_word];
+        return x;
+    };
+    // (a) bits of later slices in the last owned word (and, for tiny slices, in any owned word)
+    for (uint32_t q = 0; q < world; ++q) {
+        if (q == rank) continue;
+        const dsmfm_piece_edge &e = edges[(size_t)q * stride];
+        if (!e.count) continue;
+        for (int t = 0; t < 4; ++t) {
+            const uint64_t wf = e.first_word + t;
+            if (wf >= pc.word_first && wf < pc.word_first + pc.word_count) pc.data[wf - pc.word_first] |= e.first[t];
+            if (e.last_word + t >= 3) {
+                const uint64_t wl = e.last_word - 3 + t;
+                if (wl >= pc.word_first && wl < pc.word_first + pc.word_count) pc.data[wl - pc.word_first] |= e.last[t];
+            }
+        }
+    }
+    if (!l.dirs) return;
+    // (b) Rb of the owned words whose superblock starts in front of the slice
+    const uint64_t first_full = 4 * div_up(l.o, 256); // first word of the first superblock that starts inside the slice
+    for (uint64_t k = pc.rb_first; k < pc.rb_first + pc.rb_count && k < first_full; ++k) {
+        uint32_t sum = 0;
+        for (uint64_t w = 4 * (k / 4); w < k; ++w) {
+            uint64_t x = 0;
+            if (w >= pc.word_first && w < pc.word_first + pc.word_count) {
+                x = pc.data[w - pc.word_first];
+            } else {
+                for (uint32_t q = 0; q < world; ++q) x |= contribution(q, w);
+            }
+            sum += (uint32_t)__builtin_popcountll(x);
+        }
+        pc.Rb[k - pc.rb_first] = (uint8_t)sum;
+    }
+}
+
+// pwrite of the owned share; data_off / rs_off / rb_off: file offsets of the vector's words / Rs / Rb
+bool vec_write(int fd, const VecPiece &l, const dsmfm_piece &pc, uint64_t data_off, uint64_t rs_off, uint64_t rb_off)
+{
+    if (!l.c) return true;
+    bool ok = pwrite_all(fd, pc.data, pc.word_count * 8, data_off + pc.word_first * 8);
+    if (l.dirs) {
+        ok = ok && pwrite_all(fd, pc.Rs, pc.rs_count * 8, rs_off + pc.rs_first * 8);
+        ok = ok && pwrite_all(fd, pc.Rb, pc.rb_count, rb_off + pc.rb_first);
+    }
+    return ok;
+}
 } // namespace
 
 DSMFM_API int dsmfm_pieces_fetch(dsmfm_builder *b, dsmfm_pieces *out);
@@ -2585,32 +2767,16 @@ DSMFM_API int dsmfm_pieces_build(dsmfm_builder *b, const uint64_t *hist_all, uin
         }
         ph.piece.assign(m, dsmfm_piece());
         ph.edge.assign(m, dsmfm_piece_edge());
-        ph.bit_off.assign(m, 0);
-        ph.bit_count.assign(m, 0);
-        // layout of the device pieces: node v's bits start at local bit `base` of an array that begins at the
-        // superblock holding bit o (word G0 = 4 * (o / 256)), so that local superblocks are global superblocks
-        struct Loc { uint64_t G0, base, nb, words, nsb, nrb, off_data, off_rs, off_rb, B; bool last; };
-        std::vector<Loc> loc(m);
+        ph.vec.assign(m, VecPiece());
+        std::vector<uint64_t> ones_before(m, 0);
         size_t blob = 0;
         for (int v = 0; v < m; ++v) {
-            const uint64_t o = pp.bit_off[(size_t)rank * m + v], c = pp.count[(size_t)rank * m + v];
-            ph.bit_off[v] = o;
-            ph.bit_count[v] = c;
-            Loc &l = loc[v];
-            l.G0 = 4 * (o / 256);
-            l.base = o - 64 * l.G0;
-            l.nb = l.base + c;
-            l.words = l.nb / 64 + 1;
-            l.nsb = l.nb / 256 + 1;
-            l.nrb = l.nb / 64 + 1;
-            l.B = 0;
-            for (uint32_t q = 0; q < rank; ++q) l.B += ones_of_slice(ph.shape, v, hist_all + (size_t)q * 256);
-            l.last = c > 0;
+            const uint64_t c = pp.count[(size_t)rank * m + v];
+            bool last = c > 0;
             for (uint32_t q = rank + 1; q < world; ++q)
-                if (pp.count[(size_t)q * m + v]) l.last = false;
-            l.off_data = blob; blob += l.words * 8;
-            l.off_rs = blob;   blob += l.nsb * 8;
-            l.off_rb = blob;   blob += align8(l.nrb);
+                if (pp.count[(size_t)q * m + v]) last = false;
+            ph.vec[v] = vec_layout(pp.bit_off[(size_t)rank * m + v], c, nbits_of[v], last, true, blob);
+            for (uint32_t q = 0; q < rank; ++q) ones_before[v] += ones_of_slice(ph.shape, v, hist_all + (size_t)q * 256);
         }
         const size_t blob_bytes = blob + align8((size_t)(m ? m : 1));
         uint8_t *d_blob = static_cast<uint8_t *>(b->dmalloc(blob_bytes));
@@ -2620,16 +2786,16 @@ DSMFM_API int dsmfm_pieces_build(dsmfm_builder *b, const uint64_t *hist_all, uin
         std::vector<uint64_t> base(m);
         uint64_t max_sb = 1;
         for (int v = 0; v < m; ++v) {
-            ptrs[v] = reinterpret_cast<uint64_t *>(d_blob + loc[v].off_data);
-            base[v] = loc[v].base;
-            max_sb = std::max(max_sb, loc[v].nsb);
+            ptrs[v] = reinterpret_cast<uint64_t *>(d_blob + ph.vec[v].off_data);
+            base[v] = ph.vec[v].base;
+            max_sb = std::max(max_sb, ph.vec[v].nsb);
         }
         wavelet_fill_bits(st, b->d_bwt, slice_m, ph.shape, ptrs, base, d_ch, L);
         uint64_t *d_scratch = static_cast<uint64_t *>(b->dmalloc(sizeof(uint64_t) * (div_up(max_sb, kRankChunk) + 1)));
         for (int v = 0; v < m; ++v)
-            if (ph.bit_count[v])
-                launch_bitrank(st, ptrs[v], loc[v].nb, reinterpret_cast<uint64_t *>(d_blob + loc[v].off_rs),
-                               d_blob + loc[v].off_rb, d_scratch, L, loc[v].B);
+            if (ph.vec[v].c)
+                launch_bitrank(st, ptrs[v], ph.vec[v].nb, reinterpret_cast<uint64_t *>(d_blob + ph.vec[v].off_rs),
+                               d_blob + ph.vec[v].off_rb, d_scratch, L, ones_before[v]);
         DSM_CUDA(cudaEventRecord(e1, st));
         DSM_CUDA(cudaStreamSynchronize(st));
         float ms = 0;
@@ -2643,12 +2809,7 @@ DSMFM_API int dsmfm_pieces_build(dsmfm_builder *b, const uint64_t *hist_all, uin
         ph.d_blob = d_blob;
         ph.blob_bytes = blob_bytes;
         ph.ch_off = blob;
-        ph.loc_G0.resize(m); ph.loc_words.resize(m); ph.loc_last.resize(m);
-        ph.off_data.resize(m); ph.off_rs.resize(m); ph.off_rb.resize(m); ph.nbits_of = nbits_of; ph.node_of = node_of;
-        for (int v = 0; v < m; ++v) {
-            ph.loc_G0[v] = loc[v].G0; ph.loc_words[v] = loc[v].words; ph.loc_last[v] = loc[v].last ? 1 : 0;
-            ph.off_data[v] = loc[v].off_data; ph.off_rs[v] = loc[v].off_rs; ph.off_rb[v] = loc[v].off_rb;
-        }
+        ph.node_of = node_of;
         ph.built = true;
         ph.merged = false;
         if (out) {
@@ -2692,41 +2853,9 @@ DSMFM_API int dsmfm_pieces_fetch(dsmfm_builder *b, dsmfm_pieces *out)
         }
         uint64_t held = 0;
         for (int v = 0; v < m; ++v) {
-            const uint64_t o = ph.bit_off[v], c = ph.bit_count[v], nbits = ph.nbits_of[v];
-            const uint64_t G0 = ph.loc_G0[v], words = ph.loc_words[v];
-            const bool last = ph.loc_last[v] != 0;
-            dsmfm_piece &pc = ph.piece[v];
-            dsmfm_piece_edge &ed = ph.edge[v];
-            pc = dsmfm_piece();
-            ed = dsmfm_piece_edge();
-            pc.node = ph.node_of[v];
-            uint64_t *h_data = reinterpret_cast<uint64_t *>(ph.h_blob + ph.off_data[v]);
-            uint64_t *h_rs = reinterpret_cast<uint64_t *>(ph.h_blob + ph.off_rs[v]);
-            uint8_t *h_rb = ph.h_blob + ph.off_rb[v];
-            if (c) {
-                pc.word_first = div_up(o, 64);
-                const uint64_t w_end = last ? nbits / 64 + 1 : div_up(o + c, 64);
-                pc.word_count = w_end > pc.word_first ? w_end - pc.word_first : 0;
-                pc.rb_first = pc.word_first;
-                pc.rb_count = pc.word_count;
-                pc.rs_first = div_up(o, 256);
-                const uint64_t s_end = last ? nbits / 256 + 1 : div_up(o + c, 256);
-                pc.rs_count = s_end > pc.rs_first ? s_end - pc.rs_first : 0;
-                pc.data = h_data + (pc.word_first - G0);
-                pc.Rb = h_rb + (pc.word_first - G0);
-                pc.Rs = h_rs + (pc.rs_first - G0 / 4);
-                ed.count = c;
-                ed.first_word = o / 64;
-                ed.last_word = (o + c - 1) / 64;
-                for (int t = 0; t < 4; ++t) {
-                    const uint64_t fi = ed.first_word - G0 + t;
-                    ed.first[t] = fi < words ? h_data[fi] : 0ull;
-                    const int64_t li = (int64_t)(ed.last_word - G0) - 3 + t;
-                    ed.last[t] = li >= 0 && (uint64_t)li < words ? h_data[li] : 0ull;
-                }
-                ed.ch = ph.h_blob[ph.ch_off + v];
-                held += pc.word_count * 8 + pc.rs_count * 8 + pc.rb_count;
-            }
+            held += vec_fetch(ph.vec[v], ph.h_blob, ph.piece[v], ph.edge[v]);
+            ph.piece[v].node = ph.node_of[v];
+            if (ph.vec[v].c) ph.edge[v].ch = ph.h_blob[ph.ch_off + v];
         }
         out->n_internal = (uint32_t)m;
         out->world = ph.world;
@@ -2750,50 +2879,7 @@ DSMFM_API int dsmfm_pieces_merge(dsmfm_builder *b, const dsmfm_piece_edge *edges
     if (!ph.h_blob || world != ph.world) return b->fail(DSMFM_EINVAL, "dsmfm_pieces_merge: call dsmfm_pieces_build / dsmfm_pieces_fetch first (same world)");
     if (ph.merged) return b->fail(DSMFM_EINVAL, "dsmfm_pieces_merge: already merged");
     const int m = ph.shape.n_internal;
-    const uint32_t rank = ph.rank;
-    for (int v = 0; v < m; ++v) {
-        // what any builder contributes to data word w of node v (first / last windows of its record)
-        auto contribution = [&](uint32_t q, uint64_t w) -> uint64_t {
-            const dsmfm_piece_edge &e = edges_all[(size_t)q * m + v];
-            if (!e.count) return 0ull;
-            uint64_t x = 0;
-            if (w >= e.first_word && w < e.first_word + 4) x |= e.first[w - e.first_word];
-            if (w + 3 >= e.last_word && w <= e.last_word) x |= e.last[w + 3 - e.last_word];
-            return x;
-        };
-        dsmfm_piece &pc = ph.piece[v];
-        if (!ph.bit_count[v]) continue;
-        // (a) bits of later slices in the last owned word (and, for tiny slices, in any owned word)
-        for (uint32_t q = 0; q < world; ++q) {
-            if (q == rank) continue;
-            const dsmfm_piece_edge &e = edges_all[(size_t)q * m + v];
-            if (!e.count) continue;
-            for (int t = 0; t < 4; ++t) {
-                const uint64_t wf = e.first_word + t;
-                if (wf >= pc.word_first && wf < pc.word_first + pc.word_count) pc.data[wf - pc.word_first] |= e.first[t];
-                if (e.last_word + t >= 3) {
-                    const uint64_t wl = e.last_word - 3 + t;
-                    if (wl >= pc.word_first && wl < pc.word_first + pc.word_count) pc.data[wl - pc.word_first] |= e.last[t];
-                }
-            }
-        }
-        // (b) Rb of the owned words whose superblock starts in front of the slice
-        const uint64_t o = ph.bit_off[v];
-        const uint64_t first_full = 4 * div_up(o, 256); // first word of the first superblock that starts inside the slice
-        for (uint64_t k = pc.rb_first; k < pc.rb_first + pc.rb_count && k < first_full; ++k) {
-            uint32_t sum = 0;
-            for (uint64_t w = 4 * (k / 4); w < k; ++w) {
-                uint64_t x = 0;
-                if (w >= pc.word_first && w < pc.word_first + pc.word_count) {
-                    x = pc.data[w - pc.word_first];
-                } else {
-                    for (uint32_t q = 0; q < world; ++q) x |= contribution(q, w);
-                }
-                sum += (uint32_t)__builtin_popcountll(x);
-            }
-            pc.Rb[k - pc.rb_first] = (uint8_t)sum;
-        }
-    }
+    for (int v = 0; v < m; ++v) vec_merge(ph.vec[v], ph.piece[v], edges_all + v, (size_t)m, world, ph.rank);
     // node symbols (every builder fills the whole table: the one that writes the header needs it)
     for (size_t i = 0; i < ph.shape.nodes.size(); ++i) {
         const int v = ph.shape.internal_of_node[i];
@@ -2834,13 +2920,7 @@ DSMFM_API int dsmfm_pieces_write(dsmfm_builder *b, const char *path_prefix, int 
     fmi_layout(ph.shape, node_off, data_off, rs_off, rb_off, tail_off, total);
     bool ok = true;
     const int m = ph.shape.n_internal;
-    for (int v = 0; v < m && ok; ++v) {
-        const dsmfm_piece &pc = ph.piece[v];
-        if (!ph.bit_count[v]) continue;
-        ok = ok && pwrite_all(fd, pc.data, pc.word_count * 8, data_off[v] + pc.word_first * 8);
-        ok = ok && pwrite_all(fd, pc.Rs, pc.rs_count * 8, rs_off[v] + pc.rs_first * 8);
-        ok = ok && pwrite_all(fd, pc.Rb, pc.rb_count, rb_off[v] + pc.rb_first);
-    }
+    for (int v = 0; v < m && ok; ++v) ok = vec_write(fd, ph.vec[v], ph.piece[v], data_off[v], rs_off[v], rb_off[v]);
     if (header && ok) {
         std::vector<uint8_t> h;
         auto put = [&h](const void *p, size_t n) {
@@ -2888,6 +2968,195 @@ DSMFM_API int dsmfm_pieces_write(dsmfm_builder *b, const char *path_prefix, int 
     }
     ok = (::close(fd) == 0) && ok;
     return ok ? DSMFM_OK : b->fail(DSMFM_EIO, "dsmfm_pieces_write: write error on %s", name.c_str());
+}
+
+// ---- .sa samples of a packed-text build (include/dsmfm.h, steps 8-11) ----
+// The five vectors of FMIndex::saveSamples (FMIndex.cpp:134-143) and this builder's range of each, in bits:
+//   sampled      n bits            [rank_begin, + count)        directories, ones in front: samples of earlier slices
+//   suffixes     S * wlen          [S_<r * wlen, + s_r * wlen)  S = samples; S_<r, s_r: of earlier slices / this one
+//   suffixDocId  S * wdoc          [S_<r * wdoc, + s_r * wdoc)
+//   textLength   D * wlen          documents of this block
+//   Doc          D * wdoc          [Z_<r * wdoc, + z_r * wdoc)  Z_<r, z_r: end markers of earlier slices / this one
+namespace {
+enum { kSaSampled, kSaSuffixes, kSaDocId, kSaTextLength, kSaDoc };
+
+struct SaFileLayout {
+    uint64_t data[DSMFM_SA_VECTORS], rs, rb, hdr[DSMFM_SA_VECTORS], total;
+};
+
+// offsets in the .sa file (dsmfm_builder::make_sa_image): BitRank header and arrays, then four BlockArrays of
+// 16 header bytes and count * width / 64 + 1 words each
+SaFileLayout sa_file_layout(uint64_t n, uint64_t S, uint64_t D, unsigned wlen, unsigned wdoc)
+{
+    SaFileLayout f;
+    f.hdr[kSaSampled] = 0;
+    f.data[kSaSampled] = 24;
+    f.rs = f.data[kSaSampled] + (n / 64 + 1) * 8;
+    f.rb = f.rs + (n / 256 + 1) * 8;
+    uint64_t p = f.rb + n / 64 + 1;
+    const uint64_t count[DSMFM_SA_VECTORS] = {0, S, S, D, D};
+    const unsigned width[DSMFM_SA_VECTORS] = {0, wlen, wdoc, wlen, wdoc};
+    for (int i = 1; i < DSMFM_SA_VECTORS; ++i) {
+        f.hdr[i] = p;
+        f.data[i] = p + 16;
+        p += 16 + (count[i] * width[i] / 64 + 1) * 8;
+    }
+    f.total = p;
+    return f;
+}
+} // namespace
+
+DSMFM_API int dsmfm_sa_slice_info(dsmfm_builder *b, dsmfm_sa_info *out)
+{
+    if (!b || !out) return DSMFM_EINVAL;
+    if (!b->sah.ready)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_slice_info: needs dsmfm_build_packed on a builder with DSMFM_FLAG_KEEP_SA");
+    *out = b->sah.info;
+    return DSMFM_OK;
+}
+
+DSMFM_API int dsmfm_sa_pieces_build(dsmfm_builder *b, const dsmfm_sa_info *infos_all, uint32_t world, uint32_t rank,
+                                    dsmfm_piece_edge *edges_out)
+{
+    API_GUARD(b);
+    auto &sa = b->sah;
+    if (!sa.ready)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: needs dsmfm_build_packed on a builder with DSMFM_FLAG_KEEP_SA");
+    if (sa.built) return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: already built");
+    if (!infos_all || !edges_out) return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: bad arguments");
+    if (world != sa.world || rank >= world)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: world %u / rank %u, the build has %u blocks", world, rank, sa.world);
+    const dsmfm_sa_info &me = infos_all[rank];
+    if (me.samples != sa.info.samples || me.ends != sa.info.ends || me.documents != sa.info.documents)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: record %u is not this builder's", rank);
+    const uint64_t n = b->index.n, D = b->index.number_of_texts;
+    uint64_t S = 0, S_before = 0, Z_before = 0, D_before = 0, docs = 0, ends = 0;
+    for (uint32_t q = 0; q < world; ++q) {
+        if (q < rank) {
+            S_before += infos_all[q].samples;
+            Z_before += infos_all[q].ends;
+            D_before += infos_all[q].documents;
+        }
+        S += infos_all[q].samples;
+        docs += infos_all[q].documents;
+        ends += infos_all[q].ends;
+    }
+    if (docs != D || ends != D)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_build: the records hold %llu documents and %llu end markers, the collection %llu",
+                       (unsigned long long)docs, (unsigned long long)ends, (unsigned long long)D);
+    try {
+        cudaStream_t st = b->stream;
+        uint32_t *L = &b->stats.kernel_launches;
+        const unsigned wlen = ceil_log2(b->index.max_text_length), wdoc = ceil_log2(D);
+        const uint64_t s_r = sa.info.samples, z_r = sa.info.ends, d_r = sa.info.documents, m = b->shard_m;
+        // each vector: (bit offset, bit count, total bits) of this builder; the last builder with bits owns the tail
+        const uint64_t o[DSMFM_SA_VECTORS] = {b->shard_rank_begin, S_before * wlen, S_before * wdoc, D_before * wlen, Z_before * wdoc};
+        const uint64_t c[DSMFM_SA_VECTORS] = {m, s_r * wlen, s_r * wdoc, d_r * wlen, z_r * wdoc};
+        const uint64_t total[DSMFM_SA_VECTORS] = {n, S * wlen, S * wdoc, D * wlen, D * wdoc};
+        size_t blob = 0;
+        for (int i = 0; i < DSMFM_SA_VECTORS; ++i) {
+            const bool last = c[i] > 0 && o[i] + c[i] == total[i];
+            sa.vec[i] = vec_layout(o[i], c[i], total[i], last, i == kSaSampled, blob);
+        }
+        uint8_t *d_blob = static_cast<uint8_t *>(b->dmalloc(blob));
+        DSM_CUDA(cudaMemsetAsync(d_blob, 0, blob, st));
+        auto data = [&](int i) { return reinterpret_cast<uint64_t *>(d_blob + sa.vec[i].off_data); };
+        const VecPiece &vs = sa.vec[kSaSampled];
+        DSM_CUDA(cudaMemcpyAsync(data(kSaSampled), sa.d_sampled, vs.words * 8, cudaMemcpyDeviceToDevice, st));
+        // directories of `sampled` (final: the samples of earlier slices in front) and, local, of the end markers
+        const uint64_t ends_sb = m / 256 + 1;
+        uint64_t *d_ends_rs = static_cast<uint64_t *>(b->dmalloc(ends_sb * 8));
+        uint8_t *d_ends_rb = static_cast<uint8_t *>(b->dmalloc(m / 64 + 1 + 8));
+        uint64_t *d_scratch =
+            static_cast<uint64_t *>(b->dmalloc(sizeof(uint64_t) * (div_up(std::max(vs.nsb, ends_sb), kRankChunk) + 1)));
+        const uint64_t *sampled_rs = reinterpret_cast<const uint64_t *>(d_blob + vs.off_rs);
+        const uint8_t *sampled_rb = d_blob + vs.off_rb;
+        if (m) {
+            launch_bitrank(st, data(kSaSampled), vs.nb, reinterpret_cast<uint64_t *>(d_blob + vs.off_rs), d_blob + vs.off_rb,
+                           d_scratch, L, S_before);
+            launch_bitrank(st, sa.d_ends, m, d_ends_rs, d_ends_rb, d_scratch, L, 0);
+        }
+        // the fields: offset and document of every sample, document of every end marker, length of every document
+        launch_sa_emit64(st, b->d_sa, b->d_sa_hi, b->pos_lo_bits, data(kSaSampled), sampled_rs, sampled_rb, vs.base, S_before,
+                         m, sa.d_doc_end, (uint32_t)D, sa.slot_syms, data(kSaDocId), sa.vec[kSaDocId].base, wdoc,
+                         data(kSaSuffixes), sa.vec[kSaSuffixes].base, wlen, L);
+        launch_sa_emit64(st, b->d_sa, b->d_sa_hi, b->pos_lo_bits, sa.d_ends, d_ends_rs, d_ends_rb, 0, 0, m, sa.d_doc_end,
+                         (uint32_t)D, sa.slot_syms, data(kSaDoc), sa.vec[kSaDoc].base, wdoc, nullptr, 0, 0, L);
+        launch_sa_lengths(st, sa.d_doc_end, D_before, d_r, sa.slot_syms, data(kSaTextLength), sa.vec[kSaTextLength].base,
+                          wlen, L);
+        sa.h_blob.resize(blob);
+        DSM_CUDA(cudaMemcpyAsync(sa.h_blob.data(), d_blob, blob, cudaMemcpyDeviceToHost, st));
+        DSM_CUDA(cudaStreamSynchronize(st));
+        for (void *p : {(void *)d_blob, (void *)d_ends_rs, (void *)d_ends_rb, (void *)d_scratch, (void *)sa.d_sampled,
+                        (void *)sa.d_ends, (void *)sa.d_doc_end, (void *)b->d_sa, (void *)b->d_sa_hi})
+            b->dfree(p);
+        sa.d_sampled = sa.d_ends = sa.d_doc_end = nullptr;
+        b->d_sa = nullptr;
+        b->d_sa_hi = nullptr;
+        for (int i = 0; i < DSMFM_SA_VECTORS; ++i) {
+            vec_fetch(sa.vec[i], sa.h_blob.data(), sa.piece[i], sa.edge[i]);
+            edges_out[i] = sa.edge[i];
+        }
+        sa.rank = rank;
+        sa.samples = S;
+        sa.wlen = wlen;
+        sa.wdoc = wdoc;
+        sa.built = true;
+    } catch (const CudaError &e) {
+        return b->fail_cuda(e);
+    } catch (const std::bad_alloc &) {
+        return b->fail(DSMFM_ENOMEM, "host allocation failed");
+    }
+    return DSMFM_OK;
+}
+
+DSMFM_API int dsmfm_sa_pieces_merge(dsmfm_builder *b, const dsmfm_piece_edge *edges_all, uint32_t world)
+{
+    if (!b || !edges_all) return DSMFM_EINVAL;
+    auto &sa = b->sah;
+    if (!sa.built || world != sa.world)
+        return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_merge: call dsmfm_sa_pieces_build first (same world)");
+    if (sa.merged) return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_merge: already merged");
+    for (int i = 0; i < DSMFM_SA_VECTORS; ++i) vec_merge(sa.vec[i], sa.piece[i], edges_all + i, DSMFM_SA_VECTORS, world, sa.rank);
+    sa.merged = true;
+    return DSMFM_OK;
+}
+
+DSMFM_API int dsmfm_sa_pieces_write(dsmfm_builder *b, const char *path_prefix, int header)
+{
+    if (!b || !path_prefix) return DSMFM_EINVAL;
+    auto &sa = b->sah;
+    if (!sa.merged) return b->fail(DSMFM_EINVAL, "dsmfm_sa_pieces_write: call dsmfm_sa_pieces_merge first");
+    const std::string name = std::string(path_prefix) + ".sa"; // FMIndex.cpp:131
+    const int fd = ::open(name.c_str(), O_WRONLY | O_CREAT, 0644);
+    if (fd < 0) return b->fail(DSMFM_EIO, "dsmfm_sa_pieces_write: can not open %s", name.c_str());
+    const uint64_t n = b->index.n, D = b->index.number_of_texts;
+    const SaFileLayout f = sa_file_layout(n, sa.samples, D, sa.wlen, sa.wdoc);
+    bool ok = true;
+    for (int i = 0; i < DSMFM_SA_VECTORS && ok; ++i)
+        ok = vec_write(fd, sa.vec[i], sa.piece[i], f.data[i], f.rs, f.rb);
+    if (header && ok) {
+        const uint64_t integers = n / 64 + 1; // BitRank::integers = ceil((n+1)/64)
+        const uint32_t b64 = 64, s256 = 256;
+        uint8_t h[24];
+        std::memcpy(h, &n, 8);
+        std::memcpy(h + 8, &integers, 8);
+        std::memcpy(h + 16, &b64, 4);
+        std::memcpy(h + 20, &s256, 4);
+        ok = pwrite_all(fd, h, sizeof h, 0);
+        const uint64_t count[DSMFM_SA_VECTORS] = {0, sa.samples, sa.samples, D, D};
+        const uint64_t width[DSMFM_SA_VECTORS] = {0, sa.wlen, sa.wdoc, sa.wlen, sa.wdoc};
+        const uint64_t zero = 0;
+        for (int i = 1; i < DSMFM_SA_VECTORS && ok; ++i) {
+            const uint64_t bh[2] = {count[i], width[i]}; // BlockArray::Save (BlockArray.h:54-64)
+            ok = pwrite_all(fd, bh, sizeof bh, f.hdr[i]);
+            // a vector without bits is its one zero word, which no builder owns
+            if (ok && count[i] * width[i] == 0) ok = pwrite_all(fd, &zero, 8, f.data[i]);
+        }
+        ok = ok && ::ftruncate(fd, (off_t)f.total) == 0;
+    }
+    ok = (::close(fd) == 0) && ok;
+    return ok ? DSMFM_OK : b->fail(DSMFM_EIO, "dsmfm_sa_pieces_write: write error on %s", name.c_str());
 }
 
 DSMFM_API int dsmfm_fetch(dsmfm_builder *b, dsmfm_index *out)

@@ -2144,6 +2144,168 @@ __global__ void __launch_bounds__(256) sa_emit_kernel(const uint32_t *__restrict
     }
 }
 
+// ---- the same over one slice of a packed-text build: u64 positions in the padded text ----
+// Slot s holds geom.bytes[s] real symbols from position s * slot_syms on, then code-0 padding that must not read as
+// terminators.  slot_syms is a multiple of 16 (whole 16-word lines of slots), so the 16 positions of one thread lie
+// in one slot.
+template <int BITS>
+__device__ __forceinline__ uint32_t packed_term_mask(const uint64_t *__restrict__ packed, uint64_t n_text, const SelGeom &g,
+                                                     uint64_t p0)
+{
+    using P = Pack<BITS>;
+    const uint64_t slot_syms = g.slot_words * P::SPW;
+    if (p0 >= n_text) return 0;
+    const uint64_t s = p0 / slot_syms, in = p0 - s * slot_syms;
+    const uint64_t real = g.bytes[s] > in ? g.bytes[s] - in : 0;
+    uint32_t mask = 0;
+    for (int j = 0; j < 16 && (uint64_t)j < real; ++j)
+        if (text_symbol<BITS>(packed, p0 + j) == 0) mask |= 1u << j;
+    return mask;
+}
+
+template <int BITS>
+__global__ void __launch_bounds__(256) packed_term_count_kernel(const uint64_t *__restrict__ packed, uint64_t n_text,
+                                                                const SelGeom g, uint64_t *__restrict__ tile_count)
+{
+    __shared__ uint32_t s_sum[8];
+    const uint64_t p0 = (uint64_t)blockIdx.x * kTermTile + (uint64_t)threadIdx.x * 16;
+    uint32_t c = (uint32_t)__popc(packed_term_mask<BITS>(packed, n_text, g, p0));
+    c = warp_sum(c);
+    if ((threadIdx.x & 31) == 0) s_sum[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t t = 0;
+        for (int k = 0; k < 8; ++k) t += s_sum[k];
+        tile_count[blockIdx.x] = t;
+    }
+}
+
+template <int BITS>
+__global__ void __launch_bounds__(256) packed_term_write_kernel(const uint64_t *__restrict__ packed, uint64_t n_text,
+                                                                const SelGeom g, const uint64_t *__restrict__ tile_off,
+                                                                uint64_t *__restrict__ doc_end)
+{
+    __shared__ uint32_t scratch[9];
+    const uint64_t p0 = (uint64_t)blockIdx.x * kTermTile + (uint64_t)threadIdx.x * 16;
+    uint32_t mask = packed_term_mask<BITS>(packed, n_text, g, p0);
+    uint32_t total;
+    uint64_t o = tile_off[blockIdx.x] + block_excl_sum((uint32_t)__popc(mask), scratch, &total);
+    while (mask) {
+        const int j = __ffs(mask) - 1;
+        mask &= mask - 1;
+        doc_end[o++] = p0 + j;
+    }
+}
+
+// first position of document k: one past the previous terminator, or the first symbol of k's slot
+__device__ __forceinline__ uint64_t padded_doc_start(const uint64_t *__restrict__ doc_end, uint64_t k, uint64_t slot_syms)
+{
+    const uint64_t e = doc_end[k], slot_begin = e - e % slot_syms;
+    const uint64_t after_prev = k ? doc_end[k - 1] + 1 : 0;
+    return after_prev > slot_begin ? after_prev : slot_begin;
+}
+
+// sa_mark_kernel on padded positions
+__global__ void __launch_bounds__(256) sa_mark64_kernel(const uint64_t *__restrict__ doc_end, uint32_t ndocs, uint32_t rate,
+                                                        uint64_t slot_syms, uint32_t *__restrict__ mark)
+{
+    const uint64_t k = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (k >= ndocs) return;
+    const uint64_t e = doc_end[k], s = padded_doc_start(doc_end, k, slot_syms);
+    for (uint64_t d = rate; d <= e - s; d += rate) { // i = e - d >= s
+        const uint64_t x = e - d + 1;
+        atomicOr(&mark[x >> 5], 1u << (x & 31));
+    }
+}
+
+__device__ __forceinline__ uint64_t slice_position(const uint32_t *__restrict__ sa, const uint8_t *__restrict__ hi, int lo_bits,
+                                                   uint64_t p)
+{
+    return hi ? ((uint64_t)hi[p] << lo_bits) | sa[p] : (uint64_t)sa[p];
+}
+
+__global__ void __launch_bounds__(256) sa_slice_bits_kernel(const uint32_t *__restrict__ sa, const uint8_t *__restrict__ hi,
+                                                            int lo_bits, const uint8_t *__restrict__ bwt,
+                                                            const uint32_t *__restrict__ mark, uint64_t m,
+                                                            uint32_t *__restrict__ sampled, uint64_t sampled_base,
+                                                            uint32_t *__restrict__ ends, unsigned long long *__restrict__ counts)
+{
+    const int lane = threadIdx.x & 31;
+    const uint64_t warps = (uint64_t)gridDim.x * 8, out_words = (m + 31) / 32;
+    const uint64_t w0 = sampled_base >> 5;
+    const int sh = (int)(sampled_base & 31);
+    uint32_t n_s = 0, n_e = 0;
+    for (uint64_t w = (uint64_t)blockIdx.x * 8 + (threadIdx.x >> 5); w < out_words; w += warps) {
+        const uint64_t p = w * 32 + lane;
+        bool bs = false, be = false;
+        if (p < m) {
+            const uint64_t x = slice_position(sa, hi, lo_bits, p);
+            bs = (mark[x >> 5] >> (x & 31)) & 1u;
+            be = bwt[p] == 0;
+        }
+        const uint32_t ws = __ballot_sync(0xffffffffu, bs), we = __ballot_sync(0xffffffffu, be);
+        if (lane == 0) {
+            ends[w] = we;
+            // neighbouring warps share the boundary words of the shifted slice
+            if (ws) {
+                atomicOr(&sampled[w0 + w], ws << sh);
+                if (sh && (ws >> (32 - sh))) atomicOr(&sampled[w0 + w + 1], ws >> (32 - sh));
+            }
+            n_s += (uint32_t)__popc(ws);
+            n_e += (uint32_t)__popc(we);
+        }
+    }
+    if (lane == 0) {
+        if (n_s) atomicAdd(&counts[0], (unsigned long long)n_s);
+        if (n_e) atomicAdd(&counts[1], (unsigned long long)n_e);
+    }
+}
+
+// ORs a w-bit field (w <= 64) into a zeroed bit array, LSB first (Tools.h:49-61)
+__device__ __forceinline__ void or_field(uint64_t *__restrict__ a, uint64_t bit, unsigned w, uint64_t v)
+{
+    if (w == 0) return;
+    unsigned long long *p = reinterpret_cast<unsigned long long *>(a) + (bit >> 6);
+    const unsigned sh = (unsigned)(bit & 63);
+    atomicOr(p, (unsigned long long)(v << sh));
+    if (sh + w > 64) atomicOr(p + 1, (unsigned long long)(v >> (64 - sh)));
+}
+
+__global__ void __launch_bounds__(256) sa_emit64_kernel(const uint32_t *__restrict__ sa, const uint8_t *__restrict__ hi,
+                                                        int lo_bits, const uint64_t *__restrict__ bits,
+                                                        const uint64_t *__restrict__ Rs, const uint8_t *__restrict__ Rb,
+                                                        uint64_t bits_base, uint64_t rank_sub, uint64_t m,
+                                                        const uint64_t *__restrict__ doc_end, uint32_t ndocs, uint64_t slot_syms,
+                                                        uint64_t *__restrict__ doc_out, uint64_t doc_bit0, unsigned doc_w,
+                                                        uint64_t *__restrict__ off_out, uint64_t off_bit0, unsigned off_w)
+{
+    const uint64_t stride = (uint64_t)gridDim.x * 256;
+    for (uint64_t p = (uint64_t)blockIdx.x * 256 + threadIdx.x; p < m; p += stride) {
+        const uint64_t q = bits_base + p, word = bits[q >> 6];
+        if (!((word >> (q & 63)) & 1ull)) continue;
+        const uint64_t j = Rs[q >> 8] + Rb[q >> 6] + __popcll(word & ((1ull << (q & 63)) - 1)) - rank_sub;
+        const uint64_t x = slice_position(sa, hi, lo_bits, p);
+        uint32_t lo = 0, hi_d = ndocs - 1; // first document whose end marker is at or after x
+        while (lo < hi_d) {
+            const uint32_t mid = lo + (hi_d - lo) / 2;
+            if (doc_end[mid] >= x) hi_d = mid; else lo = mid + 1;
+        }
+        or_field(doc_out, doc_bit0 + j * doc_w, doc_w, lo);
+        if (off_out) or_field(off_out, off_bit0 + j * off_w, off_w, x - padded_doc_start(doc_end, lo, slot_syms));
+    }
+}
+
+__global__ void __launch_bounds__(256) sa_lengths_kernel(const uint64_t *__restrict__ doc_end, uint64_t first, uint64_t count,
+                                                         uint64_t slot_syms, uint64_t *__restrict__ out, uint64_t bit0,
+                                                         unsigned w)
+{
+    const uint64_t stride = (uint64_t)gridDim.x * 256;
+    for (uint64_t k = (uint64_t)blockIdx.x * 256 + threadIdx.x; k < count; k += stride) {
+        const uint64_t g = first + k;
+        or_field(out, bit0 + k * w, w, doc_end[g] - padded_doc_start(doc_end, g, slot_syms));
+    }
+}
+
 // ---------------------------------------------------------------------------
 // wavelet tree
 // ---------------------------------------------------------------------------
@@ -3145,6 +3307,64 @@ void launch_sa_emit(cudaStream_t st, const uint32_t *sa, const uint64_t *bits, c
                     uint32_t *launches)
 {
     sa_emit_kernel<<<grid_for(n, 256 * 8), 256, 0, st>>>(sa, bits, Rs, Rb, n, doc_end, ndocs, out_doc, out_off);
+    DSM_LAUNCH_CHECK();
+    if (launches) ++*launches;
+}
+
+void launch_packed_term_positions(cudaStream_t st, int bits, const uint64_t *packed, uint64_t n_text, const SelGeom &geom,
+                                  uint64_t *tile_scratch, uint64_t *doc_end, uint32_t *launches)
+{
+    const unsigned tiles = (unsigned)term_tiles(n_text);
+#define CALL(B) packed_term_count_kernel<B><<<tiles, 256, 0, st>>>(packed, n_text, geom, tile_scratch)
+    DISPATCH_BITS(bits, CALL);
+#undef CALL
+    DSM_LAUNCH_CHECK();
+    launch_wt_scan(st, tile_scratch, 1, tiles, launches);
+#define CALL(B) packed_term_write_kernel<B><<<tiles, 256, 0, st>>>(packed, n_text, geom, tile_scratch, doc_end)
+    DISPATCH_BITS(bits, CALL);
+#undef CALL
+    DSM_LAUNCH_CHECK();
+    if (launches) *launches += 2;
+}
+
+void launch_sa_mark64(cudaStream_t st, const uint64_t *doc_end, uint32_t ndocs, uint32_t rate, uint64_t slot_syms,
+                      uint32_t *mark, uint32_t *launches)
+{
+    if (ndocs == 0) return;
+    sa_mark64_kernel<<<(unsigned)div_up(ndocs, 256), 256, 0, st>>>(doc_end, ndocs, rate, slot_syms, mark);
+    DSM_LAUNCH_CHECK();
+    if (launches) ++*launches;
+}
+
+void launch_sa_slice_bits(cudaStream_t st, const uint32_t *sa, const uint8_t *hi, int lo_bits, const uint8_t *bwt,
+                          const uint32_t *mark, uint64_t m, uint64_t *sampled, uint64_t sampled_base, uint64_t *ends,
+                          unsigned long long *counts, uint32_t *launches)
+{
+    if (m == 0) return;
+    sa_slice_bits_kernel<<<grid_for(div_up(m, 32), 8 * 4), 256, 0, st>>>(sa, hi, lo_bits, bwt, mark, m,
+                                                                          reinterpret_cast<uint32_t *>(sampled), sampled_base,
+                                                                          reinterpret_cast<uint32_t *>(ends), counts);
+    DSM_LAUNCH_CHECK();
+    if (launches) ++*launches;
+}
+
+void launch_sa_emit64(cudaStream_t st, const uint32_t *sa, const uint8_t *hi, int lo_bits, const uint64_t *bits,
+                      const uint64_t *Rs, const uint8_t *Rb, uint64_t bits_base, uint64_t rank_sub, uint64_t m,
+                      const uint64_t *doc_end, uint32_t ndocs, uint64_t slot_syms, uint64_t *doc_out, uint64_t doc_bit0,
+                      unsigned doc_w, uint64_t *off_out, uint64_t off_bit0, unsigned off_w, uint32_t *launches)
+{
+    if (m == 0 || ndocs == 0) return;
+    sa_emit64_kernel<<<grid_for(m, 256 * 8), 256, 0, st>>>(sa, hi, lo_bits, bits, Rs, Rb, bits_base, rank_sub, m, doc_end, ndocs,
+                                                           slot_syms, doc_out, doc_bit0, doc_w, off_out, off_bit0, off_w);
+    DSM_LAUNCH_CHECK();
+    if (launches) ++*launches;
+}
+
+void launch_sa_lengths(cudaStream_t st, const uint64_t *doc_end, uint64_t first, uint64_t count, uint64_t slot_syms,
+                       uint64_t *out, uint64_t bit0, unsigned w, uint32_t *launches)
+{
+    if (count == 0 || w == 0) return;
+    sa_lengths_kernel<<<grid_for(count, 256 * 8), 256, 0, st>>>(doc_end, first, count, slot_syms, out, bit0, w);
     DSM_LAUNCH_CHECK();
     if (launches) ++*launches;
 }

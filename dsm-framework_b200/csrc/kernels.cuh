@@ -169,6 +169,29 @@ void launch_sa_emit(cudaStream_t st, const uint32_t *sa, const uint64_t *bits, c
                     uint64_t n, const uint32_t *doc_end, uint32_t ndocs, uint32_t *out_doc, uint32_t *out_off,
                     uint32_t *launches);
 
+// The same tables for one slice of a packed-text build (slots of geom, launch_select).  Positions are u64 positions
+// in the padded text; the first document of a slot starts at the slot's first symbol.
+// doc_end[k] (u64) = padded position of document k's terminator, padding skipped; tile_scratch: term_tiles(n_text) u64
+void launch_packed_term_positions(cudaStream_t st, int bits, const uint64_t *packed, uint64_t n_text, const SelGeom &geom,
+                                  uint64_t *tile_scratch, uint64_t *doc_end, uint32_t *launches);
+void launch_sa_mark64(cudaStream_t st, const uint64_t *doc_end, uint32_t ndocs, uint32_t rate, uint64_t slot_syms,
+                      uint32_t *mark, uint32_t *launches);
+// slice of m suffixes (position = hi << lo_bits | lo, hi may be nullptr): bit sampled_base + p of `sampled` (zeroed)
+// = mark[position of p]; bit p of `ends` (zeroed) = bwt[p] == 0; counts[0] += set bits of sampled, counts[1] of ends
+void launch_sa_slice_bits(cudaStream_t st, const uint32_t *sa, const uint8_t *hi, int lo_bits, const uint8_t *bwt,
+                          const uint32_t *mark, uint64_t m, uint64_t *sampled, uint64_t sampled_base, uint64_t *ends,
+                          unsigned long long *counts, uint32_t *launches);
+// For every set bit q = bits_base + p (p < m) of `bits` with its directories: j = rank1(q) - rank_sub; the document
+// k of the suffix's position is written as a doc_w-bit field at bit doc_bit0 + j * doc_w of doc_out (zeroed), its
+// offset in k (when off_out) as an off_w-bit field at off_bit0 + j * off_w of off_out.
+void launch_sa_emit64(cudaStream_t st, const uint32_t *sa, const uint8_t *hi, int lo_bits, const uint64_t *bits,
+                      const uint64_t *Rs, const uint8_t *Rb, uint64_t bits_base, uint64_t rank_sub, uint64_t m,
+                      const uint64_t *doc_end, uint32_t ndocs, uint64_t slot_syms, uint64_t *doc_out, uint64_t doc_bit0,
+                      unsigned doc_w, uint64_t *off_out, uint64_t off_bit0, unsigned off_w, uint32_t *launches);
+// lengths (terminator excluded) of documents [first, first + count) as w-bit fields from bit bit0 of out (zeroed)
+void launch_sa_lengths(cudaStream_t st, const uint64_t *doc_end, uint64_t first, uint64_t count, uint64_t slot_syms,
+                       uint64_t *out, uint64_t bit0, unsigned w, uint32_t *launches);
+
 // ---- wavelet tree -------------------------------------------------------------
 constexpr int kWtTile = 8192; // symbols per CTA
 constexpr int kWtMaxNodes = 255;

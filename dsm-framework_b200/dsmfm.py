@@ -57,6 +57,13 @@ class Pieces(C.Structure):
                 ("bytes", C.c_uint64), ("piece", C.POINTER(Piece)), ("edge", C.POINTER(PieceEdge))]
 
 
+class SaInfo(C.Structure):
+    _fields_ = [("samples", C.c_uint64), ("ends", C.c_uint64), ("documents", C.c_uint64)]
+
+
+SA_VECTORS = 5
+
+
 class Code(C.Structure):
     _fields_ = [("count", C.c_uint64), ("bits", C.c_uint32), ("code", C.c_uint32)]
 
@@ -162,6 +169,10 @@ def lib():
     L.dsmfm_pieces_merge.argtypes = [B, C.c_void_p, C.c_uint32]
     L.dsmfm_pieces_index.argtypes = [B, C.POINTER(Index)]
     L.dsmfm_pieces_write.argtypes = [B, C.c_char_p, C.c_int]
+    L.dsmfm_sa_slice_info.argtypes = [B, C.POINTER(SaInfo)]
+    L.dsmfm_sa_pieces_build.argtypes = [B, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]
+    L.dsmfm_sa_pieces_merge.argtypes = [B, C.c_void_p, C.c_uint32]
+    L.dsmfm_sa_pieces_write.argtypes = [B, C.c_char_p, C.c_int]
     S = C.c_void_p
     L.dsmfm_searcher_create.argtypes = [C.c_int, C.POINTER(Index), C.POINTER(S)]
     L.dsmfm_searcher_open.argtypes = [C.c_int, C.c_char_p, C.POINTER(S)]
@@ -359,6 +370,28 @@ class Builder:
 
     def pieces_write(self, prefix, header):
         self._check(self._L.dsmfm_pieces_write(self._h, os.fsencode(prefix), 1 if header else 0))
+
+    # ---- .sa samples of a packed-text build (FLAG_KEEP_SA; include/dsmfm.h steps 8-11) ----
+    def sa_slice_info(self):
+        """This builder's dsmfm_sa_info record as bytes (to be all-gathered)."""
+        info = SaInfo()
+        self._check(self._L.dsmfm_sa_slice_info(self._h, C.byref(info)))
+        return bytes(info)
+
+    def sa_pieces_build(self, infos_all, world, rank):
+        """infos_all: the records of every builder in slice order, back to back (bytes).  Returns this builder's
+        SA_VECTORS dsmfm_piece_edge records as bytes."""
+        buf = C.create_string_buffer(bytes(infos_all), len(infos_all))
+        edges = (PieceEdge * SA_VECTORS)()
+        self._check(self._L.dsmfm_sa_pieces_build(self._h, buf, world, rank, C.addressof(edges)))
+        return bytes(edges)
+
+    def sa_pieces_merge(self, edges_all, world):
+        buf = C.create_string_buffer(bytes(edges_all), len(edges_all))
+        self._check(self._L.dsmfm_sa_pieces_merge(self._h, buf, world))
+
+    def sa_pieces_write(self, prefix, header):
+        self._check(self._L.dsmfm_sa_pieces_write(self._h, os.fsencode(prefix), 1 if header else 0))
 
     def assemble(self, bwt_dev, n_total):
         """bwt_dev: device address (int) or torch CUDA tensor holding the concatenated BWT."""

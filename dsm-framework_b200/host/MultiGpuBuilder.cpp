@@ -52,7 +52,8 @@ private:
 
 } // namespace
 
-MultiGpuBuilder::MultiGpuBuilder(unsigned gpus, unsigned samplerate) : gpus_(gpus ? gpus : 1), samplerate_(samplerate)
+MultiGpuBuilder::MultiGpuBuilder(unsigned gpus, unsigned samplerate, bool samples)
+    : gpus_(gpus ? gpus : 1), samplerate_(samplerate), samples_(samples)
 {
     if (gpus_ > DSMFM_MAX_BLOCKS) die("at most 64 GPUs");
 }
@@ -91,6 +92,8 @@ void MultiGpuBuilder::Build(uchar const *text, ulong length, std::string const &
     std::vector<dsmfm_shard> shard(world);
     std::vector<dsmfm_pieces> pieces(world);
     std::vector<dsmfm_piece_edge> edges_all;
+    std::vector<dsmfm_sa_info> sa_infos(world);
+    std::vector<dsmfm_piece_edge> sa_edges((size_t)world * DSMFM_SA_VECTORS);
     std::vector<std::string> errors(world);
     dsmfm_text_plan plan;
     std::memset(&plan, 0, sizeof plan);
@@ -111,6 +114,7 @@ void MultiGpuBuilder::Build(uchar const *text, ulong length, std::string const &
         opt.shard_index = r;
         opt.shard_count = world;
         opt.shard_span = 1;
+        opt.flags = samples_ ? DSMFM_FLAG_KEEP_SA : 0u;
         if (dsmfm_create(&opt, &b[r]) != DSMFM_OK) fail("dsmfm_create");
         // 1. the block: records parsed and transformed on this GPU; its statistics
         if (ok && cut[r + 1] > cut[r] && dsmfm_append_fasta(b[r], text + cut[r], cut[r + 1] - cut[r], 1, &fasta[r]) != DSMFM_OK)
@@ -141,8 +145,10 @@ void MultiGpuBuilder::Build(uchar const *text, ulong length, std::string const &
                 std::memset(&o1, 0, sizeof o1);
                 o1.device = dev;
                 o1.samplerate = samplerate_;
+                o1.flags = samples_ ? DSMFM_FLAG_KEEP_SA : 0u;
                 if (dsmfm_create(&o1, &one) != DSMFM_OK || dsmfm_finish(one, &idx) != DSMFM_OK ||
-                    dsmfm_write_fmi(&idx, output.c_str()) != DSMFM_OK)
+                    dsmfm_write_fmi(&idx, output.c_str()) != DSMFM_OK ||
+                    (samples_ && dsmfm_write_sa(one, output.c_str()) != DSMFM_OK))
                     errors[0] = std::string("empty collection: ") + dsmfm_last_error(one);
                 dsmfm_destroy(one);
             }
@@ -188,6 +194,19 @@ void MultiGpuBuilder::Build(uchar const *text, ulong length, std::string const &
         // 6. words and directory entries next to the slice boundaries; 7. the file
         if (ok && dsmfm_pieces_merge(b[r], edges_all.data(), world) != DSMFM_OK) fail("dsmfm_pieces_merge");
         if (ok && dsmfm_pieces_write(b[r], output.c_str(), r == 0) != DSMFM_OK) fail("dsmfm_pieces_write");
+        if (!samples_)
+        {
+            barrier.wait(ok);
+            return;
+        }
+        // 8-11. the same for the .sa samples: slice counts, the rank's share of the five vectors, boundaries, file
+        if (ok && dsmfm_sa_slice_info(b[r], &sa_infos[r]) != DSMFM_OK) fail("dsmfm_sa_slice_info");
+        if (!barrier.wait(ok)) return;
+        if (ok && dsmfm_sa_pieces_build(b[r], sa_infos.data(), world, r, sa_edges.data() + (size_t)r * DSMFM_SA_VECTORS) != DSMFM_OK)
+            fail("dsmfm_sa_pieces_build");
+        if (!barrier.wait(ok)) return;
+        if (ok && dsmfm_sa_pieces_merge(b[r], sa_edges.data(), world) != DSMFM_OK) fail("dsmfm_sa_pieces_merge");
+        if (ok && dsmfm_sa_pieces_write(b[r], output.c_str(), r == 0) != DSMFM_OK) fail("dsmfm_sa_pieces_write");
         barrier.wait(ok);
     };
 

@@ -95,7 +95,8 @@ void help(char const *name)
               << "                               FMIndex::saveSamples (extension; off in the reference)." << std::endl
               << "     --host-parse              Parse and transform the reads on the host, one InsertText" << std::endl
               << "                               per read as the reference does (default: on the GPU)." << std::endl
-              << "     --gpus <int>              Build the one index on <int> GPUs of this box (extension)." << std::endl;
+              << "     --gpus <int>              Build the one index on <int> GPUs of this box (extension);" << std::endl
+              << "                               with --samples every GPU writes its share of <output>.sa." << std::endl;
 }
 
 int parse_int_at_least(char const *value, int min, char const *parameter, char const *name)
@@ -348,7 +349,7 @@ void build_multi_gpu(FILE *in, std::string const &outputfile, unsigned samplerat
         std::cerr << "Read " << have << " bytes of input (elapsed " << wall.seconds() << " s); building on " << g_gpus
                   << " GPUs" << std::endl;
     std::cerr << "Warning: not thread-safe" << std::endl;
-    MultiGpuBuilder mg(g_gpus, samplerate ? samplerate : TEXTCOLLECTION_DEFAULT_SAMPLERATE);
+    MultiGpuBuilder mg(g_gpus, samplerate ? samplerate : TEXTCOLLECTION_DEFAULT_SAMPLERATE, g_samples);
     MultiGpuBuilder::Report rep;
     mg.Build(buf, have, outputfile, rep);
     if (rep.badHeaders) throw std::out_of_range("basic_string::substr: header line without a name");
@@ -506,9 +507,9 @@ int main(int argc, char **argv)
     if (g_verbose) std::cerr << "Building the forward index:" << std::endl;
     if (g_gpus > 1)
     {
-        if (g_host_parse || g_samples)
+        if (g_host_parse)
         {
-            std::cerr << "builder: --gpus can not be combined with --host-parse or --samples" << std::endl;
+            std::cerr << "builder: --gpus can not be combined with --host-parse" << std::endl;
             return 1;
         }
         build_multi_gpu(fin, outputfile, samplerate, wall);

@@ -17,7 +17,10 @@ into one TextCollectionBuilder).  What replaces incbwt's batch merge by backward
      wavelet tree, which bits of the node every slice contributes and how many ones precede them.  Every rank
      builds its share of every node -- bit words, Rs and Rb directories -- on its own GPU, copies it to its
      own host memory, and after an exchange of the few words next to the slice boundaries (96 bytes per node
-     and rank) writes it straight into the `.fmi` file at the offsets of FMIndex::save's layout.
+     and rank) writes it straight into the `.fmi` file at the offsets of FMIndex::save's layout;
+  5. with samples (engines whose builders keep the suffix array, dsmfm.FLAG_KEEP_SA): the same for the five bit
+     vectors of the `.sa` file.  The ranks all-gather their slices' sample / end-marker / document counts (24 bytes
+     each), which fix every rank's range of every vector; the rest is step 4 again.
 
 No rank ever holds the whole index and nothing funnels through one GPU.  torch.distributed is plumbing only:
 the phases below are explicit so that the same host logic runs (a) one rank per process over NCCL or gloo and
@@ -97,6 +100,18 @@ class CudaEngine:
 
     def pieces_write(self, b, prefix, header):
         b.pieces_write(prefix, header)
+
+    def sa_info(self, b):
+        return b.sa_slice_info()
+
+    def sa_pieces_build(self, b, infos_all, world, rank):
+        return b.sa_pieces_build(infos_all, world, rank)
+
+    def sa_pieces_merge(self, b, edges_all, world):
+        b.sa_pieces_merge(edges_all, world)
+
+    def sa_pieces_write(self, b, prefix, header):
+        b.sa_pieces_write(prefix, header)
 
     def stats(self, b):
         return b.stats()
@@ -192,6 +207,24 @@ class ShardedBuild:
         """Every rank writes its share into <prefix>.fmi; rank 0 adds header, node table and tail."""
         self.engine.pieces_write(self.handle, prefix, self.rank == 0)
 
+    def sample_info(self):
+        """-> this rank's dsmfm_sa_info record: samples and end markers of its slice, documents of its block
+        (all-gather them in rank order)."""
+        return self.engine.sa_info(self.handle)
+
+    def samples(self, infos_all):
+        """-> this rank's dsmfm_piece_edge records of the five `.sa` vectors (all-gather them in rank order)."""
+        edges = self.engine.sa_pieces_build(self.handle, b"".join(infos_all), self.world, self.rank)
+        self._mark("samples")
+        return edges
+
+    def merge_samples(self, edges_all):
+        self.engine.sa_pieces_merge(self.handle, b"".join(edges_all), self.world)
+
+    def write_samples(self, prefix):
+        """Every rank writes its share into <prefix>.sa; rank 0 adds the headers."""
+        self.engine.sa_pieces_write(self.handle, prefix, self.rank == 0)
+
     def build_stats(self):
         return self.engine.stats(self.handle) if hasattr(self.engine, "stats") else None
 
@@ -230,13 +263,15 @@ def _all_gather_u64(dist, values, device):
     return np.stack([np.frombuffer(r, dtype=np.uint64) for r in recs])
 
 
-def build_sharded(dist, local_docs, engine, ranges_per_gpu=1, fetch=True):
+def build_sharded(dist, local_docs, engine, ranges_per_gpu=1, fetch=True, samples=False):
     """Builds ONE index over the documents of all ranks (rank order = document order).
 
     local_docs: uint8 tensor (pinned host or device) with this rank's '\\0'-terminated documents.
     Returns the rank's ShardedBuild, merged: sb.write(prefix) puts the rank's share into the `.fmi` file,
     sb.section_bytes is what it holds in host memory.  fetch=False stops with every rank's share of the sections
-    in its HBM (what a device-resident measurement times).  Close it when done."""
+    in its HBM (what a device-resident measurement times).  samples=True (the engine's builders keep the suffix
+    array) also exchanges the `.sa` pieces: sb.write_samples(prefix) then writes the rank's share of <prefix>.sa.
+    Close it when done."""
     world, rank = dist.get_world_size(), dist.get_rank()
     device = engine.tensor_device()
     sb = ShardedBuild(engine, rank, world, ranges_per_gpu)
@@ -254,6 +289,9 @@ def build_sharded(dist, local_docs, engine, ranges_per_gpu=1, fetch=True):
             edges = sb.pieces([int(x) for x in rec[:, 0]], [int(x) for x in rec[:, 1]], rec[:, 2:], fetch)
             if fetch:
                 sb.merge(_all_gather_bytes(dist, edges, device))
+            if samples:
+                sa_edges = sb.samples(_all_gather_bytes(dist, sb.sample_info(), device))
+                sb.merge_samples(_all_gather_bytes(dist, sa_edges, device))
     except Exception:
         sb.close()
         raise
@@ -272,7 +310,7 @@ class _Null:
 
 # ---- (b) all ranks in one process, one after the other (one GPU, or the CPU model) ----------------------------
 
-def build_sharded_local(blocks, engines, ranges_per_gpu=1):
+def build_sharded_local(blocks, engines, ranges_per_gpu=1, samples=False):
     """blocks[r]: uint8 tensor with rank r's documents; engines[r]: its engine (they may share a device).
     The exchanges of build_sharded become plain copies.  Returns the list of merged ShardedBuilds."""
     world = len(blocks)
@@ -296,6 +334,11 @@ def build_sharded_local(blocks, engines, ranges_per_gpu=1):
         edges = [sb.pieces(begins, counts, hist_all) for sb in sbs]
         for sb in sbs:
             sb.merge(edges)
+        if samples:
+            infos = [sb.sample_info() for sb in sbs]
+            sa_edges = [sb.samples(infos) for sb in sbs]
+            for sb in sbs:
+                sb.merge_samples(sa_edges)
     except Exception:
         for sb in sbs:
             sb.close()

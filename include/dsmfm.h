@@ -74,7 +74,7 @@ typedef struct dsmfm_options {
 } dsmfm_options;
 
 #define DSMFM_FLAG_KEEP_BWT 1u /* keep the plain BWT in host memory after finish (dsmfm_index.bwt)   */
-#define DSMFM_FLAG_KEEP_SA 2u  /* keep suffix array, BWT and document boundaries on the device (dsmfm_write_sa) */
+#define DSMFM_FLAG_KEEP_SA 2u  /* keep suffix array, BWT and document boundaries on the device (dsmfm_write_sa, dsmfm_sa_*) */
 #define DSMFM_FLAG_DEFAULT_STREAM 4u /* opts->stream == NULL names the legacy default stream, not "create one" */
 
 /* One Huffman code-table entry: HuffWT::TCodeEntry, HuffWT.h:13-19. */
@@ -266,6 +266,8 @@ DSMFM_API int dsmfm_assemble_pieces(dsmfm_builder *b, const uint64_t *hist_all, 
  *   6. dsmfm_pieces_merge     host: words and directory entries next to a slice boundary are completed
  *   7. dsmfm_pieces_write     every builder writes its share straight into `<prefix>.fmi` (pwrite at the offsets of
  *                             FMIndex::save's layout, FMIndex.cpp:155-217); the builder given `header` != 0 adds the rest.
+ *   8-11. (DSMFM_FLAG_KEEP_SA) the same for the `.sa` samples: dsmfm_sa_slice_info, dsmfm_sa_pieces_build /
+ *                             _merge / _write, below.
  * No builder ever holds the whole index, no GPU the whole wavelet tree, and the device-to-host copies run in parallel. */
 #define DSMFM_MAX_BLOCKS 64
 
@@ -300,7 +302,8 @@ DSMFM_API int dsmfm_text_plan_make(const dsmfm_block_info *all, uint32_t world, 
 DSMFM_API int dsmfm_block_pack(dsmfm_builder *b, const dsmfm_text_plan *plan, uint32_t rank, void *text_dev,
                                uint64_t *top_hist4096);
 /* text_dev must be complete on the builder's stream (all slots, and 8 zero words behind the last slot) and stay
- * untouched until the call returns; top_hist4096 = the sum over all builders.  DSMFM_FLAG_KEEP_SA is not supported. */
+ * untouched until the call returns; top_hist4096 = the sum over all builders.  With DSMFM_FLAG_KEEP_SA the slice is
+ * sorted in full order and what the .sa samples need is derived before the call returns (dsmfm_sa_*, step 8 on). */
 DSMFM_API int dsmfm_build_packed(dsmfm_builder *b, const dsmfm_text_plan *plan, const void *text_dev,
                                  const uint64_t *top_hist4096);
 
@@ -346,6 +349,40 @@ DSMFM_API int dsmfm_pieces_index(dsmfm_builder *b, dsmfm_index *out);
  * build writes the same file, in any order).  header != 0: also everything that is not a BitRank array, and the
  * file is cut to its final size. */
 DSMFM_API int dsmfm_pieces_write(dsmfm_builder *b, const char *path_prefix, int header);
+
+/* ---- the .sa samples of a packed-text build (builders created with DSMFM_FLAG_KEEP_SA) ----
+ * The `.sa` file (dsmfm_write_sa) is five bit vectors: `sampled` (a BitRank over the n BWT positions), then the
+ * BlockArrays `suffixes` and `suffixDocId` (one field per sample, in BWT order), `textLength` (per document) and `Doc`
+ * (per end marker, in BWT order).  Every builder holds a contiguous range of each: its BWT slice of `sampled`, the
+ * fields of its slice's samples and end markers, the lengths of its block's documents.  dsmfm_build_packed derives
+ * what needs the text or the BWT (document ends of the whole collection, the slice's sampled and end-marker bits);
+ * after the .fmi steps (or instead of them):
+ *   8. dsmfm_sa_slice_info    every builder: samples / end markers of its slice, documents of its block
+ *      -> all-gather the dsmfm_sa_info records
+ *   9. dsmfm_sa_pieces_build  every builder: its share of the five vectors at their global bit offsets (the Rs of
+ *                             `sampled` with the samples of earlier slices added), copied to its host; returns one
+ *                             dsmfm_piece_edge per vector
+ *      -> all-gather the edge records (DSMFM_SA_VECTORS per builder)
+ *  10. dsmfm_sa_pieces_merge  host: words and directory entries next to a slice boundary are completed
+ *  11. dsmfm_sa_pieces_write  every builder writes its share into `<prefix>.sa` (pwrite, never truncates); the builder
+ *                             given `header` != 0 adds the file header and the four BlockArray headers and cuts the
+ *                             file to its size.
+ * Document ids are u32 in the file's readers: collections of 2^32 documents or more are refused (DSMFM_ELIMIT). */
+#define DSMFM_SA_VECTORS 5
+
+typedef struct dsmfm_sa_info {
+    uint64_t samples;   /* sampled suffixes in this builder's BWT slice          */
+    uint64_t ends;      /* end markers (BWT symbol 0) in the slice               */
+    uint64_t documents; /* documents of this builder's block                     */
+} dsmfm_sa_info;
+
+DSMFM_API int dsmfm_sa_slice_info(dsmfm_builder *b, dsmfm_sa_info *out);
+/* infos_all[world]: dsmfm_sa_slice_info of every builder, in slice order.  edges_out[DSMFM_SA_VECTORS]. */
+DSMFM_API int dsmfm_sa_pieces_build(dsmfm_builder *b, const dsmfm_sa_info *infos_all, uint32_t world, uint32_t rank,
+                                    dsmfm_piece_edge *edges_out);
+/* edges_all[world][DSMFM_SA_VECTORS] in slice order (host). */
+DSMFM_API int dsmfm_sa_pieces_merge(dsmfm_builder *b, const dsmfm_piece_edge *edges_all, uint32_t world);
+DSMFM_API int dsmfm_sa_pieces_write(dsmfm_builder *b, const char *path_prefix, int header);
 
 /* Helpers for hosts that do not link the CUDA runtime themselves (the C++ CLI runs one thread per GPU and moves
  * the packed slots with peer copies instead of NCCL): device memory for the packed text, and the copy of slot
