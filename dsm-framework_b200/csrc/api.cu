@@ -943,18 +943,55 @@ void dsmfm_builder::append_fasta(const uint8_t *text, size_t m, dsmfm_fasta_info
 // ---------------------------------------------------------------------------
 namespace {
 constexpr uint64_t kLongKeyAbove = 3500000000ull; // indexed symbols above which the first key is 18 symbols (build())
-// first key of an unsharded build (see build()): symbols sorted by the initial radix sort, BWT symbol carried or not
-void first_key_shape(int bits, uint64_t n_idx, int *first_syms, bool *carry)
+// Dense codes (0 = terminator, 1..sigma in byte order) of the bytes that occur; returns the bits per symbol.
+int alphabet_of(const uint64_t counts[256], uint8_t code_map[256], uint32_t *sigma_out)
+{
+    std::memset(code_map, 0, 256);
+    uint32_t sigma = 0;
+    for (int c = 1; c < 256; ++c)
+        if (counts[c]) code_map[c] = (uint8_t)++sigma;
+    if (sigma_out) *sigma_out = sigma;
+    return sigma <= 7 ? 3 : (sigma <= 15 ? 4 : 8);
+}
+
+// Symbols of the first key (sorted by the initial radix sort): `first_key_bits` when > 0, else the default of
+// build() -- 48 bits, 54 / 56 above kLongKeyAbove indexed symbols, DSMFM_FIRST_KEY_BITS overriding both.
+// Widths outside [8, SPW * bits] mean the whole word.
+int first_key_syms(int bits, uint64_t n_idx, int first_key_bits)
 {
     const int spw = 64 / bits;
-    uint64_t long_key_above = kLongKeyAbove;
-    if (const char *e = std::getenv("DSMFM_LONG_KEY_ABOVE")) long_key_above = std::strtoull(e, nullptr, 10);
-    int first_key_bits = 48;
-    if (n_idx > long_key_above) first_key_bits = bits == 3 ? 54 : (bits == 4 ? 56 : 48);
-    if (const char *e = std::getenv("DSMFM_FIRST_KEY_BITS")) first_key_bits = std::atoi(e);
+    if (first_key_bits <= 0) {
+        uint64_t long_key_above = kLongKeyAbove;
+        if (const char *e = std::getenv("DSMFM_LONG_KEY_ABOVE")) long_key_above = std::strtoull(e, nullptr, 10);
+        first_key_bits = 48;
+        if (n_idx > long_key_above) first_key_bits = bits == 3 ? 54 : (bits == 4 ? 56 : 48);
+        if (const char *e = std::getenv("DSMFM_FIRST_KEY_BITS")) first_key_bits = std::atoi(e);
+    }
     if (first_key_bits < 8 || first_key_bits > spw * bits) first_key_bits = spw * bits;
-    *first_syms = std::max(1, first_key_bits / bits);
+    return std::max(1, first_key_bits / bits);
+}
+
+// first key of an unsharded build: symbols sorted, and whether the BWT symbol rides above them
+void first_key_shape(int bits, uint64_t n_idx, int first_key_bits, int *first_syms, bool *carry)
+{
+    *first_syms = first_key_syms(bits, n_idx, first_key_bits);
     *carry = *first_syms * bits + bits <= 64;
+}
+
+// One word range of a text that is packed and keyed piece by piece: packs words [w0, w0 + wn) from `raw`, the
+// text from symbol w0 * SPW on (`len` symbols of it; the last range also writes the zero words behind the text),
+// then keys every word whose successor is packed by now.  Returns the words keyed so far.
+uint64_t pack_and_key_range(cudaStream_t st, int bits, const uint8_t *raw, uint64_t len, const uint8_t *d_map,
+                            uint64_t *d_packed, uint64_t w0, uint64_t wn, bool last, uint64_t n, uint64_t *d_keys,
+                            int first_syms, bool carry, uint64_t *d_hist, uint64_t keyed_to, uint32_t *L)
+{
+    launch_pack(st, bits, raw, len, d_map, d_packed + w0, wn, L);
+    const uint64_t upto = last ? div_up(n, 64 / bits) : w0 + wn - 1;
+    if (upto > keyed_to) {
+        launch_make_keys_hist(st, bits, d_packed, n, d_keys, first_syms, carry, d_hist, L, keyed_to, upto);
+        keyed_to = upto;
+    }
+    return keyed_to;
 }
 } // namespace
 
@@ -1005,12 +1042,9 @@ bool dsmfm_builder::append_pipelined(const uint8_t *src, size_t bytes)
     uint64_t first_counts[256];
     DSM_CUDA(cudaMemcpyAsync(first_counts, pl.d_counts, sizeof first_counts, cudaMemcpyDeviceToHost, st));
     DSM_CUDA(cudaStreamSynchronize(st));
-    std::memset(pl.code_map, 0, sizeof pl.code_map);
     uint32_t sigma = 0;
-    for (int c = 1; c < 256; ++c)
-        if (first_counts[c]) pl.code_map[c] = (uint8_t)++sigma;
-    pl.bits = sigma <= 7 ? 3 : (sigma <= 15 ? 4 : 8);
-    first_key_shape(pl.bits, bytes, &pl.first_syms, &pl.carry);
+    pl.bits = alphabet_of(first_counts, pl.code_map, &sigma);
+    first_key_shape(pl.bits, bytes, 0, &pl.first_syms, &pl.carry);
     const int spw = 64 / pl.bits;
     pl.spec = sigma > 0 && (pl.first_syms * pl.bits + 7) / 8 <= kMaxPasses;
     uint64_t text_words = div_up(bytes, (uint64_t)spw);
@@ -1029,14 +1063,9 @@ bool dsmfm_builder::append_pipelined(const uint8_t *src, size_t bytes)
         if (!pl.spec) continue;
         const uint64_t o = k * kPiece, len = std::min<uint64_t>(kPiece, bytes - o);
         const bool last = k + 1 == npiece;
-        const uint64_t w0 = o / spw, wn = last ? pl.nwords - w0 : len / spw; // (the last piece also writes the zero words)
-        launch_pack(st, pl.bits, d + o, len, pl.d_map, pl.d_packed + w0, wn, L);
-        // keys of every word whose successor is packed by now
-        const uint64_t upto = last ? text_words : w0 + wn - 1;
-        if (upto > keyed_to) {
-            launch_make_keys_hist(st, pl.bits, pl.d_packed, bytes, pl.d_keys, pl.first_syms, pl.carry, pl.d_hist, L, keyed_to, upto);
-            keyed_to = upto;
-        }
+        const uint64_t w0 = o / spw, wn = last ? pl.nwords - w0 : len / spw;
+        keyed_to = pack_and_key_range(st, pl.bits, d + o, len, pl.d_map, pl.d_packed, w0, wn, last, bytes, pl.d_keys,
+                                      pl.first_syms, pl.carry, pl.d_hist, keyed_to, L);
     }
     return true;
 }
@@ -1225,11 +1254,8 @@ void dsmfm_builder::build()
     const uint64_t n_idx = packed_in ? ext->n_real : n;                                // symbols of the index
 
     uint8_t code_map[256];
-    std::memset(code_map, 0, sizeof code_map);
     uint32_t sigma = 0;
-    for (int c = 1; c < 256; ++c)
-        if (counts[c]) code_map[c] = (uint8_t)++sigma;
-    const int bits = sigma <= 7 ? 3 : (sigma <= 15 ? 4 : 8);
+    const int bits = alphabet_of(counts, code_map, &sigma);
     const int spw = 64 / bits;
     // positions are positions in the text as it lies in HBM: the packed slots with their padding when the text
     // came in packed (one slot per block), the plain text otherwise
@@ -1245,13 +1271,7 @@ void dsmfm_builder::build()
     // threshold sits between the 1 Gbp sample -- 2.02 G symbols, where the seventh pass costs what it saves -- and two
     // of them, 4.04 G, where the refinement takes 36 ms with 16 symbols.)
     // DSMFM_FIRST_KEY_BITS overrides (any multiple of bits/symbol); DSMFM_LONG_KEY_ABOVE moves the threshold (tests).
-    uint64_t long_key_above = kLongKeyAbove;
-    if (const char *e = std::getenv("DSMFM_LONG_KEY_ABOVE")) long_key_above = std::strtoull(e, nullptr, 10);
-    int first_key_bits = 48;
-    if (n_idx > long_key_above) first_key_bits = bits == 3 ? 54 : (bits == 4 ? 56 : 48);
-    if (const char *e = std::getenv("DSMFM_FIRST_KEY_BITS")) first_key_bits = std::atoi(e);
-    if (first_key_bits < 8 || first_key_bits > spw * bits) first_key_bits = spw * bits;
-    int first_syms = std::max(1, first_key_bits / bits);
+    int first_syms = first_key_syms(bits, n_idx, 0);
     // Text positions: the u32 value of the sort holds the low `lo_bits` bits (32; fewer only in tests, which
     // thereby exercise the wide path on small inputs), anything above rides in the key's spare top bits.
     // A packed-text build always takes the key-range path (its padding positions must not be sorted).
@@ -3416,6 +3436,109 @@ DSMFM_API int dsmfm_dbg_radix_sort(int device, uint64_t *keys, uint32_t *vals, u
     }
     ws.release();
     cudaFree(ka); cudaFree(kb); cudaFree(va); cudaFree(vb);
+    return rc;
+}
+
+DSMFM_API int dsmfm_dbg_initial_sort(int device, const uint8_t *docs, uint64_t n, int first_key_bits,
+                                     const uint64_t *word_cuts, uint32_t ncuts, uint64_t *keys, uint64_t *hist,
+                                     uint64_t *sorted_keys, uint32_t *sa, uint32_t *head, uint32_t *diff, uint8_t *bwt,
+                                     uint64_t *remaining, int *bits_out, int *first_syms_out, int *carry_out)
+{
+    // everything the caller hands in is checked before anything is launched
+    if (!docs || !keys || !hist || !sorted_keys || !sa || !head || !diff || !bwt || !remaining || !bits_out ||
+        !first_syms_out || !carry_out || (ncuts && !word_cuts))
+        return DSMFM_EINVAL;
+    if (n == 0 || n >= (1ull << 32) - kRefCap - 64 || docs[n - 1] != 0 || docs[0] == 0) return DSMFM_EINVAL;
+    uint64_t counts[256] = {};
+    for (uint64_t i = 0; i < n; ++i) {
+        ++counts[docs[i]];
+        if (i && docs[i] == 0 && docs[i - 1] == 0) return DSMFM_EINVAL; // an empty document
+    }
+    uint8_t code_map[256], inv_map[256] = {};
+    const int bits = alphabet_of(counts, code_map, nullptr);
+    for (int c = 1; c < 256; ++c)
+        if (code_map[c]) inv_map[code_map[c]] = (uint8_t)c;
+    const int spw = 64 / bits;
+    const uint64_t text_words = div_up(n, spw), nwords = text_words + 8;
+    for (uint32_t k = 0; k < ncuts; ++k)
+        if (word_cuts[k] == 0 || word_cuts[k] >= text_words || (k && word_cuts[k] <= word_cuts[k - 1])) return DSMFM_EINVAL;
+    int first_syms = 0;
+    bool carry = false;
+    first_key_shape(bits, n, first_key_bits, &first_syms, &carry);
+    const int key_bits = first_syms * bits;
+    if (cudaSetDevice(device < 0 ? 0 : device) != cudaSuccess) return DSMFM_ECUDA;
+
+    const uint64_t hw = head_words_for(n), out_words = div_up(n, 32);
+    uint8_t *d_raw = nullptr, *d_map = nullptr, *d_inv = nullptr, *d_bwt = nullptr;
+    uint64_t *d_packed = nullptr, *ka = nullptr, *kb = nullptr;
+    uint32_t *va = nullptr, *vb = nullptr, *d_head = nullptr, *d_diff = nullptr;
+    unsigned long long *d_rem = nullptr;
+    RadixWorkspace ws;
+    int rc = DSMFM_OK;
+    try {
+        DSM_CUDA(cudaMalloc(&d_raw, n + 64));
+        DSM_CUDA(cudaMalloc(&d_map, 256));
+        DSM_CUDA(cudaMalloc(&d_inv, 256));
+        DSM_CUDA(cudaMalloc(&d_packed, nwords * 8));
+        DSM_CUDA(cudaMalloc(&ka, n * 8));
+        DSM_CUDA(cudaMalloc(&kb, n * 8));
+        DSM_CUDA(cudaMalloc(&va, n * 4 + 16));
+        DSM_CUDA(cudaMalloc(&vb, n * 4 + 16));
+        DSM_CUDA(cudaMalloc(&d_head, hw * 4));
+        DSM_CUDA(cudaMalloc(&d_diff, hw * 4));
+        DSM_CUDA(cudaMalloc(&d_bwt, n + 64));
+        DSM_CUDA(cudaMalloc(&d_rem, 128 * 8));
+        ws.allocate(n);
+        DSM_CUDA(cudaMemcpy(d_raw, docs, n, cudaMemcpyHostToDevice));
+        DSM_CUDA(cudaMemcpy(d_map, code_map, 256, cudaMemcpyHostToDevice));
+        DSM_CUDA(cudaMemcpy(d_inv, inv_map, 256, cudaMemcpyHostToDevice));
+        // a word read before it is packed shows up as a wrong key, not as a lucky zero
+        DSM_CUDA(cudaMemset(d_packed, 0xa5, nwords * 8));
+        DSM_CUDA(cudaMemset(ws.hist, 0, sizeof(uint64_t) * kMaxPasses * kRadix));
+        if (ncuts == 0) { // build(): the whole text in one go
+            launch_pack(nullptr, bits, d_raw, n, d_map, d_packed, nwords, nullptr);
+            launch_make_keys_hist(nullptr, bits, d_packed, n, ka, first_syms, carry, ws.hist, nullptr);
+        } else { // append_pipelined(): word range by word range
+            uint64_t keyed_to = 0;
+            for (uint32_t k = 0; k <= ncuts; ++k) {
+                const uint64_t w0 = k ? word_cuts[k - 1] : 0;
+                const bool last = k == ncuts;
+                const uint64_t wn = (last ? nwords : word_cuts[k]) - w0;
+                const uint64_t len = last ? n - w0 * spw : wn * spw;
+                keyed_to = pack_and_key_range(nullptr, bits, d_raw + w0 * spw, len, d_map, d_packed, w0, wn, last, n,
+                                              ka, first_syms, carry, ws.hist, keyed_to, nullptr);
+            }
+        }
+        DSM_CUDA(cudaMemcpy(keys, ka, n * 8, cudaMemcpyDeviceToHost));
+        DSM_CUDA(cudaMemcpy(hist, ws.hist, sizeof(uint64_t) * kMaxPasses * kRadix, cudaMemcpyDeviceToHost));
+        const int p = radix_sort_pairs(nullptr, ws, ka, va, kb, vb, n, 0, key_bits, true, nullptr, nullptr, nullptr, true);
+        uint64_t *sk = (p & 1) ? kb : ka;
+        uint32_t *sv = (p & 1) ? vb : va;
+        DSM_CUDA(cudaMemset(d_rem, 0, 128 * 8));
+        launch_heads(nullptr, bits, sk, n, d_head, hw, d_rem, key_bits, d_inv, carry ? d_bwt : nullptr, nullptr, 0,
+                     carry ? d_diff : nullptr, nullptr);
+        DSM_CUDA(cudaDeviceSynchronize());
+        unsigned long long h_rem[64];
+        DSM_CUDA(cudaMemcpy(h_rem, d_rem, sizeof h_rem, cudaMemcpyDeviceToHost));
+        DSM_CUDA(cudaMemcpy(sorted_keys, sk, n * 8, cudaMemcpyDeviceToHost));
+        DSM_CUDA(cudaMemcpy(sa, sv, n * 4, cudaMemcpyDeviceToHost));
+        DSM_CUDA(cudaMemcpy(head, d_head, out_words * 4, cudaMemcpyDeviceToHost));
+        if (carry) {
+            DSM_CUDA(cudaMemcpy(diff, d_diff, out_words * 4, cudaMemcpyDeviceToHost));
+            DSM_CUDA(cudaMemcpy(bwt, d_bwt, n, cudaMemcpyDeviceToHost));
+        }
+        *remaining = 0;
+        for (int i = 0; i < 64; ++i) *remaining += h_rem[i];
+        *bits_out = bits;
+        *first_syms_out = first_syms;
+        *carry_out = carry ? 1 : 0;
+    } catch (const CudaError &e) {
+        g_create_error = std::string("dsmfm_dbg_initial_sort: ") + cudaGetErrorString(e.code) + " in " + e.what;
+        rc = DSMFM_ECUDA;
+    }
+    ws.release();
+    cudaFree(d_raw); cudaFree(d_map); cudaFree(d_inv); cudaFree(d_packed); cudaFree(ka); cudaFree(kb);
+    cudaFree(va); cudaFree(vb); cudaFree(d_head); cudaFree(d_diff); cudaFree(d_bwt); cudaFree(d_rem);
     return rc;
 }
 

@@ -201,6 +201,8 @@ def lib():
     L.dsmfm_searcher_destroy.restype = None
     L.dsmfm_dbg_guard_violations.restype = C.c_uint64
     L.dsmfm_dbg_radix_sort.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]
+    L.dsmfm_dbg_initial_sort.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint32] + \
+        [C.c_void_p] * 8 + [C.POINTER(C.c_int)] * 3
     L.dsmfm_dbg_wavelet.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.POINTER(Index), C.POINTER(C.c_void_p)]
     L.dsmfm_dbg_free_index.argtypes = [C.c_void_p]
     L.dsmfm_dbg_free_index.restype = None
@@ -658,6 +660,31 @@ def radix_sort(keys, vals, begin_bit=0, end_bit=64, device=0):
     rc = L.dsmfm_dbg_radix_sort(device, keys.ctypes.data, vals.ctypes.data, keys.size, begin_bit, end_bit)
     if rc != OK:
         raise DsmfmError(rc, (L.dsmfm_last_error(None) or b"").decode())
+
+
+def initial_sort(docs, first_key_bits=0, word_cuts=None, device=0):
+    """The initial suffix sort of an unsharded build, up to the group heads (dsmfm_dbg_initial_sort).
+    docs: numpy uint8 '\\0'-terminated documents.  Returns a dict of numpy arrays: keys, hist (8 x 256),
+    sorted_keys, sa, head, diff, bwt (diff / bwt stay zero when carry == 0) and the ints remaining, bits,
+    first_syms, carry."""
+    import numpy as np
+    L = lib()
+    docs = np.ascontiguousarray(docs, dtype=np.uint8)
+    n = docs.size
+    cuts = np.ascontiguousarray(word_cuts if word_cuts is not None else [], dtype=np.uint64)
+    hw = (n + 31) // 32
+    out = dict(keys=np.empty(n, np.uint64), hist=np.zeros((8, 256), np.uint64), sorted_keys=np.empty(n, np.uint64),
+               sa=np.empty(n, np.uint32), head=np.empty(hw, np.uint32), diff=np.zeros(hw, np.uint32),
+               bwt=np.zeros(n, np.uint8), remaining=np.zeros(1, np.uint64))
+    bits, first_syms, carry = C.c_int(), C.c_int(), C.c_int()
+    rc = L.dsmfm_dbg_initial_sort(device, docs.ctypes.data, n, first_key_bits, cuts.ctypes.data if cuts.size else None,
+                                  cuts.size, *[out[k].ctypes.data for k in ("keys", "hist", "sorted_keys", "sa", "head",
+                                                                             "diff", "bwt", "remaining")],
+                                  C.byref(bits), C.byref(first_syms), C.byref(carry))
+    if rc != OK:
+        raise DsmfmError(rc, (L.dsmfm_last_error(None) or b"").decode())
+    out.update(remaining=int(out["remaining"][0]), bits=bits.value, first_syms=first_syms.value, carry=carry.value)
+    return out
 
 
 def wavelet_fmi(seq, device=0):

@@ -514,6 +514,20 @@ DSMFM_API uint64_t dsmfm_dbg_guard_violations(void);
  * the same onesweep kernels the build uses.  Sorts in place. */
 DSMFM_API int dsmfm_dbg_radix_sort(int device, uint64_t *keys, uint32_t *vals, uint64_t n, int begin_bit, int end_bit);
 
+/* The initial suffix sort of an unsharded build, stopped after the group heads: the build's code map, first-key
+ * rule (first_key_bits <= 0: the default, else that many key bits), pack, keys with their digit counts, radix sort
+ * and heads.  `docs` holds n bytes of '\0'-terminated, non-empty documents (n < 2^32 - 2112).  With ncuts > 0 the
+ * text is packed and keyed word range by word range, as a batch streaming in from the host is: word_cuts are
+ * increasing word indices in (0, words of the text).
+ * Out (host): keys[n] (unsorted, text order), hist[8 * 256] (digit counts per 8-bit pass), sorted_keys[n], sa[n],
+ * head[ceil(n/32)], remaining (ranks in groups of >= 2), bits per symbol, first_syms, carry (1: the BWT symbol
+ * rides above the key; then diff[ceil(n/32)] and bwt[n] are written, else they are left untouched).
+ * DSMFM_EINVAL (nothing launched) on malformed input. */
+DSMFM_API int dsmfm_dbg_initial_sort(int device, const uint8_t *docs, uint64_t n, int first_key_bits,
+                                     const uint64_t *word_cuts, uint32_t ncuts, uint64_t *keys, uint64_t *hist,
+                                     uint64_t *sorted_keys, uint32_t *sa, uint32_t *head, uint32_t *diff, uint8_t *bwt,
+                                     uint64_t *remaining, int *bits, int *first_syms, int *carry);
+
 /* Wavelet tree + BitRank directories for an arbitrary byte sequence (the
  * HuffWT::makeHuffWT path alone); `out` pointers are valid until
  * dsmfm_dbg_free_index. */
