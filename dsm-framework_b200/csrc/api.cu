@@ -1480,16 +1480,10 @@ void dsmfm_builder::build()
     if (sharded && keep_sa) d_sa_all = static_cast<uint32_t *>(dmalloc(m_total * 4 + 16));
     if (wide) d_hi_buf = static_cast<uint8_t *>(dmalloc((keep_sa ? m_total : m_max) + 16));
 
-    // multi-step: one launch resolves every group that fits a CTA (DSMFM_REFINE_SINGLE_STEP=1 keeps
-    // the one-depth-per-launch schedule, used by the tests to exercise the worklist path)
-    bool multi_step = true;
-    if (const char *e = std::getenv("DSMFM_REFINE_SINGLE_STEP")) multi_step = std::atoi(e) == 0;
     // The index needs the BWT, not the suffix array: tie groups whose members share one BWT symbol stay unsorted
     // unless the suffix array itself is wanted (DSMFM_FLAG_KEEP_SA; DSMFM_REFINE_FULL_ORDER=1 forces it).
     bool full_order = keep_sa;
     if (const char *e = std::getenv("DSMFM_REFINE_FULL_ORDER")) full_order = full_order || std::atoi(e) != 0;
-    int key_words = 1; // symbols compared per step = key_words * SPW (DSMFM_REFINE_KEY_WORDS=2: 128-bit keys)
-    if (const char *e = std::getenv("DSMFM_REFINE_KEY_WORDS")) key_words = std::atoi(e) == 2 ? 2 : 1;
 
     cudaEvent_t evr[3];
     for (auto &e : evr) DSM_CUDA(cudaEventCreate(&e));
@@ -1569,7 +1563,7 @@ void dsmfm_builder::build()
         uint64_t m_act = 0;
         const char *compact_env = std::getenv("DSMFM_REFINE_COMPACT"); // 0: refine in place (tests)
         const bool compact_off = compact_env && std::atoi(compact_env) == 0;
-        const bool compact = use_diff && multi_step && !compact_off && remaining > 0;
+        const bool compact = use_diff && !compact_off && remaining > 0;
         bool c_owned = false; // the dense arrays are allocations of their own (else: carved out of a key buffer)
         if (compact) {
             // scratch of the compaction: the key buffers of the initial sort are free from here on (the large-group
@@ -1655,7 +1649,7 @@ void dsmfm_builder::build()
             ++stats.refine_launches;
             launch_refine(st, bits, d_packed, r_sa, r_head[cur], r_head[cur ^ 1], r_m, depth, win_list, n_list,
                           d_big_heads, big_cap, d_big_count, d_remaining, d_win_flag, d_win_list[wl], d_win_count,
-                          r_bwt, multi_step, key_words, r_hi, lo_bits, full_order, round == 1 ? r_diff : nullptr, L,
+                          r_bwt, r_hi, lo_bits, full_order, round == 1 ? r_diff : nullptr, L,
                           /*big_groups=*/!full_order && !(compact && m_act));
             uint32_t nbig = 0;
             DSM_CUDA(cudaMemcpyAsync(&nbig, d_big_count, 4, cudaMemcpyDeviceToHost, st));
@@ -1718,9 +1712,9 @@ void dsmfm_builder::build()
                 dfree(d_bhi);
                 remaining += total; // re-examined (and counted exactly) by the next round
             }
-            // a CTA step consumes key_words*SPW symbols, the large-group path SPW; starting the next launch at the
-            // smaller of the two is always safe (already-equal symbols just compare equal again)
-            depth_next = depth + ((multi_step || nbig > 0) ? (uint32_t)spw : (uint32_t)(key_words * spw));
+            // a launch resolves every group that fits a CTA: what is left went through the large-group path,
+            // which sorted it by the SPW symbols from `depth` on
+            depth_next = depth + (uint32_t)spw;
             DSM_CUDA(cudaMemcpyAsync(&n_list, d_win_count, 4, cudaMemcpyDeviceToHost, st));
             DSM_CUDA(cudaStreamSynchronize(st));
             win_list = d_win_list[wl];

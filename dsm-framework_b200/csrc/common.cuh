@@ -110,28 +110,6 @@ template <int BITS> __device__ __forceinline__ uint64_t text_window(const uint64
     return cut_at_terminator<BITS>(x);
 }
 
-// 2*SPW-symbol window starting at symbol p (three consecutive words), cut at the terminator:
-// hi = symbols [p, p+SPW), lo = symbols [p+SPW, p+2*SPW).
-template <int BITS>
-__device__ __forceinline__ void text_window2(const uint64_t *__restrict__ packed, uint64_t p, uint64_t &hi, uint64_t &lo)
-{
-    using P = Pack<BITS>;
-    const uint64_t w = p / P::SPW;
-    const int s = (int)(p - w * P::SPW);
-    const uint64_t x0 = __ldg(packed + w), x1 = __ldg(packed + w + 1);
-    uint64_t h = (x0 << (BITS * s)) & P::USED_MASK, l = (x1 << (BITS * s)) & P::USED_MASK;
-    if (s) {
-        const uint64_t x2 = __ldg(packed + w + 2);
-        h |= x1 >> (BITS * (P::SPW - s));
-        l |= x2 >> (BITS * (P::SPW - s));
-    }
-    const uint64_t hc = cut_at_terminator<BITS>(h);
-    // a terminator inside hi ends the suffix: nothing after it may be looked at
-    const bool ended = key_terminated<BITS>(hc);
-    hi = hc;
-    lo = ended ? 0ull : cut_at_terminator<BITS>(l);
-}
-
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ unsigned lanemask_lt() { return (1u << (threadIdx.x & 31)) - 1; }
 

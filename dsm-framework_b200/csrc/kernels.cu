@@ -214,29 +214,13 @@ template <int BITS> __device__ __forceinline__ uint32_t text_symbol(const uint64
 // low key_bits.  With carry_prev the code of the symbol BEFORE the suffix (0 at a document start) rides
 // in the bits just above: the radix sort never looks at them, so the BWT symbol of every suffix
 // arrives at its rank for free and no gather over the sorted suffix array is needed afterwards.
-template <int BITS>
-__global__ void __launch_bounds__(256) make_keys_kernel(const uint64_t *__restrict__ packed, uint64_t n,
-                                                        uint64_t *__restrict__ keys, int drop_bits, int key_bits,
-                                                        bool carry_prev)
-{
-    const uint64_t stride = (uint64_t)gridDim.x * 256;
-    for (uint64_t p = (uint64_t)blockIdx.x * 256 + threadIdx.x; p < n; p += stride) {
-        uint64_t k = text_window<BITS>(packed, p) >> drop_bits;
-        if (carry_prev && p) k |= (uint64_t)text_symbol<BITS>(packed, p - 1) << key_bits;
-        keys[p] = k;
-    }
-}
-
-// Same keys, one thread per packed word: the word and its successor hold every symbol the SPW first keys
+// One thread per packed word: the word and its successor hold every symbol the SPW first keys
 // starting in it can need, so the keys are cut out of two registers instead of two loads and a division
 // per suffix; they are staged in shared memory and leave the SM as one contiguous burst.  While the keys
 // are in registers the kernel also counts their radix digits, which saves the sort's own histogram pass
 // over the key array (8 bytes per suffix read back from HBM).
 constexpr int kHeadsU = 8;           // head words per warp iteration of heads_kernel (8: 5.9 -> 5.3 ms on C3)
-#ifndef DSMFM_HEADS_CTAS
-#define DSMFM_HEADS_CTAS 4
-#endif
-constexpr int kHeadsCtas = DSMFM_HEADS_CTAS; // resident CTAs per SM the registers of heads_kernel are budgeted for
+constexpr int kHeadsCtas = 4;        // resident CTAs per SM the registers of heads_kernel are budgeted for
 constexpr int kKeyTileThreads = 128; // one packed word per thread and tile
 constexpr int kMaxKeyPasses = 8;     // 64 key bits / 8-bit digits
 constexpr int kKeySub = 1;           // copies of every digit counter in make_keys_hist_kernel (4 copies: no gain measured)
@@ -711,7 +695,7 @@ select_sweep_kernel(const uint64_t *__restrict__ packed, uint64_t nwords, int ke
 // whether its BWT symbol differs.  "Next rank opens a group" is the head bit of the next rank, so the count of
 // suffixes left in groups of >= 2 falls out of the head words themselves.  Chunks that lie entirely inside
 // the array take a path without bounds checks and with 32-bit offsets from the chunk's base pointers.
-template <int BITS, int U>
+template <int BITS>
 __global__ void __launch_bounds__(256, kHeadsCtas) heads_kernel(const uint64_t *__restrict__ keys, uint64_t n,
                                                     uint32_t *__restrict__ head, uint64_t head_words,
                                                     unsigned long long *__restrict__ remaining, int key_bits,
@@ -720,6 +704,7 @@ __global__ void __launch_bounds__(256, kHeadsCtas) heads_kernel(const uint64_t *
                                                     uint32_t *__restrict__ diff)
 {
     constexpr uint64_t FIELD = Pack<BITS>::FIELD;
+    constexpr int U = kHeadsU;
     __shared__ unsigned long long s_cnt[8];
     __shared__ uint8_t s_inv[256];
     if (bwt) s_inv[threadIdx.x] = inv_map[threadIdx.x];
@@ -870,262 +855,6 @@ __device__ __forceinline__ int next_set_gt(const uint32_t *hw, int r)
     return (w << 5) + __ffs(m) - 1;
 }
 
-template <int KW, bool WIDE> struct RefSmem {
-    uint64_t khi[kRefCap];              // key = the next KW*SPW symbols (hi [, lo])
-    uint64_t klo[KW == 2 ? kRefCap : 1];
-    uint32_t sa[2][kRefCap];            // suffixes, double buffered across a step
-    uint16_t list[2][kRefCap];          // unresolved slots (relative to the window), current / next step
-    uint8_t bw[2][kRefCap];             // BWT bytes travelling with the suffixes
-    uint8_t hi[2][WIDE ? kRefCap : 1];  // wide builds: text position = hi << lo_bits | sa
-    uint32_t head_a[kRefCap / 32 + 2];  // group heads the ranking phase reads
-    uint32_t head_b[kRefCap / 32 + 2];  // = head_a plus the heads found in the current step
-    int n[2];
-    int range[3];
-};
-
-// One CTA owns the groups whose head lies in its window of kRefWindow slots and keeps refining
-// them in shared memory -- key = the next KW*SPW symbols, stable rank inside the group, split --
-// until they are all resolved (multi-step) or for a single step.  The suffix array (and the BWT
-// bytes that travel with it) are read once; a suffix is written back the moment it becomes a
-// singleton; only the text is touched again in every step.  A step is two phases and two barriers:
-//   rank:     every unresolved suffix finds its stable rank inside its group (all pairs), moves to
-//             the other buffer and marks the new group heads;
-//   classify: resolved suffixes go home; the others fetch their next key and join the next list.
-template <int BITS, int KW, bool WIDE>
-__global__ void __launch_bounds__(kRefThreads, KW == 2 ? 3 : 4)
-refine_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ sa, const uint32_t *__restrict__ head_cur,
-              uint32_t *__restrict__ head_next, uint64_t n, uint32_t depth, const uint32_t *__restrict__ win_list,
-              uint32_t *__restrict__ big_heads, uint32_t big_cap, uint32_t *__restrict__ big_count,
-              unsigned long long *__restrict__ remaining, uint32_t *__restrict__ win_flag,
-              uint32_t *__restrict__ win_next, uint32_t *__restrict__ win_next_count, uint32_t nwin,
-              uint8_t *__restrict__ bwt, int max_steps, uint8_t *__restrict__ sa_hi, int lo_bits)
-{
-    constexpr int HW = kRefCap / 32 + 2;            // head words held in shared memory
-    constexpr int WIN_WORDS = kRefWindow / 32;      // 32: one warp scans the window
-    static_assert(WIN_WORDS == 32 && kRefGroupMax / 32 == 32, "window and group limit are one warp of words each");
-    static_assert(kRefCap <= 65536, "slot lists are 16-bit");
-    extern __shared__ __align__(16) unsigned char ref_smem_raw[];
-    RefSmem<KW, WIDE> &S = *reinterpret_cast<RefSmem<KW, WIDE> *>(ref_smem_raw);
-    uint64_t *s_khi = S.khi, *s_klo = S.klo;
-    uint32_t(*s_sa)[kRefCap] = S.sa;
-    uint8_t(*s_bw)[kRefCap] = S.bw;
-    uint8_t(*s_hi)[WIDE ? kRefCap : 1] = S.hi;
-    uint16_t(*s_list)[kRefCap] = S.list;
-    uint32_t *s_ha = S.head_a, *s_hb = S.head_b;
-    int *s_n = S.n, *s_range = S.range;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t wid = win_list ? win_list[blockIdx.x] : blockIdx.x; // window owned by this CTA
-    const uint64_t win = (uint64_t)wid * kRefWindow;                    // its first slot
-    const uint64_t w0 = win >> 5;
-    for (int i = tid; i < HW; i += kRefThreads) {
-        const uint32_t h = head_cur[w0 + i];
-        s_ha[i] = h;
-        s_hb[i] = h;
-    }
-    if (tid < 2) s_n[tid] = 0;
-    __syncthreads();
-
-    // Ownership: this CTA sorts the groups whose head lies in [win, win+kRefWindow).
-    if (warp == 0) {
-        const uint32_t hw = s_ha[lane];
-        const uint32_t nz = __ballot_sync(0xffffffffu, hw != 0);
-        int start = -1, end = -1, big = 0;
-        if (nz) {
-            const int fl = __ffs(nz) - 1, ll = 31 - __clz(nz);
-            const uint32_t fw = __shfl_sync(0xffffffffu, hw, fl), lw = __shfl_sync(0xffffffffu, hw, ll);
-            start = fl * 32 + __ffs(fw) - 1;
-            const int hl = ll * 32 + 31 - __clz(lw); // head of the last owned group
-            // its end: first head at or after the window end
-            const uint32_t ew = s_ha[WIN_WORDS + lane];
-            const uint32_t enz = __ballot_sync(0xffffffffu, ew != 0);
-            int e = -1;
-            if (enz) {
-                const int el = __ffs(enz) - 1;
-                const uint32_t x = __shfl_sync(0xffffffffu, ew, el);
-                e = kRefWindow + el * 32 + __ffs(x) - 1;
-            }
-            if (e >= 0 && e - hl <= kRefGroupMax) {
-                end = e;
-            } else {
-                // the last group is too large for shared memory: leave it to the global path
-                end = hl;
-                big = 1;
-                if (lane == 0) {
-                    const uint32_t slot = atomicAdd(big_count, 1u);
-                    if (slot < big_cap) big_heads[slot] = (uint32_t)(win + hl);
-                }
-            }
-        }
-        if (lane == 0) {
-            s_range[0] = start;
-            s_range[1] = end;
-            s_range[2] = big;
-        }
-    }
-    __syncthreads();
-    const int start = s_range[0], end = s_range[1];
-    if (start < 0 || end <= start) return;
-
-    // Appends `slot` to list `which` for the lanes with `take` set (whole warp must call).
-    auto append = [&](int which, bool take, int slot) {
-        const uint32_t m = __ballot_sync(0xffffffffu, take);
-        if (m == 0) return;
-        int base = 0;
-        if (lane == 0) base = atomicAdd(&s_n[which], __popc(m));
-        base = __shfl_sync(0xffffffffu, base, 0);
-        if (take) s_list[which][base + __popc(m & lanemask_lt())] = (uint16_t)slot;
-    };
-    auto fetch_key = [&](int slot, uint64_t pos, uint32_t dd) {
-        if (KW == 2) {
-            uint64_t hi, lo;
-            text_window2<BITS>(packed, pos + dd, hi, lo);
-            s_khi[slot] = hi;
-            s_klo[slot] = lo;
-        } else {
-            s_khi[slot] = text_window<BITS>(packed, pos + dd);
-        }
-    };
-
-    // load the suffixes (and their BWT bytes) that sit in groups of >= 2, and their first keys
-    uint32_t d = depth;
-    for (int b0 = start + (tid & ~31); b0 < end; b0 += 4 * kRefThreads) { // b0 is warp-uniform (append ballots)
-        const int base = b0 + lane;
-        uint32_t sv[4];
-        uint8_t bv[4], hv[4];
-        bool act[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int r = base + u * kRefThreads;
-            act[u] = false;
-            bv[u] = 0;
-            hv[u] = 0;
-            sv[u] = 0;
-            if (r < end) {
-                const bool h0 = (s_ha[r >> 5] >> (r & 31)) & 1u;
-                const bool h1 = (s_ha[(r + 1) >> 5] >> ((r + 1) & 31)) & 1u;
-                act[u] = !(h0 && h1);
-                if (act[u]) {
-                    sv[u] = sa[win + r];
-                    if (bwt) bv[u] = bwt[win + r];
-                    if (WIDE) hv[u] = sa_hi[win + r];
-                }
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int r = base + u * kRefThreads;
-            if (act[u]) {
-                s_sa[0][r] = sv[u];
-                s_bw[0][r] = bv[u];
-                if (WIDE) s_hi[0][r] = hv[u];
-                fetch_key(r, WIDE ? (((uint64_t)hv[u] << lo_bits) | sv[u]) : (uint64_t)sv[u], d);
-            }
-            append(0, act[u], r);
-        }
-    }
-    __syncthreads();
-
-    int c = 0, lc = 0;
-    unsigned long long fetched = 0; // keys gathered from the text by this CTA (statistics)
-    for (int step = 0; step < max_steps; ++step) {
-        const int cnt = s_n[lc];
-        if (cnt == 0) break;
-        fetched += (unsigned)cnt;
-        if (tid == 0) s_n[lc ^ 1] = 0;
-        // rank: stable position inside the group; a suffix opens a new group iff no earlier member
-        // carries the same key (or its key holds the terminator, which makes it unique)
-        for (int i = tid; i < cnt; i += kRefThreads) {
-            const int r = s_list[lc][i];
-            const int gs = prev_set_le(s_ha, r);
-            const int ge = next_set_gt(s_ha, r);
-            const uint64_t mh = s_khi[r], ml = KW == 2 ? s_klo[r] : mh;
-            int lt = 0, eq = 0;
-            if (KW == 2) {
-                for (int j = gs; j < r; ++j) {
-                    const uint64_t oh = s_khi[j];
-                    if (oh < mh) {
-                        ++lt;
-                    } else if (oh == mh) {
-                        const uint64_t ol = s_klo[j];
-                        lt += ol < ml;
-                        eq += ol == ml;
-                    }
-                }
-                for (int j = r + 1; j < ge; ++j) {
-                    const uint64_t oh = s_khi[j];
-                    lt += (oh < mh) || (oh == mh && s_klo[j] < ml);
-                }
-            } else {
-                for (int j = gs; j < r; ++j) {
-                    const uint64_t o = s_khi[j];
-                    lt += o < mh;
-                    eq += o == mh;
-                }
-                for (int j = r + 1; j < ge; ++j) lt += s_khi[j] < mh;
-            }
-            const int p = gs + lt + eq;
-            if (p != gs && (eq == 0 || key_terminated<BITS>(ml))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
-            s_sa[c ^ 1][p] = s_sa[c][r];
-            s_bw[c ^ 1][p] = s_bw[c][r]; // the BWT symbol moves with its suffix
-            if (WIDE) s_hi[c ^ 1][p] = s_hi[c][r];
-            s_list[lc][i] = (uint16_t)p;  // where this suffix went
-        }
-        __syncthreads();
-        // classify: resolved suffixes go home now; the rest fetch the next key and form the next list
-        d += KW * Pack<BITS>::SPW;
-        const bool more_steps = step + 1 < max_steps;
-        for (int i = tid; (i & ~31) < cnt; i += kRefThreads) {
-            bool again = false;
-            int p = 0;
-            if (i < cnt) {
-                p = s_list[lc][i];
-                const bool h0 = (s_hb[p >> 5] >> (p & 31)) & 1u;
-                const bool h1 = (s_hb[(p + 1) >> 5] >> ((p + 1) & 31)) & 1u;
-                again = !(h0 && h1);
-                const uint32_t pos = s_sa[c ^ 1][p];
-                if (!again) {
-                    sa[win + p] = pos;
-                    if (bwt) bwt[win + p] = s_bw[c ^ 1][p];
-                    if (WIDE) sa_hi[win + p] = s_hi[c ^ 1][p];
-                } else if (more_steps) {
-                    fetch_key(p, WIDE ? (((uint64_t)s_hi[c ^ 1][p] << lo_bits) | pos) : (uint64_t)pos, d);
-                }
-            }
-            append(lc ^ 1, again, p);
-        }
-        for (int i = tid; i < HW; i += kRefThreads) s_ha[i] = s_hb[i]; // not read in this phase
-        c ^= 1;
-        lc ^= 1;
-        __syncthreads();
-    }
-
-    // single-step mode: unresolved suffixes are written back in their new order and handed to the next launch
-    const int left = s_n[lc];
-    bool mine_here = s_range[2] != 0 && tid == 0, mine_next = false;
-    for (int i = tid; i < left; i += kRefThreads) {
-        const int p = s_list[lc][i];
-        sa[win + p] = s_sa[c][p];
-        if (bwt) bwt[win + p] = s_bw[c][p];
-        if (WIDE) sa_hi[win + p] = s_hi[c][p];
-        // the group's head decides the owner: this window, or the next one if it lies in the overhang
-        if (prev_set_le(s_hb, p) >= kRefWindow) mine_next = true; else mine_here = true;
-    }
-    for (int i = tid; i < HW; i += kRefThreads) {
-        const uint32_t fresh = s_hb[i] & ~head_cur[w0 + i];
-        if (fresh) atomicOr(&head_next[w0 + i], fresh);
-    }
-    const int any_here = __syncthreads_or(mine_here);
-    const int any_next = __syncthreads_or(mine_next);
-    if (tid == 0) {
-        if (left) atomicAdd(&remaining[wid & 63], (unsigned long long)left);
-        if (fetched) atomicAdd(&remaining[64 + (wid & 63)], fetched);
-        if (any_here && atomicExch(&win_flag[wid], 1u) == 0u) win_next[atomicAdd(win_next_count, 1u)] = wid;
-        if (any_next && wid + 1 < nwin && atomicExch(&win_flag[wid + 1], 1u) == 0u)
-            win_next[atomicAdd(win_next_count, 1u)] = wid + 1;
-    }
-}
-
 // SPW-symbol window that starts `s` symbols into word x0 and runs on into x1, cut at the terminator
 template <int BITS> __device__ __forceinline__ uint64_t window_of(uint64_t x0, uint64_t x1, int s)
 {
@@ -1138,16 +867,21 @@ template <int BITS> __device__ __forceinline__ uint64_t window_of(uint64_t x0, u
 // ---------------------------------------------------------------------------
 // refinement with independent warps
 // ---------------------------------------------------------------------------
-// Same contract as the multi-step refine_kernel.  Groups never interact, so nothing forces the warps
-// of a CTA through the steps together: in refine_kernel every step costs two CTA-wide barriers and the
-// CTA runs as many steps as its slowest suffix needs, with most warps idle in the tail.  Here the CTA
-// only shares the window in shared memory.  Warp w owns the groups whose head lies in its 128-slot
-// part of the window -- a contiguous slot range [first head >= 128w, first head >= 128(w+1)) -- and
-// runs the rank / classify steps over that range on its own, synchronising with __syncwarp only.
+// One CTA owns the groups whose head lies in its window of kRefWindow slots and keeps refining them in
+// shared memory -- key = the next SPW symbols, stable rank inside the group, split -- until they are all
+// resolved.  The suffix array (and the BWT bytes that travel with it) are read once; a suffix is written
+// back the moment it becomes a singleton; only the text is touched again in every step.  A step is two phases:
+//   rank:     every unresolved suffix finds its stable rank inside its group, moves to the other buffer
+//             and marks the new group heads;
+//   classify: resolved suffixes go home; the others fetch their next key and stay on the list.
+// Groups never interact, so nothing forces the warps of a CTA through the steps together (CTA-wide steps
+// cost two barriers each and run as many steps as the slowest suffix needs, with most warps idle in the
+// tail): the CTA only shares the window in shared memory.  Warp w owns the groups whose head lies in its
+// 128-slot part of the window -- a contiguous slot range [first head >= 128w, first head >= 128(w+1)) --
+// and runs the rank / classify steps over that range on its own, synchronising with __syncwarp only.
 // Head bits of neighbouring ranges can share a 32-bit word: words are only ever OR-ed (atomically), a
 // warp publishes (head_b -> head_a) just the bits of its own range, and the bit scans stop at the
-// heads that bound the range, which are set from the start.  KW = 2 compares 2*SPW symbols per step
-// (128-bit keys): fewer steps per suffix, and every step has a fixed cost per suffix.
+// heads that bound the range, which are set from the start.
 constexpr int kRwGroupMax = kRefGroupMaxWarps;
 constexpr int kRwCap = kRefWindow + kRwGroupMax;
 // Groups of at least this many members are ranked by the whole warp at once.  In repetitive collections (high
@@ -1158,9 +892,8 @@ constexpr int kRwCap = kRefWindow + kRwGroupMax;
 // ranks only the others against each other: (0.3 g)^2 comparisons instead of g^2.
 constexpr int kRwBigGroup = 64;
 
-template <int KW, bool WIDE> struct RwSmem {
-    uint64_t khi[kRwCap];
-    uint64_t klo[KW == 2 ? kRwCap : 1];
+template <bool WIDE> struct RwSmem {
+    uint64_t key[kRwCap];              // the next SPW symbols of the suffix in each slot
     uint32_t sa[2][kRwCap];            // suffixes, double buffered across a step
     uint16_t list[kRwCap];             // unresolved slots of each warp's range, compacted in place
     uint8_t bw[2][kRwCap];             // BWT bytes travelling with the suffixes
@@ -1183,21 +916,17 @@ template <int KW, bool WIDE> struct RwSmem {
 // from reads overlapping the same stretch of a genome, and they agree on the symbol in front of it too.  Only
 // groups with mixed symbols are loaded and refined, and a group that becomes uniform after a split is dropped
 // at once.  (ORDER = true, DSMFM_FLAG_KEEP_SA: the full order, as needed for the .sa samples.)
-#ifndef DSMFM_RW_CTAS
-#define DSMFM_RW_CTAS 4
-#endif
-constexpr int kRwCtas = DSMFM_RW_CTAS; // resident CTAs per SM the compiler budgets registers for
+constexpr int kRwCtas = 4; // resident CTAs per SM the compiler budgets registers for
 // COOP: groups of big_thr members or more are ranked by the whole warp around their dominant key (a separate
 // instantiation: with both ranking schemes in one kernel the whole-warp path lost 10 % to the other's code).
-template <int BITS, int KW, bool WIDE, bool ORDER, bool COOP>
+template <int BITS, bool WIDE, bool ORDER, bool COOP>
 __global__ void __launch_bounds__(kRefThreads, kRwCtas)
 refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ sa, const uint32_t *__restrict__ head_cur,
                     uint32_t *__restrict__ head_next, uint64_t n, uint32_t depth, const uint32_t *__restrict__ win_list,
                     uint32_t *__restrict__ big_heads, uint32_t big_cap, uint32_t *__restrict__ big_count,
                     unsigned long long *__restrict__ remaining, uint32_t *__restrict__ win_flag,
                     uint32_t *__restrict__ win_next, uint32_t *__restrict__ win_next_count, uint8_t *__restrict__ bwt,
-                    uint8_t *__restrict__ sa_hi, int lo_bits, const uint32_t *__restrict__ diff_bits, int big_thr,
-                    bool chunked)
+                    uint8_t *__restrict__ sa_hi, int lo_bits, const uint32_t *__restrict__ diff_bits, int big_thr)
 {
     using P = Pack<BITS>;
     constexpr int HW = kRwCap / 32 + 2;
@@ -1207,8 +936,8 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
     constexpr int PART = kRefWindow / NWARP; // slots of the window whose heads one warp owns
     static_assert(WIN_WORDS == 32 && OVER_WORDS <= 32, "one warp scans the window / the overhang");
     extern __shared__ __align__(16) unsigned char ref_smem_raw[];
-    RwSmem<KW, WIDE> &S = *reinterpret_cast<RwSmem<KW, WIDE> *>(ref_smem_raw);
-    uint64_t *s_khi = S.khi, *s_klo = S.klo;
+    RwSmem<WIDE> &S = *reinterpret_cast<RwSmem<WIDE> *>(ref_smem_raw);
+    uint64_t *s_key = S.key;
     uint32_t(*s_sa)[kRwCap] = S.sa;
     uint8_t(*s_bw)[kRwCap] = S.bw;
     uint8_t(*s_hi)[WIDE ? kRwCap : 1] = S.hi;
@@ -1286,7 +1015,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
 
     // keys of up to four suffixes per lane: all text words are requested before the first one is used
     auto fetch4 = [&](const uint64_t (&pos)[4], const int (&slot)[4], uint32_t dd) {
-        uint64_t x0[4], x1[4], x2[4];
+        uint64_t x0[4], x1[4];
         int sh[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -1296,17 +1025,11 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                 sh[u] = (int)(q - w * P::SPW);
                 x0[u] = __ldg(packed + w);
                 x1[u] = __ldg(packed + w + 1);
-                if (KW == 2) x2[u] = __ldg(packed + w + 2);
             }
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            if (slot[u] >= 0) {
-                const uint64_t h = window_of<BITS>(x0[u], x1[u], sh[u]);
-                s_khi[slot[u]] = h;
-                // a terminator inside hi ends the suffix: nothing after it may be looked at
-                if (KW == 2) s_klo[slot[u]] = key_terminated<BITS>(h) ? 0ull : window_of<BITS>(x1[u], x2[u], sh[u]);
-            }
+            if (slot[u] >= 0) s_key[slot[u]] = window_of<BITS>(x0[u], x1[u], sh[u]);
         }
     };
 
@@ -1421,7 +1144,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
         // rank: stable position inside the group; a suffix opens a new group iff no earlier member
         // carries the same key (or its key holds the terminator, which makes it unique)
         int nbig = 0; // large groups of this warp's range seen in this step (warp-uniform)
-        if (!COOP && chunked) {
+        if (!COOP) {
             // Whole groups, as many as fit the 32 lanes, one member per lane.  The list holds whole groups in slot
             // order (it starts that way, and the classification below compacts it in order), so a group is a run of
             // lanes between two head flags; match.any finds the lanes that carry
@@ -1443,16 +1166,16 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                     const int ge = next_set_gt(s_ha, gs);
                     for (int ii = i0 + lane; ii < i0 + (ge - gs); ii += 32) {
                         const int rr = list[ii];
-                        const uint64_t mh = s_khi[rr], ml = KW == 2 ? s_klo[rr] : mh;
+                        const uint64_t mk = s_key[rr];
                         int lt = 0, eq = 0;
                         for (int j = gs; j < ge; ++j) {
-                            const uint64_t oh = s_khi[j], ol = KW == 2 ? s_klo[j] : oh;
-                            lt += (oh < mh) | ((oh == mh) & (ol < ml));
-                            eq += (oh == mh) & (ol == ml) & (j < rr);
+                            const uint64_t o = s_key[j];
+                            lt += o < mk;
+                            eq += (o == mk) & (j < rr);
                         }
                         const int p = gs + lt + eq;
-                        if (p != gs && (eq == 0 || key_terminated<BITS>(ml))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
-                        ghead[p] = (uint16_t)(key_terminated<BITS>(ml) ? p : gs + lt);
+                        if (p != gs && (eq == 0 || key_terminated<BITS>(mk))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
+                        ghead[p] = (uint16_t)(key_terminated<BITS>(mk) ? p : gs + lt);
                         s_sa[c ^ 1][p] = s_sa[c][rr];
                         s_bw[c ^ 1][p] = s_bw[c][rr];
                         if (WIDE) s_hi[c ^ 1][p] = s_hi[c][rr];
@@ -1467,28 +1190,25 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                 const uint32_t above = hb & ~upto & takemask;
                 const int el = above ? __ffs(above) - 1 : take;                  // one behind my group's last lane
                 const uint32_t gmask = (el >= 32 ? 0xffffffffu : ((1u << el) - 1)) & ~((1u << sl) - 1);
-                const uint64_t mh = valid ? s_khi[r] : 0ull, ml = KW == 2 ? (valid ? s_klo[r] : 0ull) : mh;
-                uint32_t E = __match_any_sync(0xffffffffu, mh);
-                if (KW == 2) E &= __match_any_sync(0xffffffffu, ml);
-                E &= gmask;
+                const uint64_t mk = valid ? s_key[r] : 0ull;
+                const uint32_t E = __match_any_sync(0xffffffffu, mk) & gmask;
                 const int eq = __popc(E & lanemask_lt());
                 int lt = 0;
                 uint32_t rem = in ? (gmask & ~E) : 0u; // members of my group with other keys
                 while (__any_sync(0xffffffffu, rem != 0)) {
                     const int l = rem ? __ffs(rem) - 1 : lane;
-                    const uint64_t kh = __shfl_sync(0xffffffffu, mh, l);
-                    const uint64_t kl = KW == 2 ? __shfl_sync(0xffffffffu, ml, l) : kh;
+                    const uint64_t kl = __shfl_sync(0xffffffffu, mk, l);
                     const uint32_t El = __shfl_sync(0xffffffffu, E, l);
                     if (rem) {
-                        if ((kh < mh) | ((kh == mh) & (kl < ml))) lt += __popc(El);
+                        if (kl < mk) lt += __popc(El);
                         rem &= ~El;
                     }
                 }
                 const int gs = __shfl_sync(0xffffffffu, r, sl);
                 if (in) {
                     const int p = gs + lt + eq;
-                    if (p != gs && (eq == 0 || key_terminated<BITS>(ml))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
-                    ghead[p] = (uint16_t)(key_terminated<BITS>(ml) ? p : gs + lt); // the equal ones start at gs + lt
+                    if (p != gs && (eq == 0 || key_terminated<BITS>(mk))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
+                    ghead[p] = (uint16_t)(key_terminated<BITS>(mk) ? p : gs + lt); // the equal ones start at gs + lt
                     s_sa[c ^ 1][p] = s_sa[c][r];
                     s_bw[c ^ 1][p] = s_bw[c][r]; // the BWT symbol moves with its suffix
                     if (WIDE) s_hi[c ^ 1][p] = s_hi[c][r];
@@ -1496,34 +1216,6 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                     // only need the set of slots -- in slot order, which the next step's lane runs rely on)
                 }
                 i0 += take;
-            }
-        } else if (!COOP) { // every group by its own members (all pairs)
-            for (int i = lane; i < cnt; i += 32) {
-                const int r = list[i];
-                const int gs = prev_set_le(s_ha, r);
-                const int ge = next_set_gt(s_ha, r);
-                const uint64_t mh = s_khi[r], ml = KW == 2 ? s_klo[r] : mh;
-                int lt = 0, eq = 0;
-                if (KW == 2) {
-                    for (int j = gs; j < ge; ++j) {
-                        const uint64_t oh = s_khi[j], ol = s_klo[j];
-                        lt += (oh < mh) | ((oh == mh) & (ol < ml));
-                        eq += (oh == mh) & (ol == ml) & (j < r);
-                    }
-                } else {
-                    for (int j = gs; j < r; ++j) {
-                        const uint64_t o = s_khi[j];
-                        lt += o < mh;
-                        eq += o == mh;
-                    }
-                    for (int j = r + 1; j < ge; ++j) lt += s_khi[j] < mh;
-                }
-                const int p = gs + lt + eq;
-                if (p != gs && (eq == 0 || key_terminated<BITS>(ml))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
-                ghead[p] = (uint16_t)(key_terminated<BITS>(ml) ? p : gs + lt); // the equal ones start at gs + lt
-                s_sa[c ^ 1][p] = s_sa[c][r];
-                s_bw[c ^ 1][p] = s_bw[c][r]; // the BWT symbol moves with its suffix
-                if (WIDE) s_hi[c ^ 1][p] = s_hi[c][r];
             }
         } else
         for (int i0 = 0; i0 < cnt; i0 += 32) {
@@ -1537,25 +1229,17 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                 if (ge - gs >= big_thr) {
                     big_first = r == gs; // the whole warp ranks this group below
                 } else {
-                    const uint64_t mh = s_khi[r], ml = KW == 2 ? s_klo[r] : mh;
+                    const uint64_t mk = s_key[r];
                     int lt = 0, eq = 0;
-                    if (KW == 2) {
-                        for (int j = gs; j < ge; ++j) {
-                            const uint64_t oh = s_khi[j], ol = s_klo[j];
-                            lt += (oh < mh) | ((oh == mh) & (ol < ml));
-                            eq += (oh == mh) & (ol == ml) & (j < r);
-                        }
-                    } else {
-                        for (int j = gs; j < r; ++j) {
-                            const uint64_t o = s_khi[j];
-                            lt += o < mh;
-                            eq += o == mh;
-                        }
-                        for (int j = r + 1; j < ge; ++j) lt += s_khi[j] < mh;
+                    for (int j = gs; j < r; ++j) {
+                        const uint64_t o = s_key[j];
+                        lt += o < mk;
+                        eq += o == mk;
                     }
+                    for (int j = r + 1; j < ge; ++j) lt += s_key[j] < mk;
                     const int p = gs + lt + eq;
-                    if (p != gs && (eq == 0 || key_terminated<BITS>(ml))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
-                    ghead[p] = (uint16_t)(key_terminated<BITS>(ml) ? p : gs + lt);
+                    if (p != gs && (eq == 0 || key_terminated<BITS>(mk))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
+                    ghead[p] = (uint16_t)(key_terminated<BITS>(mk) ? p : gs + lt);
                     s_sa[c ^ 1][p] = s_sa[c][r];
                     s_bw[c ^ 1][p] = s_bw[c][r]; // the BWT symbol moves with its suffix
                     if (WIDE) s_hi[c ^ 1][p] = s_hi[c][r];
@@ -1571,7 +1255,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
             const int ge = next_set_gt(s_ha, gs);
             const int g = ge - gs;
             // candidate for the dominant key: the member in the middle of the group
-            const uint64_t ch = s_khi[gs + (g >> 1)], cl = KW == 2 ? s_klo[gs + (g >> 1)] : 0ull;
+            const uint64_t ck = s_key[gs + (g >> 1)];
             __syncwarp();
             // pass 1: classes.  The members that do not carry the candidate key are compacted, in slot order, to
             // the front of the group's own key slots (a key is read by its lane before anything of its chunk is
@@ -1580,13 +1264,12 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
             for (int b0 = gs; b0 < ge; b0 += 32) {
                 const int r = b0 + lane;
                 const bool in = r < ge;
-                uint64_t mh = 0, ml = 0;
+                uint64_t mk = 0;
                 bool is_eq = false, is_lt = false;
                 if (in) {
-                    mh = s_khi[r];
-                    ml = KW == 2 ? s_klo[r] : 0ull;
-                    is_eq = mh == ch && ml == cl;
-                    is_lt = mh < ch || (KW == 2 && mh == ch && ml < cl);
+                    mk = s_key[r];
+                    is_eq = mk == ck;
+                    is_lt = mk < ck;
                 }
                 const uint32_t eqm = __ballot_sync(0xffffffffu, is_eq), ltm = __ballot_sync(0xffffffffu, is_lt);
                 const uint32_t ndm = __ballot_sync(0xffffffffu, in && !is_eq);
@@ -1595,8 +1278,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                     const int t = gs + n_nd + __popc(ndm & lanemask_lt());
                     S.newpos[r] = 0xffffu; // not a carrier of the candidate key
                     S.nd[t] = (uint16_t)r;
-                    s_khi[t] = mh;
-                    if (KW == 2) s_klo[t] = ml;
+                    s_key[t] = mk;
                 }
                 n_eq += __popc(eqm);
                 n_lt += __popc(ltm);
@@ -1604,7 +1286,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
                 __syncwarp();
             }
             // the carriers of the candidate key: their stable rank is their running count, no comparisons at all
-            const bool term = key_terminated<BITS>(KW == 2 ? cl : ch);
+            const bool term = key_terminated<BITS>(ck);
             for (int r = gs + lane; r < ge; r += 32) {
                 const int e = S.newpos[r];
                 if (e != 0xffff) {
@@ -1619,20 +1301,19 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
             // the others against each other (dense keys in the first n_nd key slots of the group)
             for (int t = lane; t < n_nd; t += 32) {
                 const int r = S.nd[gs + t];
-                const uint64_t mh = s_khi[gs + t], ml = KW == 2 ? s_klo[gs + t] : 0ull;
+                const uint64_t mk = s_key[gs + t];
                 int lt = 0, eq = 0;
                 for (int u = 0; u < n_nd; ++u) {
-                    const uint64_t oh = s_khi[gs + u], ol = KW == 2 ? s_klo[gs + u] : 0ull;
-                    lt += (oh < mh) | ((oh == mh) & (ol < ml));
-                    eq += (oh == mh) & (ol == ml) & (u < t);
+                    const uint64_t o = s_key[gs + u];
+                    lt += o < mk;
+                    eq += (o == mk) & (u < t);
                 }
-                const bool above = mh > ch || (KW == 2 && mh == ch && ml > cl);
-                const int p = gs + lt + eq + (above ? n_eq : 0);
-                if (p != gs && (eq == 0 || key_terminated<BITS>(KW == 2 ? ml : mh))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
+                const int p = gs + lt + eq + (mk > ck ? n_eq : 0);
+                if (p != gs && (eq == 0 || key_terminated<BITS>(mk))) atomicOr(&s_hb[p >> 5], 1u << (p & 31));
                 s_sa[c ^ 1][p] = s_sa[c][r];
                 s_bw[c ^ 1][p] = s_bw[c][r];
                 if (WIDE) s_hi[c ^ 1][p] = s_hi[c][r];
-                ghead[p] = (uint16_t)(key_terminated<BITS>(KW == 2 ? ml : mh) ? p : p - eq);
+                ghead[p] = (uint16_t)(key_terminated<BITS>(mk) ? p : p - eq);
             }
             __syncwarp();
         }
@@ -1650,7 +1331,7 @@ refine_warps_kernel(const uint64_t *__restrict__ packed, uint32_t *__restrict__ 
         }
         // classify: resolved suffixes go home now; the rest stay on the list (compacted in place: an entry
         // is written at or before the position it was read from, and a warp reads 32 entries before it writes)
-        d += KW * P::SPW;
+        d += P::SPW;
         int next = 0;
         for (int i = lane; (i & ~31) < cnt; i += 32) {
             bool again = false;
@@ -2920,19 +2601,6 @@ void launch_pack(cudaStream_t st, int bits, const uint8_t *raw, uint64_t n, cons
     if (launches) ++*launches;
 }
 
-void launch_make_keys(cudaStream_t st, int bits, const uint64_t *packed, uint64_t n, uint64_t *keys, int first_syms,
-                      bool carry_prev, uint32_t *launches)
-{
-    const int drop_bits = (64 / bits - first_syms) * bits;
-    const int key_bits = first_syms * bits;
-#define CALL(B) \
-    make_keys_kernel<B><<<grid_for(n, 256 * 8), 256, 0, st>>>(packed, n, keys, drop_bits, key_bits, carry_prev)
-    DISPATCH_BITS(bits, CALL);
-#undef CALL
-    DSM_LAUNCH_CHECK();
-    if (launches) ++*launches;
-}
-
 // The fast kernels classify by the top 12 key bits; they apply when the first key has at least 12 bits
 // and at least TopBits::SYMS symbols (always, except under DSMFM_FIRST_KEY_BITS experiments).
 static bool select_fast_ok(int bits, int first_syms, int top_bits)
@@ -3056,17 +2724,9 @@ void launch_heads(cudaStream_t st, int bits, const uint64_t *sorted_keys, uint64
                   uint64_t head_words, unsigned long long *remaining, int key_bits, const uint8_t *inv_map,
                   uint8_t *bwt, uint8_t *pos_hi, int hi_shift, uint32_t *diff, uint32_t *launches)
 {
-    // ranks per warp iteration: 128 or 256 (DSMFM_HEADS_U=4|8: eight key loads in flight per lane instead of four)
-    static const int u_env = std::getenv("DSMFM_HEADS_U") ? std::atoi(std::getenv("DSMFM_HEADS_U")) : kHeadsU;
 #define CALL(B)                                                                                                      \
-    do {                                                                                                             \
-        if (u_env == 8)                                                                                              \
-            heads_kernel<B, 8><<<grid_for(head_words, 8 * 16), 256, 0, st>>>(sorted_keys, n, head, head_words, remaining, \
-                                                                             key_bits, inv_map, bwt, pos_hi, hi_shift, diff); \
-        else                                                                                                         \
-            heads_kernel<B, 4><<<grid_for(head_words, 8 * 16), 256, 0, st>>>(sorted_keys, n, head, head_words, remaining, \
-                                                                             key_bits, inv_map, bwt, pos_hi, hi_shift, diff); \
-    } while (0)
+    heads_kernel<B><<<grid_for(head_words, 8 * 16), 256, 0, st>>>(sorted_keys, n, head, head_words, remaining, key_bits, \
+                                                                   inv_map, bwt, pos_hi, hi_shift, diff)
     DISPATCH_BITS(bits, CALL);
 #undef CALL
     DSM_LAUNCH_CHECK();
@@ -3076,98 +2736,52 @@ void launch_heads(cudaStream_t st, int bits, const uint64_t *sorted_keys, uint64
 void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
                    uint32_t *head_next, uint64_t n, uint32_t depth, const uint32_t *win_list, uint32_t n_list,
                    uint32_t *big_heads, uint32_t big_cap, uint32_t *big_count, unsigned long long *remaining,
-                   uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, bool multi_step,
-                   int key_words, uint8_t *sa_hi, int lo_bits, bool full_order, const uint32_t *diff_bits,
-                   uint32_t *launches, bool big_groups)
+                   uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, uint8_t *sa_hi,
+                   int lo_bits, bool full_order, const uint32_t *diff_bits, uint32_t *launches, bool big_groups)
 {
-    const uint32_t nwin = (uint32_t)div_up(n, kRefWindow);
-    const int max_steps = multi_step ? (1 << 30) : 1;
+    const unsigned grid = win_list ? n_list : (unsigned)div_up(n, kRefWindow);
+    if (grid == 0) return;
+    // groups of at least big_thr members are ranked by the whole warp around their dominant key
+    // (DSMFM_REFINE_BIG=<members>; 0 or unset: every group by its own members)
+    // -- the default when the refinement runs in place, i.e. when most suffixes sit in groups that have to be
+    // sorted (high repetition: C5 refinement 118 -> 98 ms); on the dense arrays of a read collection with few
+    // large groups the per-member path is the faster one (C3: 25.2 vs 26.6 ms).
+    const char *big_str = std::getenv("DSMFM_REFINE_BIG"); // (read per launch: the tests switch it)
+    const int big_env = big_str ? std::atoi(big_str) : -1;
+    const int big_want = big_env >= 0 ? big_env : (big_groups ? kRwBigGroup : 0);
+    const int big_thr = big_want >= 32 ? (big_want < kRwBigGroup ? kRwBigGroup : big_want) : kRwCap + 1;
     static DeviceOnce attr_once;
     attr_once.run([] {
-#define SET(B, K)                                                                                             \
-    DSM_CUDA(cudaFuncSetAttribute(refine_kernel<B, K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,    \
-                                  (int)sizeof(RefSmem<K, false>)));                                           \
-    DSM_CUDA(cudaFuncSetAttribute(refine_kernel<B, K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
-                                  (int)sizeof(RefSmem<K, true>)))
-        SET(3, 1); SET(4, 1); SET(8, 1); SET(3, 2); SET(4, 2); SET(8, 2);
+#define SET2(B, W, O)                                                                                                 \
+    DSM_CUDA(cudaFuncSetAttribute(refine_warps_kernel<B, W, O, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                  (int)sizeof(RwSmem<W>)));                                                         \
+    DSM_CUDA(cudaFuncSetAttribute(refine_warps_kernel<B, W, O, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
+                                  (int)sizeof(RwSmem<W>)))
+#define SET(B) SET2(B, false, false); SET2(B, true, false); SET2(B, false, true); SET2(B, true, true)
+        SET(3); SET(4); SET(8);
 #undef SET
+#undef SET2
     });
-    const unsigned grid = win_list ? n_list : nwin;
-    if (grid == 0) return;
-    // default schedule: multi-step with the text of the unresolved suffixes resident in shared memory
-    const char *variant_env = std::getenv("DSMFM_REFINE_VARIANT"); // 0: CTA-wide steps (refine_kernel), 2: independent warps
-    const int variant = variant_env ? std::atoi(variant_env) : 2;
-    if (multi_step && variant == 2) {
-        // groups of at least big_thr members are ranked by the whole warp around their dominant key
-        // (DSMFM_REFINE_BIG=<members>; 0 or unset: every group by its own members)
-        // -- the default when the refinement runs in place, i.e. when most suffixes sit in groups that have to be
-        // sorted (high repetition: C5 refinement 118 -> 98 ms); on the dense arrays of a read collection with few
-        // large groups the per-member path is the faster one (C3: 25.2 vs 26.6 ms).
-        const char *big_str = std::getenv("DSMFM_REFINE_BIG"); // (read per launch: the tests switch it)
-        const int big_env = big_str ? std::atoi(big_str) : -1;
-        const int big_want = big_env >= 0 ? big_env : (big_groups ? kRwBigGroup : 0);
-        const int big_thr = big_want >= 32 ? (big_want < kRwBigGroup ? kRwBigGroup : big_want) : kRwCap + 1;
-        // groups of up to 32 members are ranked a warp-load of whole groups at a time (match.any; DSMFM_REFINE_RANK=0:
-        // every member loops over its group)
-        const char *rank_str = std::getenv("DSMFM_REFINE_RANK");
-        const bool chunked = !(rank_str && std::atoi(rank_str) == 0);
-        static DeviceOnce attr3_once;
-        attr3_once.run([] {
-#define SET3(B, K)                                                                                                      \
-    SET4(B, K, false, false); SET4(B, K, true, false); SET4(B, K, false, true); SET4(B, K, true, true)
-#define SET4(B, K, W, O)                                                                                                \
-    DSM_CUDA(cudaFuncSetAttribute(refine_warps_kernel<B, K, W, O, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                  (int)sizeof(RwSmem<K, W>)));                                                          \
-    DSM_CUDA(cudaFuncSetAttribute(refine_warps_kernel<B, K, W, O, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                                  (int)sizeof(RwSmem<K, W>)))
-            SET3(3, 1); SET3(4, 1); SET3(8, 1); SET3(3, 2); SET3(4, 2); SET3(8, 2);
-#undef SET4
-#undef SET3
-        });
-#define RW3(B, K, W, O, C)                                                                                        \
-    refine_warps_kernel<B, K, W, O, C><<<grid, kRefThreads, sizeof(RwSmem<K, W>), st>>>(                          \
+#define RW2(B, W, O, C)                                                                                           \
+    refine_warps_kernel<B, W, O, C><<<grid, kRefThreads, sizeof(RwSmem<W>), st>>>(                                \
         packed, sa, head_cur, head_next, n, depth, win_list, big_heads, big_cap, big_count, remaining, win_flag,  \
-        win_next, win_next_count, bwt, sa_hi, lo_bits, diff_bits, big_thr, chunked)
-#define RW2(B, K, W, O)                                                                                           \
+        win_next, win_next_count, bwt, sa_hi, lo_bits, diff_bits, big_thr)
+#define RW(B, W, O)                                                                                               \
     do {                                                                                                          \
-        if (big_thr <= kRwCap) RW3(B, K, W, O, true); else RW3(B, K, W, O, false);                                \
+        if (big_thr <= kRwCap) RW2(B, W, O, true); else RW2(B, W, O, false);                                      \
     } while (0)
-#define RW(B, K, W)                                                                                               \
+#define CALL(B)                                                                                                   \
     do {                                                                                                          \
-        if (full_order || !bwt) RW2(B, K, W, true); else RW2(B, K, W, false);                                     \
-    } while (0)
-#define CALL3(B)                                                                                                  \
-    do {                                                                                                          \
-        if (key_words == 2) {                                                                                     \
-            if (sa_hi) RW(B, 2, true); else RW(B, 2, false);                                                      \
+        if (full_order || !bwt) {                                                                                 \
+            if (sa_hi) RW(B, true, true); else RW(B, false, true);                                                \
         } else {                                                                                                  \
-            if (sa_hi) RW(B, 1, true); else RW(B, 1, false);                                                      \
+            if (sa_hi) RW(B, true, false); else RW(B, false, false);                                              \
         }                                                                                                         \
-    } while (0)
-        DISPATCH_BITS(bits, CALL3);
-#undef CALL3
-#undef RW
-#undef RW2
-#undef RW3
-        DSM_LAUNCH_CHECK();
-        if (launches) ++*launches;
-        return;
-    }
-#define REFINE(B, K, W)                                                                                             \
-    refine_kernel<B, K, W><<<grid, kRefThreads, sizeof(RefSmem<K, W>), st>>>(                                       \
-        packed, sa, head_cur, head_next, n, depth, win_list, big_heads, big_cap, big_count, remaining, win_flag,   \
-        win_next, win_next_count, nwin, bwt, max_steps, sa_hi, lo_bits)
-#define CALL(B)                                                                                                     \
-    do {                                                                                                            \
-        if (key_words == 2) {                                                                                       \
-            if (sa_hi) REFINE(B, 2, true); else REFINE(B, 2, false);                                                \
-        } else {                                                                                                    \
-            if (sa_hi) REFINE(B, 1, true); else REFINE(B, 1, false);                                                \
-        }                                                                                                           \
     } while (0)
     DISPATCH_BITS(bits, CALL);
 #undef CALL
-#undef REFINE
+#undef RW
+#undef RW2
     DSM_LAUNCH_CHECK();
     if (launches) ++*launches;
 }

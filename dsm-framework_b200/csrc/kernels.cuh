@@ -28,10 +28,7 @@ void launch_pack(cudaStream_t st, int bits, const uint8_t *raw, uint64_t n, cons
 // ---- suffix sorting ---------------------------------------------------------
 // key[p] = the first `first_syms` (<= SPW) symbols of suffix p, cut at its terminator, right-aligned.
 // With carry_prev the code of the symbol before the suffix rides in the BITS bits above the key.
-void launch_make_keys(cudaStream_t st, int bits, const uint64_t *packed, uint64_t n, uint64_t *keys, int first_syms,
-                      bool carry_prev, uint32_t *launches);
-
-// The same keys plus, in ghist[pass][256] (zeroed u64), the counts of their 8-bit digits from bit 0 up to
+// Also, in ghist[pass][256] (zeroed u64), the counts of the keys' 8-bit digits from bit 0 up to
 // first_syms*bits -- the histogram the LSD sort needs (radix_sort_pairs with hist_ready).
 // word_begin / word_end (0 = all): only the suffixes starting in these words of the packed text -- a text that
 // streams in from the host is keyed piece by piece; the word behind the last one must already be packed.
@@ -80,23 +77,23 @@ void launch_heads(cudaStream_t st, int bits, const uint64_t *sorted_keys, uint64
 
 constexpr int kRefThreads = 256;
 constexpr int kRefWindow = 1024;   // group heads owned by one CTA lie in a window of this many slots
-constexpr int kRefGroupMax = 1024; // larger groups go through the global path
-constexpr int kRefCap = kRefWindow + kRefGroupMax;
-constexpr int kRefGroupMaxWarps = 768; // the same limit in the default (independent-warps) schedule
+constexpr int kRefGroupMaxWarps = 768; // larger groups go through the global path
+// Slots of the head bitmap behind the last suffix (head_words_for), more than a window plus its largest
+// group can reach; it also bounds a sort range: fewer than 2^32 - kRefCap - 64 suffixes.
+constexpr int kRefCap = 2048;
 
 inline uint64_t head_words_for(uint64_t n) { return div_up(n, 32) + kRefCap / 32 + 8; }
 
 // One refinement round: every group of >= 2 suffixes that still agree on their
 // first `depth` symbols is sorted (stably) by the next SPW symbols and split.
-// head_next must hold a copy of head_cur.  Groups larger than kRefGroupMax are
+// head_next must hold a copy of head_cur.  Groups larger than kRefGroupMaxWarps are
 // left untouched and their head slots appended to big_heads.  win_list (n_list
 // entries; nullptr = every window) names the windows to visit; windows that
 // still own unresolved groups afterwards are appended to win_next (deduplicated
 // through the zeroed win_flag array, one u32 per window).  If bwt != nullptr the BWT bytes
-// (one per rank) are permuted together with the suffix array.  With multi_step a CTA keeps
-// extending the keys (depth += SPW) until every group it owns is resolved, so that one launch
-// finishes everything except the groups that do not fit a CTA.  key_words = 1 or 2: a step compares
-// SPW or 2*SPW symbols (64- or 128-bit keys).  full_order = false (default schedule, needs bwt): groups whose
+// (one per rank) are permuted together with the suffix array.  A CTA keeps extending the keys
+// (depth += SPW) until every group it owns is resolved, so that one launch finishes everything
+// except the groups that do not fit a CTA.  full_order = false (default schedule, needs bwt): groups whose
 // members all carry the same BWT symbol are left as they are -- their order cannot change the BWT -- so the
 // suffix array is then only sorted as far as the BWT needs it.  diff_bits: launch_heads' bitmap while it is
 // still valid (first launch after the initial sort), nullptr afterwards (the kernel then compares the bytes).
@@ -104,9 +101,8 @@ inline uint64_t head_words_for(uint64_t n) { return div_up(n, 32) + kRefCap / 32
 void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
                    uint32_t *head_next, uint64_t n, uint32_t depth, const uint32_t *win_list, uint32_t n_list,
                    uint32_t *big_heads, uint32_t big_cap, uint32_t *big_count, unsigned long long *remaining,
-                   uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, bool multi_step,
-                   int key_words, uint8_t *sa_hi, int lo_bits, bool full_order, const uint32_t *diff_bits,
-                   uint32_t *launches, bool big_groups = false);
+                   uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, uint8_t *sa_hi,
+                   int lo_bits, bool full_order, const uint32_t *diff_bits, uint32_t *launches, bool big_groups = false);
 
 // BWT-only builds: the groups with mixed BWT symbols, copied out in order so that the refinement works on dense
 // arrays.  launch_mark_active: act (zeroed, head_words words) gets the slots of those groups (diff is read 16 bytes

@@ -1,8 +1,6 @@
 // radix_sort.cu -- one-sweep LSD radix sort kernels (see radix_sort.cuh).
 #include "radix_sort.cuh"
 
-#include <cstdlib>
-
 namespace dsmfm {
 
 namespace {
@@ -79,15 +77,15 @@ __global__ void __launch_bounds__(kRadix) radix_scan_kernel(uint64_t *__restrict
     h[tid] = base + incl - v;
 }
 
-template <int WARPS> struct SweepSmemT {
+struct SweepSmem {
     uint64_t keys[kSweepTile];                 // tile in sorted order
     uint32_t vals[kSweepTile];
     uint64_t goff[kRadix];                     // global offset of digit run minus its tile-local start
-    uint16_t cnt[WARPS][kRadix];               // per-warp digit counters -> per-warp digit bases (<= tile size)
+    uint16_t cnt[kSweepThreads / 32][kRadix];  // per-warp digit counters -> per-warp digit bases (<= tile size)
     uint32_t excl[kRadix];                     // tile-local start of each digit run
     uint32_t warp_sum[kRadix / 32];
     uint32_t tile;
-    alignas(8) uint64_t mbar[2];               // TMA ingest: completion barriers of the tile's bulk copies (keys, values)
+    alignas(8) uint64_t mbar;                  // completion barrier of the bulk copy of the tile's keys
 };
 
 // ---- TMA (bulk async copy) helpers: cp.async.bulk + mbarrier, sm_90+ PTX ----
@@ -120,37 +118,31 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t phase)
 // -> publish the tile's digit counts -> stage keys in sorted order in shared memory -> fetch values
 // while the look-back over the preceding tiles resolves the global offsets -> stage values -> write
 // both out, one contiguous burst per digit.  Key registers die before the values are fetched.
-// Two shapes of the same tile: 256 threads x 16 pairs (64 registers, 4 CTAs = 32 warps per SM) and
-// 512 threads x 8 pairs (fewer registers per thread: 3 CTAs = 48 warps per SM); the kernel is bound by
-// latency (shared-memory round trips of the ranking, DRAM loads), not by issue slots or bandwidth,
-// so the warps in flight are what counts.  Threads 0..255 own one digit each in the scan / look-back phases.
-// TMA: a whole tile's keys arrive by ONE bulk asynchronous copy (cp.async.bulk, the 1-D form of TMA) into the very
+// 256 threads x 16 pairs: 64 registers, 4 CTAs = 32 warps per SM.  The kernel is bound by latency
+// (shared-memory round trips of the ranking, DRAM loads), not by issue slots or bandwidth, so the warps in
+// flight are what counts.  Threads 0..255 own one digit each in the scan / look-back phases.
+// A whole tile's keys arrive by ONE bulk asynchronous copy (cp.async.bulk, the 1-D form of TMA) into the very
 // staging buffer the sorted keys overwrite later, signalled through an mbarrier; the threads then take their keys
 // from shared memory (16 conflict-free LDS.64 instead of 16 predicated LDG.64 with their address arithmetic).
-template <bool IOTA, bool HW_MATCH, int THREADS, int ITEMS, bool HINTS, bool TMA = false>
-__global__ void __launch_bounds__(THREADS, THREADS == 256 ? kSweepCtasPerSm : (kSweepTile > 4096 ? 2 : 3))
+// The partial last tile of a portion loads its keys from global memory.
+template <bool IOTA>
+__global__ void __launch_bounds__(kSweepThreads, kSweepCtasPerSm)
 onesweep_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__restrict__ vals_in,
                 uint64_t *__restrict__ keys_out, uint32_t *__restrict__ vals_out, uint32_t n, uint64_t iota_base,
                 int shift, uint32_t mask, const uint64_t *__restrict__ base_in, uint64_t *__restrict__ base_out,
                 volatile uint32_t *status, uint32_t *counter, uint32_t last_tile)
 {
-    static_assert(THREADS * ITEMS == kSweepTile && THREADS >= kRadix, "one tile, at least one thread per digit");
-    constexpr int WARPS = THREADS / 32;
+    constexpr int THREADS = kSweepThreads, ITEMS = kSweepItems, WARPS = THREADS / 32;
+    static_assert(THREADS * ITEMS == kSweepTile && THREADS == kRadix, "one tile, one thread per digit");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    SweepSmemT<WARPS> &s = *reinterpret_cast<SweepSmemT<WARPS> *>(smem_raw);
+    SweepSmem &s = *reinterpret_cast<SweepSmem *>(smem_raw);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     if (tid == 0) {
         s.tile = atomicAdd(counter, 1u);
-        if (TMA) {
-            mbar_init(&s.mbar[0], 1);
-            mbar_init(&s.mbar[1], 1);
-            const uint32_t t0 = s.tile * (uint32_t)kSweepTile;
-            if (n - t0 >= (uint32_t)kSweepTile) { // whole tiles only
-                bulk_load(s.keys, keys_in + t0, kSweepTile * 8, &s.mbar[0]);
-                if (!IOTA && kSweepTmaVals) bulk_load(s.vals, vals_in + t0, kSweepTile * 4, &s.mbar[1]);
-            }
-        }
+        mbar_init(&s.mbar, 1);
+        const uint32_t t0 = s.tile * (uint32_t)kSweepTile;
+        if (n - t0 >= (uint32_t)kSweepTile) bulk_load(s.keys, keys_in + t0, kSweepTile * 8, &s.mbar); // whole tiles only
     }
     for (int i = tid; i < WARPS * kRadix / 2; i += THREADS) reinterpret_cast<uint32_t *>(&s.cnt[0][0])[i] = 0;
     __syncthreads();
@@ -162,24 +154,22 @@ onesweep_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__restrict
     // warp-striped load: item k of lane l is element first + 32k, so the order
     // (warp, k, lane) is the input order and the ranking below is stable
     uint64_t key[ITEMS];
-    if (TMA && valid == (uint32_t)kSweepTile) {
-        mbar_wait(&s.mbar[0], 0);
+    if (valid == (uint32_t)kSweepTile) {
+        mbar_wait(&s.mbar, 0);
 #pragma unroll
         for (int k = 0; k < ITEMS; ++k) key[k] = s.keys[warp * (32 * ITEMS) + 32 * k + lane];
     } else
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) {
         const uint32_t idx = first + 32 * k;
-        // (HINTS: every pair is read once and written once per pass -- evict-first loads, streaming stores)
-        key[k] = idx < n ? (HINTS ? __ldcs(reinterpret_cast<const unsigned long long *>(keys_in) + idx) : keys_in[idx])
-                         : ~0ull; // padding sorts to the very end of the tile
+        key[k] = idx < n ? keys_in[idx] : ~0ull; // padding sorts to the very end of the tile
     }
 
     uint16_t lpos[ITEMS];
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) {
         const uint32_t d = (uint32_t)(key[k] >> shift) & mask;
-        const uint32_t peers = HW_MATCH ? __match_any_sync(0xffffffffu, d) : match_digit(d);
+        const uint32_t peers = match_digit(d);
         const int leader = __ffs(peers) - 1;
         uint32_t old = 0;
         if (lane == leader) {
@@ -240,21 +230,13 @@ onesweep_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__restrict
 
     // values are fetched now so that their latency overlaps the look-back
     uint32_t val[ITEMS];
-    // (the values by bulk copy as well: measured 3.02 ms per launch against 2.98 with the keys alone -- the extra
-    // barrier between taking them out of the buffer and permuting them into it costs what the earlier fetch gains)
-    const bool vals_in_smem = kSweepTmaVals && TMA && !IOTA && valid == (uint32_t)kSweepTile;
-    if (vals_in_smem) {
-        mbar_wait(&s.mbar[1], 0);
-#pragma unroll
-        for (int k = 0; k < ITEMS; ++k) val[k] = s.vals[warp * (32 * ITEMS) + 32 * k + lane];
-    } else
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) {
         const uint32_t idx = first + 32 * k;
         if (IOTA)
             val[k] = (uint32_t)(iota_base + idx);
         else
-            val[k] = idx < n ? (HINTS ? __ldcs(vals_in + idx) : vals_in[idx]) : 0u;
+            val[k] = idx < n ? vals_in[idx] : 0u;
     }
 
     // decoupled look-back, one chain per digit, four predecessors in flight at a time
@@ -289,7 +271,6 @@ onesweep_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__restrict
         if (tile == last_tile) base_out[tid] = gbase + pub;
     }
 
-    if (vals_in_smem) __syncthreads(); // everybody has taken its values out of the buffer they are now permuted into
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) s.vals[lpos[k]] = val[k];
     __syncthreads();
@@ -299,13 +280,8 @@ onesweep_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__restrict
         const uint64_t kk = s.keys[i];
         const uint32_t d = (uint32_t)(kk >> shift) & mask;
         const uint64_t o = s.goff[d] + i;
-        if (HINTS) {
-            __stcs(reinterpret_cast<unsigned long long *>(keys_out) + o, (unsigned long long)kk);
-            __stcs(vals_out + o, s.vals[i]);
-        } else {
-            keys_out[o] = kk;
-            vals_out[o] = s.vals[i];
-        }
+        keys_out[o] = kk;
+        vals_out[o] = s.vals[i];
     }
 }
 
@@ -345,41 +321,15 @@ int radix_sort_pairs(cudaStream_t stream, RadixWorkspace &ws, uint64_t *keys_a, 
     if (n >= (1ull << 32)) throw CudaError{cudaErrorInvalidValue, "radix_sort_pairs: 2^32 pairs or more", __FILE__, __LINE__};
     if (div_up(n < kSweepPortion ? n : kSweepPortion, kSweepTile) > ws.status_tiles)
         throw CudaError{cudaErrorInvalidValue, "radix_sort_pairs: workspace too small", __FILE__, __LINE__};
+    if ((reinterpret_cast<uintptr_t>(keys_a) & 15) != 0 || (reinterpret_cast<uintptr_t>(keys_b) & 15) != 0)
+        throw CudaError{cudaErrorInvalidValue, "radix_sort_pairs: key arrays not 16-byte aligned", __FILE__, __LINE__};
 
     static DeviceOnce attr_once;
-    static const bool hw_match = [] { // experiment: match.any instead of the ballot rounds
-        const char *e = getenv("DSMFM_SWEEP_MATCH");
-        return e && atoi(e) != 0;
-    }();
-    static const bool hints = [] { // evict-first loads and streaming stores (DSMFM_SWEEP_HINTS=0|1)
-        const char *e = getenv("DSMFM_SWEEP_HINTS");
-        return e ? atoi(e) != 0 : kSweepHintsDefault;
-    }();
-    static const bool tma = [] { // the tile's keys by one bulk asynchronous copy (DSMFM_SWEEP_TMA=0|1)
-        const char *e = getenv("DSMFM_SWEEP_TMA");
-        return e ? atoi(e) != 0 : kSweepTmaDefault;
-    }();
-    static const bool wide_cta = [] { // 512 threads x 8 pairs instead of 256 x 16 (DSMFM_SWEEP_THREADS=256|512)
-        const char *e = getenv("DSMFM_SWEEP_THREADS");
-        return e ? atoi(e) == 512 : kSweepWideDefault;
-    }();
     attr_once.run([] {
-#define ATTR1(I, M, T, N, H)                                                                                      \
-    DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<I, M, T, N, H>, cudaFuncAttributeMaxDynamicSharedMemorySize,    \
-                                  (int)sizeof(SweepSmemT<T / 32>)));                                              \
-    DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<I, M, T, N, H>, cudaFuncAttributePreferredSharedMemoryCarveout, 100))
-#define ATTR(I, M, T, N) ATTR1(I, M, T, N, false); ATTR1(I, M, T, N, true)
-        DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<false, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)sizeof(SweepSmemT<kSweepTmaThreads / 32>)));
-        DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<false, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<true, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)sizeof(SweepSmemT<kSweepTmaThreads / 32>)));
-        DSM_CUDA(cudaFuncSetAttribute(onesweep_kernel<true, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        ATTR(true, false, kSweepNarrow, kSweepTile / kSweepNarrow); ATTR(false, false, kSweepNarrow, kSweepTile / kSweepNarrow);
-        ATTR(true, true, kSweepNarrow, kSweepTile / kSweepNarrow); ATTR(false, true, kSweepNarrow, kSweepTile / kSweepNarrow);
-        ATTR(true, false, 512, kSweepTile / 512);  ATTR(false, false, 512, kSweepTile / 512);  ATTR(true, true, 512, kSweepTile / 512);  ATTR(false, true, 512, kSweepTile / 512);
-#undef ATTR
-#undef ATTR1
+        for (auto kernel : {onesweep_kernel<false>, onesweep_kernel<true>}) {
+            DSM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+            DSM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        }
     });
 
     if (!hist_ready) {
@@ -409,38 +359,10 @@ int radix_sort_pairs(cudaStream_t stream, RadixWorkspace &ws, uint64_t *keys_a, 
             uint64_t *base_out = ws.carry + (size_t)flip * kRadix;
             DSM_CUDA(cudaMemsetAsync(ws.status, 0, sizeof(uint32_t) * (size_t)tiles * kRadix, stream));
             DSM_CUDA(cudaMemsetAsync(ws.counter, 0, sizeof(uint32_t), stream));
-#define SWEEP3(I, M, T, N, H)                                                                                    \
-    onesweep_kernel<I, M, T, N, H><<<tiles, T, sizeof(SweepSmemT<T / 32>), stream>>>(                            \
-        src_k + start, (I) ? nullptr : src_v + start, dst_k, dst_v, (uint32_t)cnt, start, shift, mask, base_in, \
-        base_out, ws.status, ws.counter, tiles - 1)
-#define SWEEP2(I, M, T, N)                                                                                       \
-    do {                                                                                                         \
-        if (hints) SWEEP3(I, M, T, N, true); else SWEEP3(I, M, T, N, false);                                     \
-    } while (0)
-#define SWEEP(I, M)                                                                                              \
-    do {                                                                                                         \
-        if (wide_cta) SWEEP2(I, M, 512, kSweepTile / 512); else SWEEP2(I, M, kSweepNarrow, kSweepTile / kSweepNarrow);       \
-    } while (0)
-            // bulk copies need 16-byte aligned sources: portions start at multiples of 2^29 pairs
-            const bool use_tma = tma && !hw_match && !wide_cta && !hints && (reinterpret_cast<uintptr_t>(src_k + start) & 15) == 0 &&
-                                 (iota || (reinterpret_cast<uintptr_t>(src_v + start) & 15) == 0);
-            if (use_tma) {
-                if (iota)
-                    onesweep_kernel<true, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true><<<tiles, kSweepTmaThreads, sizeof(SweepSmemT<kSweepTmaThreads / 32>), stream>>>(
-                        src_k + start, nullptr, dst_k, dst_v, (uint32_t)cnt, start, shift, mask, base_in, base_out, ws.status,
-                        ws.counter, tiles - 1);
-                else
-                    onesweep_kernel<false, false, kSweepTmaThreads, kSweepTile / kSweepTmaThreads, false, true><<<tiles, kSweepTmaThreads, sizeof(SweepSmemT<kSweepTmaThreads / 32>), stream>>>(
-                        src_k + start, src_v + start, dst_k, dst_v, (uint32_t)cnt, start, shift, mask, base_in, base_out, ws.status,
-                        ws.counter, tiles - 1);
-            } else if (iota) {
-                if (hw_match) SWEEP(true, true); else SWEEP(true, false);
-            } else {
-                if (hw_match) SWEEP(false, true); else SWEEP(false, false);
-            }
-#undef SWEEP2
-#undef SWEEP3
-#undef SWEEP
+            // (the bulk copy of a tile's keys needs a 16-byte aligned source: portions start at multiples of 2^29 pairs)
+            (iota ? onesweep_kernel<true> : onesweep_kernel<false>)<<<tiles, kSweepThreads, sizeof(SweepSmem), stream>>>(
+                src_k + start, iota ? nullptr : src_v + start, dst_k, dst_v, (uint32_t)cnt, start, shift, mask, base_in,
+                base_out, ws.status, ws.counter, tiles - 1);
             DSM_LAUNCH_CHECK();
             if (launches) *launches += 1;
             base_in = base_out;

@@ -18,21 +18,14 @@ constexpr int kRadixBits = 8;
 constexpr int kRadix = 1 << kRadixBits;
 constexpr int kMaxPasses = 8;
 
-// Tile of the one-sweep kernel: 4096 pairs, as 256 threads x 16 pairs or 512 threads x 8 pairs.
-#ifndef DSMFM_SWEEP_TILE
-#define DSMFM_SWEEP_TILE 4096
-#endif
-constexpr int kSweepTile = DSMFM_SWEEP_TILE; // pairs per CTA (a multiple of 512)
-constexpr int kSweepCtasPerSm = kSweepTile <= 3072 ? 5 : 4;
-constexpr bool kSweepWideDefault = false;
-constexpr bool kSweepHintsDefault = false;
-constexpr bool kSweepTmaVals = false;
-constexpr bool kSweepTmaDefault = true; // measured: 3.08 -> 2.98 ms per launch with the keys, see DESIGN.md section 5
+// Tile of the one-sweep kernel: 4096 pairs, 256 threads x 16 pairs.
+constexpr int kSweepTile = 4096;
+constexpr int kSweepThreads = 256;
+constexpr int kSweepItems = kSweepTile / kSweepThreads;
+constexpr int kSweepCtasPerSm = 4;
 // A launch handles at most this many pairs so that tile prefixes fit the
 // 30-bit payload of a status word; longer inputs run as several portions.
-constexpr uint64_t kSweepPortion = (uint64_t)kSweepTile * (kSweepTile > 4096 ? 65536 : 131072); // 2^29 for tiles of 4096 / 8192
-constexpr int kSweepTmaThreads = kSweepTile > 4096 ? 512 : 256; // threads of the default (bulk-copy ingest) kernel: 16 pairs each
-constexpr int kSweepNarrow = kSweepTile > 4096 ? 512 : 256;     // the narrower of the two switchable shapes
+constexpr uint64_t kSweepPortion = (uint64_t)kSweepTile * 131072; // 2^29
 
 struct RadixWorkspace {
     uint64_t *hist = nullptr;     // [kMaxPasses][256] digit counts, then exclusive bases
@@ -61,6 +54,7 @@ struct KeysFromArray {
 // (optional) are recorded around the one-sweep passes (histogram excluded).
 // hist_ready: ws.hist[pass][256] already holds the digit counts of the keys (whoever produced the keys
 // counted them on the way), so the histogram pass over the key array is skipped.
+// keys_a and keys_b must be 16-byte aligned: every whole tile's keys arrive by one bulk copy.
 int radix_sort_pairs(cudaStream_t stream, RadixWorkspace &ws, uint64_t *keys_a, uint32_t *vals_a, uint64_t *keys_b,
                      uint32_t *vals_b, uint64_t n, int begin_bit, int end_bit, bool iota_first,
                      uint32_t *launches, cudaEvent_t ev_begin = nullptr, cudaEvent_t ev_end = nullptr,

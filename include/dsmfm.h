@@ -142,7 +142,7 @@ typedef struct dsmfm_stats {
     uint32_t streamed;           /* 1: the text streamed in from the host in pieces and was packed and keyed   */
                                  /* piece by piece behind the copy (dsmfm_append_batch of a whole collection)  */
     uint64_t refine_key_fetches; /* 8-byte keys the refinement kernel gathered from the text */
-    uint64_t refine_launches;    /* refine_kernel launches                                  */
+    uint64_t refine_launches;    /* refinement launches                                     */
     uint64_t refine_members;     /* suffixes in the tie groups that had to be sorted: all of them when the */
                                  /* suffix array is kept, else those of groups with mixed BWT symbols       */
 } dsmfm_stats;

@@ -1,19 +1,14 @@
 """GPU suite: the initial suffix sort of an unsharded build, stage by stage (dsmfm.initial_sort stops after the group
 heads): the first keys and their digit counts, the one-sweep passes across tiles and portions, the group heads, the
 difference bits, `remaining` and the carried BWT, each against a numpy reference restated from the raw bytes
-(DESIGN.md section 3, items 2-4).  Also: keying in word ranges (a batch streaming in from the host), the
-environment switches that pick other kernel instantiations (initial_sort_variant_check.py, one process per setting),
-and streamed batches whose speculative pack is kept."""
+(DESIGN.md section 3, items 2-4).  Also: keying in word ranges (a batch streaming in from the host), and streamed
+batches whose speculative pack is kept."""
 import ctypes as C
 import hashlib
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
-
-HERE = os.path.dirname(os.path.abspath(__file__))
 
 CHUNK = 1 << 24
 PIECE = 21 * 3145728  # bytes per piece of a batch that streams in from the host (append_pipelined)
@@ -320,19 +315,6 @@ def test_initial_sort_across_portions():
     docs = dsmgen.docs(**kw)
     assert docs.size > PORTION
     run(docs)
-
-
-# ---- environment switches: other kernel instantiations, one process per setting ---------------------------------
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("setting", ["DSMFM_SWEEP_MATCH=1", "DSMFM_SWEEP_HINTS=1", "DSMFM_SWEEP_TMA=0",
-                                     "DSMFM_SWEEP_THREADS=512", "DSMFM_HEADS_U=4"])
-def test_initial_sort_under_switch(setting):
-    name, value = setting.split("=")
-    env = dict(os.environ, **{name: value})
-    r = subprocess.run([sys.executable, os.path.join(HERE, "initial_sort_variant_check.py")], env=env,
-                       capture_output=True, text=True)
-    assert r.returncode == 0 and "INITIAL_SORT_VARIANT_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
 
 
 # ---- batches that stream in from pinned host memory and keep their speculative pack ----------------------------
