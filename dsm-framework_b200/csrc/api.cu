@@ -858,6 +858,22 @@ struct dsmfm_builder {
     void append_fasta(const uint8_t *text, size_t m, dsmfm_fasta_info *info);
     void gather_raw();
     void block_stats(uint32_t *L);
+    // buffers of the refinement of one key range, sized by build() for the largest range (m_max suffixes)
+    struct RefineBufs {
+        uint64_t m_max = 0;
+        uint64_t *keys_a = nullptr, *keys_b = nullptr; // 8 m_max bytes each: the key buffers of the initial sort
+        uint32_t *other_vals = nullptr;                // 4 m_max + 16 bytes: the value buffer the sort left free
+        RadixWorkspace *ws = nullptr;
+        uint32_t *head[2] = {nullptr, nullptr};        // head_words_for(m_max) words each; head[0] from the sort
+        uint32_t *diff = nullptr;
+        unsigned long long *remaining = nullptr;       // 128 counters (see build())
+        uint32_t big_cap = 0, *big_heads = nullptr, *big_len = nullptr, *big_count = nullptr;
+        uint32_t *win_flag = nullptr, *win_list[2] = {nullptr, nullptr}, *win_count = nullptr;
+    };
+    uint64_t read_remaining(unsigned long long *d_remaining);
+    uint32_t refine_range(const RefineBufs &rb, int bits, const uint64_t *d_packed, const uint8_t *d_inv,
+                          uint64_t maxgap, int lo_bits, bool full_order, uint32_t *sa, uint64_t m, uint8_t *bwt,
+                          uint8_t *hi, uint32_t depth, bool use_diff, uint64_t remaining, uint32_t *paths);
     void build();
     void fetch();
     void make_sa_image();
@@ -1197,6 +1213,231 @@ void dsmfm_builder::block_stats(uint32_t *L)
 }
 
 // ---------------------------------------------------------------------------
+// the refinement of one key range (build(), dsmfm_dbg_refine)
+// ---------------------------------------------------------------------------
+// suffixes left in groups of >= 2 (counters [0,64) of d_remaining); the keys gathered from the text ([64,128)) go
+// to the statistics
+uint64_t dsmfm_builder::read_remaining(unsigned long long *d_remaining)
+{
+    unsigned long long h[128];
+    DSM_CUDA(cudaMemcpyAsync(h, d_remaining, sizeof h, cudaMemcpyDeviceToHost, stream));
+    DSM_CUDA(cudaStreamSynchronize(stream));
+    uint64_t t = 0;
+    for (int i = 0; i < 64; ++i) t += h[i];
+    for (int i = 64; i < 128; ++i) stats.refine_key_fetches += h[i];
+    return t;
+}
+
+// State in: sa[m] in the order of the first `depth` symbols, rb.head[0] (head_words_for(m) words, every bit from m
+// on set), the BWT bytes in bwt[m] (nullptr: no carried BWT) and hi[m] (wide positions, else nullptr), rb.diff when
+// use_diff, `remaining` suffixes in groups of >= 2.  Sorts sa (and bwt / hi with it) as far as full_order asks and
+// returns the rounds it ran; paths (optional) gets the DSMFM_RPATH_* bits of the choices made on the way.
+uint32_t dsmfm_builder::refine_range(const RefineBufs &rb, int bits, const uint64_t *d_packed, const uint8_t *d_inv,
+                                     uint64_t maxgap, int lo_bits, bool full_order, uint32_t *sa, uint64_t m,
+                                     uint8_t *bwt, uint8_t *hi, uint32_t depth, bool use_diff, uint64_t remaining,
+                                     uint32_t *paths)
+{
+    static_assert(kRwLaunchedCoop == DSMFM_RPATH_COOP && kRwLaunchedWide == DSMFM_RPATH_WIDE &&
+                  kRwLaunchedOrder == DSMFM_RPATH_ORDER && kRwLaunchedBitsShift == DSMFM_RPATH_BITS_SHIFT,
+                  "launch_refine reports DSMFM_RPATH_* bits");
+    cudaStream_t st = stream;
+    uint32_t *L = &stats.kernel_launches;
+    const bool wide = hi != nullptr;
+    const int spw = 64 / bits;
+    const int full_key_bits = spw * bits; // sorted bits of a refinement key (large-group path)
+    const uint64_t m_max = rb.m_max, hw = head_words_for(m);
+    uint64_t *d_keys_a = rb.keys_a, *d_keys_b = rb.keys_b;
+    RadixWorkspace &ws = *rb.ws;
+    uint32_t path = 0;
+
+    // What the refinement works on: the suffix array itself or, in BWT-only builds, dense copies of the groups
+    // whose members carry different BWT symbols (kernels.cu, "compaction of the groups that have to be sorted").
+    uint32_t *r_sa = sa;
+    uint32_t *r_head[2] = {rb.head[0], rb.head[1]};
+    uint8_t *r_bwt = bwt;
+    uint8_t *r_hi = hi;
+    uint64_t r_m = m, r_hw = hw;
+    const uint32_t *r_diff = use_diff ? rb.diff : nullptr;
+    uint32_t *c_sa = nullptr, *c_orig = nullptr, *c_head[2] = {nullptr, nullptr};
+    uint8_t *c_bw = nullptr, *c_hi = nullptr;
+    uint64_t m_act = 0;
+    const char *compact_env = std::getenv("DSMFM_REFINE_COMPACT"); // 0: refine in place (tests)
+    const bool compact_off = compact_env && std::atoi(compact_env) == 0;
+    const bool compact = use_diff && !compact_off && remaining > 0;
+    bool c_owned = false; // the dense arrays are allocations of their own (else: carved out of a key buffer)
+    if (compact) {
+        // scratch of the compaction: the key buffers of the initial sort are free from here on (the large-group
+        // path, their only other user, starts later and never needs more than 8 bytes per dense entry)
+        const uint64_t ntile = active_tiles(div_up(m, 32));
+        uint32_t *d_act = reinterpret_cast<uint32_t *>(d_keys_a);
+        uint64_t *d_tile = reinterpret_cast<uint64_t *>(d_keys_a) + (hw + 1) / 2;
+        const bool scratch_fits = (hw + 1) / 2 + ntile + 1 <= m_max;
+        if (!scratch_fits) {
+            d_act = static_cast<uint32_t *>(dmalloc(hw * 4));
+            d_tile = static_cast<uint64_t *>(dmalloc((ntile + 1) * 8));
+            path |= DSMFM_RPATH_SCRATCH_ALLOC;
+        }
+        DSM_CUDA(cudaMemsetAsync(d_act, 0, hw * 4, st));
+        launch_mark_active(st, rb.head[0], rb.diff, m, d_act, d_tile, L);
+        DSM_CUDA(cudaMemcpyAsync(&m_act, d_tile + ntile, 8, cudaMemcpyDeviceToHost, st));
+        DSM_CUDA(cudaStreamSynchronize(st));
+        stats.refine_members += m_act;
+        if (m_act == 0) {
+            remaining = 0; // every tie group carries a single BWT symbol
+        } else if (m_act * 2 > remaining) {
+            m_act = 0; // most members have to be sorted anyway (high repetition): refine in place
+        } else {
+            r_m = m_act;
+            r_hw = head_words_for(m_act);
+            auto up16 = [](uint64_t x) { return (x + 15) & ~(uint64_t)15; };
+            const uint64_t b_sa = up16(m_act * 4 + 16), b_bw = up16(m_act + 16), b_hi = wide ? up16(m_act + 16) : 0,
+                           b_head = up16(r_hw * 4);
+            const uint64_t need = 2 * b_sa + b_bw + b_hi + 2 * b_head;
+            // the upper part of the second key buffer, above what the large-group path can touch
+            uint8_t *base = reinterpret_cast<uint8_t *>(d_keys_b) + up16(m_act * 8);
+            c_owned = up16(m_act * 8) + need > m_max * 8;
+            if (c_owned) {
+                base = static_cast<uint8_t *>(dmalloc(need));
+                path |= DSMFM_RPATH_DENSE_ALLOC;
+            }
+            c_sa = reinterpret_cast<uint32_t *>(base);
+            c_orig = reinterpret_cast<uint32_t *>(base + b_sa);
+            c_bw = base + 2 * b_sa;
+            c_hi = wide ? base + 2 * b_sa + b_bw : nullptr;
+            c_head[0] = reinterpret_cast<uint32_t *>(base + 2 * b_sa + b_bw + b_hi);
+            c_head[1] = reinterpret_cast<uint32_t *>(base + 2 * b_sa + b_bw + b_hi + b_head);
+            DSM_CUDA(cudaMemsetAsync(c_head[0], 0, r_hw * 4, st));
+            launch_compact_active(st, d_act, rb.head[0], m, d_tile, sa, bwt, hi, m_act, c_sa, c_bw, c_hi, c_orig,
+                                  c_head[0], r_hw, L);
+            r_sa = c_sa;
+            r_head[0] = c_head[0];
+            r_head[1] = c_head[1];
+            r_bwt = c_bw;
+            r_hi = c_hi;
+            r_diff = nullptr;
+            path |= DSMFM_RPATH_COMPACT;
+        }
+        if (!scratch_fits) {
+            dfree(d_act);
+            dfree(d_tile);
+        }
+    } else if (remaining > 0) {
+        stats.refine_members += remaining;
+    }
+
+    // ---- refinement rounds ------------------------------------------------------------
+    // Suffixes that still agree on their first `depth` symbols are re-sorted by the next
+    // SPW symbols taken straight from the packed text.  (The reference re-keys with the
+    // ranks of the suffixes h positions ahead, utils.cpp:236-262; documents here are short,
+    // the text fits in HBM next to the suffix array, and extending the key from the text
+    // needs neither an inverse suffix array nor rank scatter traffic.)
+    int cur = 0;
+    uint32_t round = 0;
+    uint32_t depth_next = depth; // symbols every unresolved group is known to agree on
+    const uint32_t max_rounds = (uint32_t)(maxgap / spw + 4);
+    // windows that still own unresolved groups: all of them in the first round, a compact list afterwards
+    const uint32_t nwin = (uint32_t)div_up(r_m, kRefWindow);
+    const uint32_t *win_list = nullptr;
+    uint32_t n_list = nwin;
+    int wl = 0;
+    while (remaining > 0) {
+        if (round >= max_rounds)
+            throw CudaError{cudaErrorUnknown, "refinement did not converge (internal error)", __FILE__, __LINE__};
+        if (round < 32) stats.active[round] += remaining;
+        ++round;
+        const uint32_t depth = depth_next;
+        DSM_CUDA(cudaMemcpyAsync(r_head[cur ^ 1], r_head[cur], r_hw * 4, cudaMemcpyDeviceToDevice, st));
+        DSM_CUDA(cudaMemsetAsync(rb.remaining, 0, 128 * 8, st));
+        DSM_CUDA(cudaMemsetAsync(rb.big_count, 0, 4, st));
+        DSM_CUDA(cudaMemsetAsync(rb.win_flag, 0, (size_t)nwin * 4, st));
+        DSM_CUDA(cudaMemsetAsync(rb.win_count, 0, 4, st));
+        ++stats.refine_launches;
+        path |= launch_refine(st, bits, d_packed, r_sa, r_head[cur], r_head[cur ^ 1], r_m, depth, win_list, n_list,
+                              rb.big_heads, rb.big_cap, rb.big_count, rb.remaining, rb.win_flag, rb.win_list[wl],
+                              rb.win_count, r_bwt, r_hi, lo_bits, full_order, round == 1 ? r_diff : nullptr, L,
+                              /*big_groups=*/!full_order && !(compact && m_act));
+        uint32_t nbig = 0;
+        DSM_CUDA(cudaMemcpyAsync(&nbig, rb.big_count, 4, cudaMemcpyDeviceToHost, st));
+        remaining = read_remaining(rb.remaining);
+        if (nbig > 0) {
+            // groups too large for one CTA: one global (group, key) radix sort over all of them
+            if (nbig > rb.big_cap) throw CudaError{cudaErrorUnknown, "large-group list overflow", __FILE__, __LINE__};
+            launch_big_extent(st, r_head[cur], r_m, rb.big_heads, nbig, rb.big_len, L);
+            std::vector<uint32_t> heads(nbig), lens(nbig);
+            DSM_CUDA(cudaMemcpyAsync(heads.data(), rb.big_heads, (size_t)nbig * 4, cudaMemcpyDeviceToHost, st));
+            DSM_CUDA(cudaMemcpyAsync(lens.data(), rb.big_len, (size_t)nbig * 4, cudaMemcpyDeviceToHost, st));
+            DSM_CUDA(cudaStreamSynchronize(st));
+            std::vector<uint32_t> order(nbig);
+            for (uint32_t i = 0; i < nbig; ++i) order[i] = i;
+            std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return heads[a] < heads[b]; });
+            std::vector<uint32_t> sheads(nbig);
+            std::vector<uint64_t> offs(nbig + 1);
+            uint64_t total = 0;
+            for (uint32_t i = 0; i < nbig; ++i) {
+                sheads[i] = heads[order[i]];
+                offs[i] = total;
+                total += lens[order[i]];
+            }
+            offs[nbig] = total;
+            stats.fallback_elems += total;
+            uint64_t *d_off = static_cast<uint64_t *>(dmalloc((size_t)(nbig + 1) * 8));
+            uint32_t *d_bsa = static_cast<uint32_t *>(dmalloc(total * 4));
+            uint32_t *d_bgid = static_cast<uint32_t *>(dmalloc(total * 4));
+            uint64_t *d_bkey = static_cast<uint64_t *>(dmalloc(total * 8));
+            uint32_t *d_perm = static_cast<uint32_t *>(dmalloc(total * 4 + 16));
+            uint8_t *d_bhi = wide ? static_cast<uint8_t *>(dmalloc(total + 16)) : nullptr;
+            DSM_CUDA(cudaMemcpyAsync(rb.big_heads, sheads.data(), (size_t)nbig * 4, cudaMemcpyHostToDevice, st));
+            DSM_CUDA(cudaMemcpyAsync(d_off, offs.data(), (size_t)(nbig + 1) * 8, cudaMemcpyHostToDevice, st));
+            launch_big_gather(st, bits, d_packed, r_sa, depth, rb.big_heads, d_off, nbig, total, d_bsa,
+                              d_bkey, d_bgid, r_hi, d_bhi, lo_bits, L);
+            // the key buffers of the initial sort are free by now
+            DSM_CUDA(cudaMemcpyAsync(d_keys_a, d_bkey, total * 8, cudaMemcpyDeviceToDevice, st));
+            int p1 = radix_sort_pairs(st, ws, d_keys_a, rb.other_vals, d_keys_b, d_perm, total, 0, full_key_bits, true, L);
+            // pass 0 writes (keys_b, perm); an odd pass count leaves the result there
+            uint64_t *kfree = (p1 & 1) ? d_keys_a : d_keys_b;
+            uint32_t *pres = (p1 & 1) ? d_perm : rb.other_vals;
+            uint32_t *pfree = (p1 & 1) ? rb.other_vals : d_perm;
+            if (nbig > 1) {
+                int gbits = 1;
+                while ((1ull << gbits) < nbig) ++gbits;
+                launch_gather_u32_to_u64(st, d_bgid, pres, total, kfree, L);
+                uint64_t *k2a = kfree, *k2b = (kfree == d_keys_a) ? d_keys_b : d_keys_a;
+                int p2 = radix_sort_pairs(st, ws, k2a, pres, k2b, pfree, total, 0, gbits, false, L);
+                if (p2 & 1) std::swap(pres, pfree);
+                path |= DSMFM_RPATH_BIG_MULTI;
+            }
+            launch_big_scatter(st, bits, pres, d_bsa, d_bkey, d_bgid, rb.big_heads, d_off, total, r_sa,
+                               r_head[cur ^ 1], rb.win_flag, rb.win_list[wl], rb.win_count, d_packed, d_inv,
+                               r_bwt, d_bhi, r_hi, lo_bits, L);
+            DSM_CUDA(cudaStreamSynchronize(st)); // sheads / offs are host vectors
+            dfree(d_off);
+            dfree(d_bsa);
+            dfree(d_bgid);
+            dfree(d_bkey);
+            dfree(d_perm);
+            dfree(d_bhi);
+            remaining += total; // re-examined (and counted exactly) by the next round
+        }
+        // a launch resolves every group that fits a CTA: what is left went through the large-group path,
+        // which sorted it by the SPW symbols from `depth` on
+        depth_next = depth + (uint32_t)spw;
+        DSM_CUDA(cudaMemcpyAsync(&n_list, rb.win_count, 4, cudaMemcpyDeviceToHost, st));
+        DSM_CUDA(cudaStreamSynchronize(st));
+        win_list = rb.win_list[wl];
+        wl ^= 1;
+        cur ^= 1;
+        if (remaining > 0 && n_list == 0)
+            throw CudaError{cudaErrorUnknown, "unresolved groups without an owning window (internal error)", __FILE__, __LINE__};
+    }
+    if (compact && m_act) { // the BWT bytes of the sorted groups go back to their slots
+        launch_scatter_bwt(st, c_orig, c_bw, m_act, bwt, L);
+        if (c_owned) dfree(c_sa);
+    }
+    if (paths) *paths = path;
+    return round;
+}
+
+// ---------------------------------------------------------------------------
 // the device build
 // ---------------------------------------------------------------------------
 void dsmfm_builder::build()
@@ -1453,7 +1694,6 @@ void dsmfm_builder::build()
         sel_geom.bytes[0] = n;
     }
     uint32_t *d_sel_lut = sharded ? static_cast<uint32_t *>(dmalloc(sizeof(uint32_t) * kSelLutWords)) : nullptr;
-    const int full_key_bits = spw * bits; // sorted bits of a refinement key (large-group path)
     const uint64_t hwords = head_words_for(m_max);
     uint32_t *d_head[2];
     d_head[0] = static_cast<uint32_t *>(dmalloc(hwords * 4));
@@ -1471,6 +1711,23 @@ void dsmfm_builder::build()
     d_win_list[0] = static_cast<uint32_t *>(dmalloc((size_t)nwin_max * 4));
     d_win_list[1] = static_cast<uint32_t *>(dmalloc((size_t)nwin_max * 4));
     uint32_t *d_win_count = static_cast<uint32_t *>(dmalloc(4));
+    RefineBufs rb;
+    rb.m_max = m_max;
+    rb.keys_a = d_keys_a;
+    rb.keys_b = d_keys_b;
+    rb.ws = &ws;
+    rb.head[0] = d_head[0];
+    rb.head[1] = d_head[1];
+    rb.diff = d_diff;
+    rb.remaining = d_remaining;
+    rb.big_cap = big_cap;
+    rb.big_heads = d_big_heads;
+    rb.big_len = d_big_len;
+    rb.big_count = d_big_count;
+    rb.win_flag = d_win_flag;
+    rb.win_list[0] = d_win_list[0];
+    rb.win_list[1] = d_win_list[1];
+    rb.win_count = d_win_count;
     // results of the whole slice: the BWT (its own buffer: the key buffers are still needed by the
     // large-group path), optionally the suffix array
     d_bwt = static_cast<uint8_t *>(dmalloc(m_total + 64));
@@ -1527,6 +1784,7 @@ void dsmfm_builder::build()
         uint32_t *d_other_vals = (passes & 1) ? d_vals_a : d_vals_b;
         d_last_sorted_vals = d_sorted_vals;
         d_last_other_vals = d_other_vals;
+        rb.other_vals = d_other_vals;
         stats.sort_passes = passes;
         pass_launches += (uint32_t)passes * (uint32_t)div_up(m, kSweepPortion); // a pass is one launch per portion
         pass_launch_bytes += (uint64_t)passes * m * 24ull;
@@ -1538,195 +1796,11 @@ void dsmfm_builder::build()
                      carry_bwt ? bwt_out : nullptr, hi_out, hi_shift, use_diff ? d_diff : nullptr, L);
         DSM_CUDA(cudaEventRecord(evr[1], st));
 
-        auto read_remaining = [&]() -> uint64_t {
-            unsigned long long h[128];
-            DSM_CUDA(cudaMemcpyAsync(h, d_remaining, sizeof h, cudaMemcpyDeviceToHost, st));
-            DSM_CUDA(cudaStreamSynchronize(st));
-            uint64_t t = 0;
-            for (int i = 0; i < 64; ++i) t += h[i];
-            for (int i = 64; i < 128; ++i) stats.refine_key_fetches += h[i];
-            return t;
-        };
-        uint64_t remaining = read_remaining();
+        uint64_t remaining = read_remaining(d_remaining);
         trace("build: initial sort done");
-
-        // What the refinement works on: the suffix array itself or, in BWT-only builds, dense copies of the groups
-        // whose members carry different BWT symbols (kernels.cu, "compaction of the groups that have to be sorted").
-        uint32_t *r_sa = d_sorted_vals;
-        uint32_t *r_head[2] = {d_head[0], d_head[1]};
-        uint8_t *r_bwt = carry_bwt ? bwt_out : nullptr;
-        uint8_t *r_hi = hi_out;
-        uint64_t r_m = m, r_hw = hw;
-        const uint32_t *r_diff = use_diff ? d_diff : nullptr;
-        uint32_t *c_sa = nullptr, *c_orig = nullptr, *c_head[2] = {nullptr, nullptr};
-        uint8_t *c_bw = nullptr, *c_hi = nullptr;
-        uint64_t m_act = 0;
-        const char *compact_env = std::getenv("DSMFM_REFINE_COMPACT"); // 0: refine in place (tests)
-        const bool compact_off = compact_env && std::atoi(compact_env) == 0;
-        const bool compact = use_diff && !compact_off && remaining > 0;
-        bool c_owned = false; // the dense arrays are allocations of their own (else: carved out of a key buffer)
-        if (compact) {
-            // scratch of the compaction: the key buffers of the initial sort are free from here on (the large-group
-            // path, their only other user, starts later and never needs more than 8 bytes per dense entry)
-            const uint64_t ntile = active_tiles(div_up(m, 32));
-            uint32_t *d_act = reinterpret_cast<uint32_t *>(d_keys_a);
-            uint64_t *d_tile = reinterpret_cast<uint64_t *>(d_keys_a) + (hw + 1) / 2;
-            const bool scratch_fits = (hw + 1) / 2 + ntile + 1 <= m_max;
-            if (!scratch_fits) {
-                d_act = static_cast<uint32_t *>(dmalloc(hw * 4));
-                d_tile = static_cast<uint64_t *>(dmalloc((ntile + 1) * 8));
-            }
-            DSM_CUDA(cudaMemsetAsync(d_act, 0, hw * 4, st));
-            launch_mark_active(st, d_head[0], d_diff, m, d_act, d_tile, L);
-            DSM_CUDA(cudaMemcpyAsync(&m_act, d_tile + ntile, 8, cudaMemcpyDeviceToHost, st));
-            DSM_CUDA(cudaStreamSynchronize(st));
-            stats.refine_members += m_act;
-            if (m_act == 0) {
-                remaining = 0; // every tie group carries a single BWT symbol
-            } else if (m_act * 2 > remaining) {
-                m_act = 0; // most members have to be sorted anyway (high repetition): refine in place
-            } else {
-                r_m = m_act;
-                r_hw = head_words_for(m_act);
-                auto up16 = [](uint64_t x) { return (x + 15) & ~(uint64_t)15; };
-                const uint64_t b_sa = up16(m_act * 4 + 16), b_bw = up16(m_act + 16), b_hi = wide ? up16(m_act + 16) : 0,
-                               b_head = up16(r_hw * 4);
-                const uint64_t need = 2 * b_sa + b_bw + b_hi + 2 * b_head;
-                // the upper part of the second key buffer, above what the large-group path can touch
-                uint8_t *base = reinterpret_cast<uint8_t *>(d_keys_b) + up16(m_act * 8);
-                c_owned = up16(m_act * 8) + need > m_max * 8;
-                if (c_owned) base = static_cast<uint8_t *>(dmalloc(need));
-                c_sa = reinterpret_cast<uint32_t *>(base);
-                c_orig = reinterpret_cast<uint32_t *>(base + b_sa);
-                c_bw = base + 2 * b_sa;
-                c_hi = wide ? base + 2 * b_sa + b_bw : nullptr;
-                c_head[0] = reinterpret_cast<uint32_t *>(base + 2 * b_sa + b_bw + b_hi);
-                c_head[1] = reinterpret_cast<uint32_t *>(base + 2 * b_sa + b_bw + b_hi + b_head);
-                DSM_CUDA(cudaMemsetAsync(c_head[0], 0, r_hw * 4, st));
-                launch_compact_active(st, d_act, d_head[0], m, d_tile, d_sorted_vals, bwt_out, hi_out, m_act, c_sa, c_bw,
-                                      c_hi, c_orig, c_head[0], r_hw, L);
-                r_sa = c_sa;
-                r_head[0] = c_head[0];
-                r_head[1] = c_head[1];
-                r_bwt = c_bw;
-                r_hi = c_hi;
-                r_diff = nullptr;
-            }
-            if (!scratch_fits) {
-                dfree(d_act);
-                dfree(d_tile);
-            }
-        } else if (remaining > 0) {
-            stats.refine_members += remaining;
-        }
-
-        // ---- refinement rounds ------------------------------------------------------------
-        // Suffixes that still agree on their first `depth` symbols are re-sorted by the next
-        // SPW symbols taken straight from the packed text.  (The reference re-keys with the
-        // ranks of the suffixes h positions ahead, utils.cpp:236-262; documents here are short,
-        // the text fits in HBM next to the suffix array, and extending the key from the text
-        // needs neither an inverse suffix array nor rank scatter traffic.)
-        int cur = 0;
-        uint32_t round = 0;
-        uint32_t depth_next = (uint32_t)first_syms; // symbols every unresolved group is known to agree on
-        const uint32_t max_rounds = (uint32_t)(maxgap / spw + 4);
-        // windows that still own unresolved groups: all of them in the first round, a compact list afterwards
-        const uint32_t nwin = (uint32_t)div_up(r_m, kRefWindow);
-        const uint32_t *win_list = nullptr;
-        uint32_t n_list = nwin;
-        int wl = 0;
-        while (remaining > 0) {
-            if (round >= max_rounds)
-                throw CudaError{cudaErrorUnknown, "refinement did not converge (internal error)", __FILE__, __LINE__};
-            if (round < 32) stats.active[round] += remaining;
-            ++round;
-            const uint32_t depth = depth_next;
-            DSM_CUDA(cudaMemcpyAsync(r_head[cur ^ 1], r_head[cur], r_hw * 4, cudaMemcpyDeviceToDevice, st));
-            DSM_CUDA(cudaMemsetAsync(d_remaining, 0, 128 * 8, st));
-            DSM_CUDA(cudaMemsetAsync(d_big_count, 0, 4, st));
-            DSM_CUDA(cudaMemsetAsync(d_win_flag, 0, (size_t)nwin * 4, st));
-            DSM_CUDA(cudaMemsetAsync(d_win_count, 0, 4, st));
-            ++stats.refine_launches;
-            launch_refine(st, bits, d_packed, r_sa, r_head[cur], r_head[cur ^ 1], r_m, depth, win_list, n_list,
-                          d_big_heads, big_cap, d_big_count, d_remaining, d_win_flag, d_win_list[wl], d_win_count,
-                          r_bwt, r_hi, lo_bits, full_order, round == 1 ? r_diff : nullptr, L,
-                          /*big_groups=*/!full_order && !(compact && m_act));
-            uint32_t nbig = 0;
-            DSM_CUDA(cudaMemcpyAsync(&nbig, d_big_count, 4, cudaMemcpyDeviceToHost, st));
-            remaining = read_remaining();
-            if (nbig > 0) {
-                // groups too large for one CTA: one global (group, key) radix sort over all of them
-                if (nbig > big_cap) throw CudaError{cudaErrorUnknown, "large-group list overflow", __FILE__, __LINE__};
-                launch_big_extent(st, r_head[cur], r_m, d_big_heads, nbig, d_big_len, L);
-                std::vector<uint32_t> heads(nbig), lens(nbig);
-                DSM_CUDA(cudaMemcpyAsync(heads.data(), d_big_heads, (size_t)nbig * 4, cudaMemcpyDeviceToHost, st));
-                DSM_CUDA(cudaMemcpyAsync(lens.data(), d_big_len, (size_t)nbig * 4, cudaMemcpyDeviceToHost, st));
-                DSM_CUDA(cudaStreamSynchronize(st));
-                std::vector<uint32_t> order(nbig);
-                for (uint32_t i = 0; i < nbig; ++i) order[i] = i;
-                std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return heads[a] < heads[b]; });
-                std::vector<uint32_t> sheads(nbig);
-                std::vector<uint64_t> offs(nbig + 1);
-                uint64_t total = 0;
-                for (uint32_t i = 0; i < nbig; ++i) {
-                    sheads[i] = heads[order[i]];
-                    offs[i] = total;
-                    total += lens[order[i]];
-                }
-                offs[nbig] = total;
-                stats.fallback_elems += total;
-                uint64_t *d_off = static_cast<uint64_t *>(dmalloc((size_t)(nbig + 1) * 8));
-                uint32_t *d_bsa = static_cast<uint32_t *>(dmalloc(total * 4));
-                uint32_t *d_bgid = static_cast<uint32_t *>(dmalloc(total * 4));
-                uint64_t *d_bkey = static_cast<uint64_t *>(dmalloc(total * 8));
-                uint32_t *d_perm = static_cast<uint32_t *>(dmalloc(total * 4 + 16));
-                uint8_t *d_bhi = wide ? static_cast<uint8_t *>(dmalloc(total + 16)) : nullptr;
-                DSM_CUDA(cudaMemcpyAsync(d_big_heads, sheads.data(), (size_t)nbig * 4, cudaMemcpyHostToDevice, st));
-                DSM_CUDA(cudaMemcpyAsync(d_off, offs.data(), (size_t)(nbig + 1) * 8, cudaMemcpyHostToDevice, st));
-                launch_big_gather(st, bits, d_packed, r_sa, depth, d_big_heads, d_off, nbig, total, d_bsa,
-                                  d_bkey, d_bgid, r_hi, d_bhi, lo_bits, L);
-                // the key buffers of the initial sort are free by now
-                DSM_CUDA(cudaMemcpyAsync(d_keys_a, d_bkey, total * 8, cudaMemcpyDeviceToDevice, st));
-                int p1 = radix_sort_pairs(st, ws, d_keys_a, d_other_vals, d_keys_b, d_perm, total, 0, full_key_bits, true, L);
-                // pass 0 writes (keys_b, perm); an odd pass count leaves the result there
-                uint64_t *kfree = (p1 & 1) ? d_keys_a : d_keys_b;
-                uint32_t *pres = (p1 & 1) ? d_perm : d_other_vals;
-                uint32_t *pfree = (p1 & 1) ? d_other_vals : d_perm;
-                if (nbig > 1) {
-                    int gbits = 1;
-                    while ((1ull << gbits) < nbig) ++gbits;
-                    launch_gather_u32_to_u64(st, d_bgid, pres, total, kfree, L);
-                    uint64_t *k2a = kfree, *k2b = (kfree == d_keys_a) ? d_keys_b : d_keys_a;
-                    int p2 = radix_sort_pairs(st, ws, k2a, pres, k2b, pfree, total, 0, gbits, false, L);
-                    if (p2 & 1) std::swap(pres, pfree);
-                }
-                launch_big_scatter(st, bits, pres, d_bsa, d_bkey, d_bgid, d_big_heads, d_off, total, r_sa,
-                                   r_head[cur ^ 1], d_win_flag, d_win_list[wl], d_win_count, d_packed, d_inv,
-                                   r_bwt, d_bhi, r_hi, lo_bits, L);
-                DSM_CUDA(cudaStreamSynchronize(st)); // sheads / offs are host vectors
-                dfree(d_off);
-                dfree(d_bsa);
-                dfree(d_bgid);
-                dfree(d_bkey);
-                dfree(d_perm);
-                dfree(d_bhi);
-                remaining += total; // re-examined (and counted exactly) by the next round
-            }
-            // a launch resolves every group that fits a CTA: what is left went through the large-group path,
-            // which sorted it by the SPW symbols from `depth` on
-            depth_next = depth + (uint32_t)spw;
-            DSM_CUDA(cudaMemcpyAsync(&n_list, d_win_count, 4, cudaMemcpyDeviceToHost, st));
-            DSM_CUDA(cudaStreamSynchronize(st));
-            win_list = d_win_list[wl];
-            wl ^= 1;
-            cur ^= 1;
-            if (remaining > 0 && n_list == 0)
-                throw CudaError{cudaErrorUnknown, "unresolved groups without an owning window (internal error)", __FILE__, __LINE__};
-        }
-        if (compact && m_act) { // the BWT bytes of the sorted groups go back to their slots
-            launch_scatter_bwt(st, c_orig, c_bw, m_act, bwt_out, L);
-            if (c_owned) dfree(c_sa);
-        }
+        const uint32_t round = refine_range(rb, bits, d_packed, d_inv, maxgap, lo_bits, full_order, d_sorted_vals, m,
+                                            carry_bwt ? bwt_out : nullptr, hi_out, (uint32_t)first_syms, use_diff,
+                                            remaining, nullptr);
         rounds_max = std::max(rounds_max, round);
         // ---- BWT when it could not ride along (64-bit first keys, unsharded only) -----------
         if (!carry_bwt) launch_bwt(st, bits, d_packed, d_inv, d_sorted_vals, m, bwt_out, L);
@@ -3533,6 +3607,139 @@ DSMFM_API int dsmfm_dbg_initial_sort(int device, const uint8_t *docs, uint64_t n
     ws.release();
     cudaFree(d_raw); cudaFree(d_map); cudaFree(d_inv); cudaFree(d_packed); cudaFree(ka); cudaFree(kb);
     cudaFree(va); cudaFree(vb); cudaFree(d_head); cudaFree(d_diff); cudaFree(d_bwt); cudaFree(d_rem);
+    return rc;
+}
+
+DSMFM_API int dsmfm_dbg_refine(int device, const uint8_t *docs, uint64_t n, const uint64_t *sa_in,
+                               const uint32_t *head_in, uint64_t m, uint32_t depth, uint32_t flags, int lo_bits,
+                               uint64_t *sa_out, uint8_t *bwt_out, dsmfm_stats *stats_out, uint32_t *paths)
+{
+    // everything the caller hands in is checked before anything is launched: a state that passes is one the
+    // initial sort of a build could have left
+    if (!docs || !sa_in || !head_in || !sa_out || !bwt_out || !stats_out || !paths) return DSMFM_EINVAL;
+    if (n == 0 || n >= (1ull << 32) - kRefCap - 64 || docs[n - 1] != 0 || docs[0] == 0) return DSMFM_EINVAL;
+    if (m == 0 || m > n || (flags & ~DSMFM_FLAG_KEEP_SA) || (lo_bits != 0 && (lo_bits < 4 || lo_bits > 32)))
+        return DSMFM_EINVAL;
+    uint64_t counts[256] = {}, maxgap = 0, doc_begin = 0;
+    for (uint64_t i = 0; i < n; ++i) {
+        ++counts[docs[i]];
+        if (i && docs[i] == 0 && docs[i - 1] == 0) return DSMFM_EINVAL; // an empty document
+        if (docs[i] == 0) {
+            maxgap = std::max(maxgap, i + 1 - doc_begin);
+            doc_begin = i + 1;
+        }
+    }
+    const uint64_t pos_end = lo_bits && lo_bits + 8 < 64 ? std::min<uint64_t>(n, 1ull << (lo_bits + 8)) : n;
+    std::vector<bool> seen(n);
+    for (uint64_t i = 0; i < m; ++i) {
+        if (sa_in[i] >= pos_end || seen[sa_in[i]]) return DSMFM_EINVAL;
+        seen[sa_in[i]] = true;
+    }
+    const uint64_t hw = head_words_for(m);
+    std::vector<uint32_t> head(hw, ~0u), diff(hw, 0u);
+    std::memcpy(head.data(), head_in, div_up(m, 32) * 4);
+    if (m % 32) head[m / 32] |= ~0u << (m % 32); // ranks behind the last suffix count as heads
+    if (!(head[0] & 1u)) return DSMFM_EINVAL;
+    auto is_head = [&](uint64_t i) { return (head[i >> 5] >> (i & 31)) & 1u; };
+    std::vector<uint8_t> bwt(m);
+    uint64_t remaining = 0;
+    for (uint64_t g = 0; g < m;) {
+        uint64_t e = g + 1;
+        while (e < m && !is_head(e)) ++e;
+        if (e - g >= 2) {
+            remaining += e - g;
+            const uint64_t p0 = sa_in[g];
+            for (uint64_t i = g + 1; i < e; ++i) {
+                if (sa_in[i] <= sa_in[i - 1]) return DSMFM_EINVAL; // a stable sort leaves tied suffixes in text order
+                for (uint32_t j = 0; j < depth; ++j)
+                    if (docs[p0 + j] == 0 || docs[sa_in[i] + j] != docs[p0 + j]) return DSMFM_EINVAL;
+            }
+        }
+        for (uint64_t i = g; i < e; ++i) {
+            bwt[i] = sa_in[i] ? docs[sa_in[i] - 1] : 0;
+            if (i > g && bwt[i] != bwt[i - 1]) diff[i >> 5] |= 1u << (i & 31);
+        }
+        g = e;
+    }
+
+    uint8_t code_map[256], inv_map[256] = {};
+    const int bits = alphabet_of(counts, code_map, nullptr);
+    for (int c = 1; c < 256; ++c)
+        if (code_map[c]) inv_map[code_map[c]] = (uint8_t)c;
+    const uint64_t nwords = div_up(n, 64 / bits) + 8; // zero words behind the text: refinement rows read ahead
+    const bool wide = lo_bits > 0;
+    const int klo = wide ? lo_bits : 32;
+    const bool keep_sa = (flags & DSMFM_FLAG_KEEP_SA) != 0;
+    std::vector<uint32_t> lo(m);
+    std::vector<uint8_t> hi(wide ? m : 0);
+    for (uint64_t i = 0; i < m; ++i) {
+        lo[i] = (uint32_t)(klo == 32 ? sa_in[i] : sa_in[i] & ((1ull << klo) - 1));
+        if (wide) hi[i] = (uint8_t)(sa_in[i] >> klo);
+    }
+
+    // the buffers build() allocates for a key range of m suffixes, through a builder of its own (DSMFM_GUARD)
+    dsmfm_options opts;
+    std::memset(&opts, 0, sizeof opts);
+    opts.device = device < 0 ? 0 : device;
+    dsmfm_builder *b = nullptr;
+    int rc = dsmfm_create(&opts, &b);
+    if (rc != DSMFM_OK) return rc;
+    try {
+        cudaStream_t st = b->stream;
+        uint8_t *d_raw = static_cast<uint8_t *>(b->dmalloc(n + 64));
+        uint8_t *d_map = static_cast<uint8_t *>(b->dmalloc(256));
+        uint8_t *d_inv = static_cast<uint8_t *>(b->dmalloc(256));
+        uint64_t *d_packed = static_cast<uint64_t *>(b->dmalloc(nwords * 8));
+        DSM_CUDA(cudaMemcpyAsync(d_raw, docs, n, cudaMemcpyHostToDevice, st));
+        DSM_CUDA(cudaMemcpyAsync(d_map, code_map, 256, cudaMemcpyHostToDevice, st));
+        DSM_CUDA(cudaMemcpyAsync(d_inv, inv_map, 256, cudaMemcpyHostToDevice, st));
+        launch_pack(st, bits, d_raw, n, d_map, d_packed, nwords, nullptr);
+        RadixWorkspace ws;
+        ws.status_tiles = div_up(m < kSweepPortion ? m : kSweepPortion, kSweepTile);
+        ws.hist = static_cast<uint64_t *>(b->dmalloc(sizeof(uint64_t) * kMaxPasses * kRadix));
+        ws.carry = static_cast<uint64_t *>(b->dmalloc(sizeof(uint64_t) * 2 * kRadix));
+        ws.status = static_cast<uint32_t *>(b->dmalloc(sizeof(uint32_t) * ws.status_tiles * kRadix));
+        ws.counter = static_cast<uint32_t *>(b->dmalloc(sizeof(uint32_t)));
+        dsmfm_builder::RefineBufs rb;
+        rb.m_max = m;
+        rb.keys_a = static_cast<uint64_t *>(b->dmalloc(m * 8));
+        rb.keys_b = static_cast<uint64_t *>(b->dmalloc(m * 8));
+        uint32_t *d_sa = static_cast<uint32_t *>(b->dmalloc(m * 4 + 16));
+        rb.other_vals = static_cast<uint32_t *>(b->dmalloc(m * 4 + 16));
+        rb.ws = &ws;
+        rb.head[0] = static_cast<uint32_t *>(b->dmalloc(hw * 4));
+        rb.head[1] = static_cast<uint32_t *>(b->dmalloc(hw * 4));
+        rb.diff = static_cast<uint32_t *>(b->dmalloc(hw * 4));
+        rb.remaining = static_cast<unsigned long long *>(b->dmalloc(128 * 8));
+        rb.big_cap = (uint32_t)(m / kRefGroupMaxWarps + 2);
+        rb.big_heads = static_cast<uint32_t *>(b->dmalloc((size_t)rb.big_cap * 4));
+        rb.big_len = static_cast<uint32_t *>(b->dmalloc((size_t)rb.big_cap * 4));
+        rb.big_count = static_cast<uint32_t *>(b->dmalloc(4));
+        const uint64_t nwin = div_up(m, kRefWindow);
+        rb.win_flag = static_cast<uint32_t *>(b->dmalloc(nwin * 4));
+        rb.win_list[0] = static_cast<uint32_t *>(b->dmalloc(nwin * 4));
+        rb.win_list[1] = static_cast<uint32_t *>(b->dmalloc(nwin * 4));
+        rb.win_count = static_cast<uint32_t *>(b->dmalloc(4));
+        uint8_t *d_bwt = static_cast<uint8_t *>(b->dmalloc(m + 64));
+        uint8_t *d_hi = wide ? static_cast<uint8_t *>(b->dmalloc(m + 16)) : nullptr;
+        DSM_CUDA(cudaMemcpyAsync(d_sa, lo.data(), m * 4, cudaMemcpyHostToDevice, st));
+        DSM_CUDA(cudaMemcpyAsync(rb.head[0], head.data(), hw * 4, cudaMemcpyHostToDevice, st));
+        DSM_CUDA(cudaMemcpyAsync(rb.diff, diff.data(), hw * 4, cudaMemcpyHostToDevice, st));
+        DSM_CUDA(cudaMemcpyAsync(d_bwt, bwt.data(), m, cudaMemcpyHostToDevice, st));
+        if (wide) DSM_CUDA(cudaMemcpyAsync(d_hi, hi.data(), m, cudaMemcpyHostToDevice, st));
+        b->stats.rounds = b->refine_range(rb, bits, d_packed, d_inv, maxgap, klo, keep_sa, d_sa, m, d_bwt, d_hi, depth,
+                                          !keep_sa, remaining, paths);
+        DSM_CUDA(cudaMemcpyAsync(lo.data(), d_sa, m * 4, cudaMemcpyDeviceToHost, st));
+        DSM_CUDA(cudaMemcpyAsync(bwt_out, d_bwt, m, cudaMemcpyDeviceToHost, st));
+        if (wide) DSM_CUDA(cudaMemcpyAsync(hi.data(), d_hi, m, cudaMemcpyDeviceToHost, st));
+        DSM_CUDA(cudaStreamSynchronize(st));
+        for (uint64_t i = 0; i < m; ++i) sa_out[i] = wide ? (uint64_t)hi[i] << klo | lo[i] : lo[i];
+        *stats_out = b->stats;
+    } catch (const CudaError &e) {
+        g_create_error = std::string("dsmfm_dbg_refine: ") + cudaGetErrorString(e.code) + " in " + e.what;
+        rc = DSMFM_ECUDA;
+    }
+    dsmfm_destroy(b);
     return rc;
 }
 

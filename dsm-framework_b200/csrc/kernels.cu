@@ -2733,14 +2733,14 @@ void launch_heads(cudaStream_t st, int bits, const uint64_t *sorted_keys, uint64
     if (launches) ++*launches;
 }
 
-void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
+uint32_t launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
                    uint32_t *head_next, uint64_t n, uint32_t depth, const uint32_t *win_list, uint32_t n_list,
                    uint32_t *big_heads, uint32_t big_cap, uint32_t *big_count, unsigned long long *remaining,
                    uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, uint8_t *sa_hi,
                    int lo_bits, bool full_order, const uint32_t *diff_bits, uint32_t *launches, bool big_groups)
 {
     const unsigned grid = win_list ? n_list : (unsigned)div_up(n, kRefWindow);
-    if (grid == 0) return;
+    if (grid == 0) return 0;
     // groups of at least big_thr members are ranked by the whole warp around their dominant key
     // (DSMFM_REFINE_BIG=<members>; 0 or unset: every group by its own members)
     // -- the default when the refinement runs in place, i.e. when most suffixes sit in groups that have to be
@@ -2762,10 +2762,13 @@ void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *
 #undef SET
 #undef SET2
     });
+    uint32_t ran = 0; // the instantiation launched, set beside its launch
 #define RW2(B, W, O, C)                                                                                           \
-    refine_warps_kernel<B, W, O, C><<<grid, kRefThreads, sizeof(RwSmem<W>), st>>>(                                \
-        packed, sa, head_cur, head_next, n, depth, win_list, big_heads, big_cap, big_count, remaining, win_flag,  \
-        win_next, win_next_count, bwt, sa_hi, lo_bits, diff_bits, big_thr)
+    (refine_warps_kernel<B, W, O, C><<<grid, kRefThreads, sizeof(RwSmem<W>), st>>>(                               \
+         packed, sa, head_cur, head_next, n, depth, win_list, big_heads, big_cap, big_count, remaining, win_flag, \
+         win_next, win_next_count, bwt, sa_hi, lo_bits, diff_bits, big_thr),                                     \
+     ran = (uint32_t)B << kRwLaunchedBitsShift | (W ? kRwLaunchedWide : 0u) | (O ? kRwLaunchedOrder : 0u) |      \
+           (C ? kRwLaunchedCoop : 0u))
 #define RW(B, W, O)                                                                                               \
     do {                                                                                                          \
         if (big_thr <= kRwCap) RW2(B, W, O, true); else RW2(B, W, O, false);                                      \
@@ -2784,6 +2787,7 @@ void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *
 #undef RW2
     DSM_LAUNCH_CHECK();
     if (launches) ++*launches;
+    return ran;
 }
 
 uint64_t active_tiles(uint64_t head_words) { return div_up(head_words, kActTileWords); }

@@ -98,7 +98,10 @@ inline uint64_t head_words_for(uint64_t n) { return div_up(n, 32) + kRefCap / 32
 // suffix array is then only sorted as far as the BWT needs it.  diff_bits: launch_heads' bitmap while it is
 // still valid (first launch after the initial sort), nullptr afterwards (the kernel then compares the bytes).
 // big_groups: groups of 64+ members are ranked by the whole warp around their dominant key (kernels.cu, kRwBigGroup).
-void launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
+// Returns which instantiation of the kernel ran: kRwLaunched* bits and BITS << kRwLaunchedBitsShift (0: no window
+// to visit, nothing launched).
+constexpr uint32_t kRwLaunchedCoop = 2, kRwLaunchedWide = 4, kRwLaunchedOrder = 8, kRwLaunchedBitsShift = 8;
+uint32_t launch_refine(cudaStream_t st, int bits, const uint64_t *packed, uint32_t *sa, const uint32_t *head_cur,
                    uint32_t *head_next, uint64_t n, uint32_t depth, const uint32_t *win_list, uint32_t n_list,
                    uint32_t *big_heads, uint32_t big_cap, uint32_t *big_count, unsigned long long *remaining,
                    uint32_t *win_flag, uint32_t *win_next, uint32_t *win_next_count, uint8_t *bwt, uint8_t *sa_hi,

@@ -203,6 +203,8 @@ def lib():
     L.dsmfm_dbg_radix_sort.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]
     L.dsmfm_dbg_initial_sort.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint32] + \
         [C.c_void_p] * 8 + [C.POINTER(C.c_int)] * 3
+    L.dsmfm_dbg_refine.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32,
+                                   C.c_uint32, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(Stats), C.POINTER(C.c_uint32)]
     L.dsmfm_dbg_wavelet.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.POINTER(Index), C.POINTER(C.c_void_p)]
     L.dsmfm_dbg_free_index.argtypes = [C.c_void_p]
     L.dsmfm_dbg_free_index.restype = None
@@ -685,6 +687,33 @@ def initial_sort(docs, first_key_bits=0, word_cuts=None, device=0):
         raise DsmfmError(rc, (L.dsmfm_last_error(None) or b"").decode())
     out.update(remaining=int(out["remaining"][0]), bits=bits.value, first_syms=first_syms.value, carry=carry.value)
     return out
+
+
+RPATH_COMPACT, RPATH_COOP, RPATH_WIDE, RPATH_ORDER, RPATH_SCRATCH_ALLOC, RPATH_DENSE_ALLOC, RPATH_BIG_MULTI = \
+    1, 2, 4, 8, 16, 32, 64
+RPATH_BITS_SHIFT = 8  # (paths >> RPATH_BITS_SHIFT) & 15: bits per symbol of the refinement kernel launched
+
+
+def refine(docs, sa, head, depth, keep_sa=False, lo_bits=0, device=0):
+    """The refinement of one key range as the build runs it (dsmfm_dbg_refine), from the state the initial sort
+    leaves: sa (text positions), head (uint32 words, bit i: slot i opens a group) and the symbols `depth` that
+    every group's members share.  Returns a dict: sa (uint64), bwt (uint8), stats (dict) and paths (RPATH_* bits)."""
+    import numpy as np
+    L = lib()
+    docs = np.ascontiguousarray(docs, dtype=np.uint8)
+    sa = np.ascontiguousarray(sa, dtype=np.uint64)
+    head = np.ascontiguousarray(head, dtype=np.uint32)
+    m = sa.size
+    if head.size < (m + 31) // 32:
+        raise ValueError("head needs %d words" % ((m + 31) // 32))
+    sa_out, bwt_out = np.empty(m, np.uint64), np.empty(m, np.uint8)
+    st, paths = Stats(), C.c_uint32()
+    rc = L.dsmfm_dbg_refine(device, docs.ctypes.data, docs.size, sa.ctypes.data, head.ctypes.data, m, depth,
+                            FLAG_KEEP_SA if keep_sa else 0, lo_bits, sa_out.ctypes.data, bwt_out.ctypes.data,
+                            C.byref(st), C.byref(paths))
+    if rc != OK:
+        raise DsmfmError(rc, (L.dsmfm_last_error(None) or b"").decode())
+    return dict(sa=sa_out, bwt=bwt_out, stats=st.as_dict(), paths=paths.value)
 
 
 def wavelet_fmi(seq, device=0):

@@ -528,6 +528,35 @@ DSMFM_API int dsmfm_dbg_initial_sort(int device, const uint8_t *docs, uint64_t n
                                      uint64_t *sorted_keys, uint32_t *sa, uint32_t *head, uint32_t *diff, uint8_t *bwt,
                                      uint64_t *remaining, int *bits, int *first_syms, int *carry);
 
+/* The refinement of one key range, as build() runs it after the initial sort: the compaction of the groups with
+ * mixed BWT symbols (or refinement in place), the rounds with their window worklist and large-group path, and the
+ * BWT bytes scattered back.  State in (host): the text docs[n] (as dsmfm_dbg_initial_sort takes it), sa_in[m]
+ * (text positions, 1 <= m <= n; a subset of the suffixes is allowed, as a key range of a sharded build is),
+ * head_in[ceil(m/32)] (bit i: slot i opens a group; bit 0 set), depth (symbols the members of every group are known
+ * to share).  flags: 0 (the BWT-only order: groups whose members share one BWT symbol stay as they are) or
+ * DSMFM_FLAG_KEEP_SA (the full suffix order).  lo_bits: 0 (u32 positions), or 4..32 (positions split into
+ * lo_bits low bits and a high byte, the wide kernels).  The carried BWT bytes, the difference bits and the
+ * count of suffixes in groups of >= 2 are derived on the host as the initial sort would hand them over.
+ * Out (host): sa_out[m], bwt_out[m], stats (refine_launches, fallback_elems, rounds, refine_members, active[],
+ * refine_key_fetches), paths (DSMFM_RPATH_* bits, DSMFM_RPATH_BITS: bits per symbol of the kernel launched).
+ * Buffers are allocated as build() allocates them for a range of m suffixes (DSMFM_GUARD covers them).
+ * DSMFM_EINVAL (nothing launched) on malformed text (as dsmfm_dbg_initial_sort refuses it, n < 2^32 - 2112
+ * included), m outside [1, n], a position >= n or listed twice, head bit 0 clear, a group of >= 2 whose positions
+ * do not ascend or whose members differ or reach a terminator within their first `depth` symbols, lo_bits
+ * outside {0} and [4, 32], a position >= 2^(lo_bits + 8), or unknown flags. */
+#define DSMFM_RPATH_COMPACT 1u       /* the mixed groups were refined as dense copies (else: in place)         */
+#define DSMFM_RPATH_COOP 2u          /* the whole-warp ranking instantiation of the kernel ran                  */
+#define DSMFM_RPATH_WIDE 4u          /* the wide-position instantiation ran                                     */
+#define DSMFM_RPATH_ORDER 8u         /* the full-order instantiation ran                                        */
+#define DSMFM_RPATH_SCRATCH_ALLOC 16u /* the compaction scratch was allocated (else: carved from a key buffer)  */
+#define DSMFM_RPATH_DENSE_ALLOC 32u  /* the dense arrays were allocated (else: carved from a key buffer)        */
+#define DSMFM_RPATH_BIG_MULTI 64u    /* a round sent several groups down the large-group path (sort by group id) */
+#define DSMFM_RPATH_BITS_SHIFT 8     /* bits 8..11: bits per symbol (3, 4, 8) of the refinement kernel launched    */
+#define DSMFM_RPATH_BITS(paths) (((paths) >> DSMFM_RPATH_BITS_SHIFT) & 15u)
+DSMFM_API int dsmfm_dbg_refine(int device, const uint8_t *docs, uint64_t n, const uint64_t *sa_in,
+                               const uint32_t *head_in, uint64_t m, uint32_t depth, uint32_t flags, int lo_bits,
+                               uint64_t *sa_out, uint8_t *bwt_out, dsmfm_stats *stats, uint32_t *paths);
+
 /* Wavelet tree + BitRank directories for an arbitrary byte sequence (the
  * HuffWT::makeHuffWT path alone); `out` pointers are valid until
  * dsmfm_dbg_free_index. */
